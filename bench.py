@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the localization-inference hot path (BASELINE.json: videos/s, fwd + decode + soft-NMS).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload audio|av12|av13]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload audio|av12|av13] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = 32 batches of 32 synthetic AV-Deepfake1M-shaped videos (1024 videos) on every rank, each batch one pass of
@@ -213,12 +213,8 @@ def run_reference(args):
     vals = []
     for _ in range(args.warmup if args.warmup < 1 else 1):
         cpu_reference(args.workload, 2, threads)
-    t_total = 0.0
-    for _ in range(max(1, args.steps)):
-        v, dt = cpu_reference(args.workload, n, threads)
-        vals.append(v); t_total += dt
-        if t_total > 60:       # bounded sample: the whole arm ends within ~1.5 minutes whatever --steps says
-            break
+    for _ in range(args.steps):
+        vals.append(cpu_reference(args.workload, n, threads)[0])
     v = float(np.mean(vals))
     line = {"impl": "reference", "metric": "videos/sec localization inference (fwd+decode+soft-NMS)", "value": v, "unit": "videos/s",
             "n_gpus": args.gpus, "steps": len(vals), "warmup": args.warmup, "ms_per_step": 1000.0 * n / v,
@@ -460,6 +456,14 @@ def measure_workload(args, workload, steps, rank, world, local, dist, full):
     value = world * n_batches * BATCH / (ms / 1000.0)
     assert int(counter.item()) == n_batches * BATCH and allrec.shape[0] == world * n_batches * BATCH
     assert bool((ring[:, 1] >= 0).all()) and float(ring[:, 1].max()) <= K
+    last_step = None
+    if full and args.dump_outputs:
+        # every step replays the same pool of batches, so the last step computed one result per pool video of every rank.
+        # The lanes append records in whatever order they finish and a step's last records can land after the next
+        # step's first ones: keep one row per video index over all timed rows (rows sorted by index, then contents).
+        rows = allrec.cpu().numpy()
+        rows = rows[np.lexsort(rows.T[::-1])]
+        last_step = rows[np.unique(rows[:, 0], return_index=True)[1]]
 
     # ---------------- end to end through the public API (host buffers) ----------------
     # model.stream(batches): host numpy arrays in, host tensors out; every step packs its videos into pinned
@@ -530,7 +534,8 @@ def measure_workload(args, workload, steps, rank, world, local, dist, full):
         del dsts
     res = {"value": value, "ms": ms, "launches": launches, "clocks": clocks, "e2e": e2e_value, "e2e_pageable": e2e_pageable,
            "e2e_shard": e2e_shard, "h2d_ceiling": ceiling,
-           "h2d": h2d_step, "d2h": d2h_step, "desc": desc, "cfg": cfg, "name": name, "n_lanes": n_lanes, "h2d_batch": h2d}
+           "h2d": h2d_step, "d2h": d2h_step, "desc": desc, "cfg": cfg, "name": name, "n_lanes": n_lanes, "h2d_batch": h2d,
+           "last_step": last_step, "K": K}
     if not full:
         return res, None
 
@@ -647,6 +652,8 @@ def run_ours(args):
 
     line = None
     if rank == 0:
+        if args.dump_outputs:
+            dump_records(args.dump_outputs, r["last_step"], r["K"])
         ms_step = r["ms"] / args.steps
         line = {"metric": "videos/sec localization inference (fwd+decode+soft-NMS)", "value": r["value"], "unit": "videos/s",
                 "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms_step,
@@ -723,6 +730,16 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_records(out_dir, rows, K):
+    """The timed pass's per-video results (what model.forward_streams returns per video, padded to K segments) as
+    out_dir/<name>.npy: video_index, n_segments, video_cls [N]; scores [N, K]; segments [N, K, 2] (seconds)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"video_index": rows[:, 0], "n_segments": rows[:, 1], "video_cls": rows[:, 2],
+              "scores": rows[:, 3:3 + K], "segments": rows[:, 3 + K:3 + 3 * K].reshape(-1, K, 2)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 _REAL_STDOUT = None
 
 
@@ -758,7 +775,13 @@ def main():
     ap.add_argument("--lanes", type=int, default=8, help="batches in flight at once (each on its own stream and buffer set)")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from Python instead of replaying CUDA graphs")
     ap.add_argument("--dump-launches", default=None, help="write the per-launch CUDA-event timings of one step to this json")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the per-video results of the last timed step as DIR/<name>.npy (same inputs on every run)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "ours" and args.gpus > 1 and world == 1:
         # convenience: relaunch under torchrun
