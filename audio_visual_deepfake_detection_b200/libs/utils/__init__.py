@@ -1,6 +1,8 @@
 from .nms import batched_nms
-from .infer_utils import inference_one_epoch, inference_sharded, fix_random_seed, AverageMeter
-from .results import merge_results, filter_segments, video_probability
+from .infer_utils import inference_one_epoch, inference_sharded, valid_one_epoch, fix_random_seed, AverageMeter
+from .results import merge_results, filter_segments, video_probability, iter_result_records
+from .metrics import ANETdetection, load_gt_seg_from_json, load_gt_seg_from_metadata
 
-__all__ = ["batched_nms", "inference_one_epoch", "inference_sharded", "fix_random_seed", "AverageMeter", "merge_results", "filter_segments",
-           "video_probability"]
+__all__ = ["batched_nms", "inference_one_epoch", "inference_sharded", "valid_one_epoch", "fix_random_seed", "AverageMeter",
+           "merge_results", "filter_segments", "video_probability", "iter_result_records", "ANETdetection",
+           "load_gt_seg_from_json", "load_gt_seg_from_metadata"]

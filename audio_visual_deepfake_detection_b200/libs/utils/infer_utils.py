@@ -1,9 +1,11 @@
 """Inference driver with the reference's interface (libs/utils/train_utils.py:510-596
-`inference_one_epoch`, :22-40 `fix_random_seed`). Training utilities (optimizer, scheduler,
-EMA, checkpoint saving) are outside the accelerated path."""
+`inference_one_epoch`, :22-40 `fix_random_seed`, `valid_one_epoch`). Training utilities (optimizer,
+scheduler, EMA, checkpoint saving) are outside the accelerated path."""
 import json
 import os
+import pickle
 import random
+import time
 
 import numpy as np
 import torch
@@ -62,6 +64,50 @@ def inference_one_epoch(val_loader, model, curr_epoch, ext_score_file=None, eval
         with open(f"{output_folder}/data_left.json", "w", encoding="utf-8") as f:
             json.dump(batch_results, f, ensure_ascii=False, indent=4)
     return batch_results
+
+
+def valid_one_epoch(val_loader, model, curr_epoch, ext_score_file=None, evaluator=None, output_file=None, tb_writer=None,
+                    print_freq=20):
+    """The reference's validation loop: runs `model(video_list)` over the loader, collects every segment into the
+    evaluator's dict form (video-id, t-start, t-end, label, score) and returns the evaluator's average mAP
+    (libs/utils/metrics.py ANETdetection, on the GPU). Without an evaluator the dict is pickled to `output_file` and
+    0.0 is returned. ext_score_file (the reference's external classification scores, postprocess_results) is not
+    supported."""
+    assert (evaluator is not None) or (output_file is not None)
+    if ext_score_file is not None:
+        raise NotImplementedError("ext_score_file (postprocess_results with external classification scores) is not supported")
+    batch_time = AverageMeter()
+    model.eval()
+    results = {"video-id": [], "t-start": [], "t-end": [], "label": [], "score": []}
+    start = time.time()
+    for iter_idx, video_list in enumerate(val_loader, 0):
+        with torch.no_grad():
+            output = model(video_list)
+            for vid_idx in range(len(output)):
+                n = output[vid_idx]["segments"].shape[0]
+                if n > 0:
+                    results["video-id"].extend([output[vid_idx]["video_id"]] * n)
+                    results["t-start"].append(output[vid_idx]["segments"][:, 0])
+                    results["t-end"].append(output[vid_idx]["segments"][:, 1])
+                    results["label"].append(output[vid_idx]["labels"])
+                    results["score"].append(output[vid_idx]["scores"])
+        if (iter_idx != 0) and iter_idx % print_freq == 0:
+            torch.cuda.synchronize()
+            batch_time.update((time.time() - start) / print_freq)
+            start = time.time()
+            print("Test: [{0:05d}/{1:05d}]\tTime {batch_time.val:.2f} ({batch_time.avg:.2f})".format(
+                iter_idx, len(val_loader), batch_time=batch_time))
+    for k, dt in (("t-start", torch.float32), ("t-end", torch.float32), ("label", torch.long), ("score", torch.float32)):
+        results[k] = torch.cat(results[k]).cpu().numpy() if results[k] else torch.zeros(0, dtype=dt).numpy()
+    if evaluator is not None:
+        _, mAP, _ = evaluator.evaluate(results, verbose=True)
+    else:
+        with open(output_file, "wb") as f:
+            pickle.dump(results, f)
+        mAP = 0.0
+    if tb_writer is not None:
+        tb_writer.add_scalar("validation/mAP", mAP, curr_epoch)
+    return mAP
 
 
 def inference_sharded(dataset, model, output_folder, batch_size=32, rank=0, world=1, print_freq=0):

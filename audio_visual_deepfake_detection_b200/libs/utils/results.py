@@ -23,11 +23,12 @@ def filter_segments(scores, segments, min_score=0.2):
     return out if out else [[0, 0, 0]]
 
 
-def merge_results(folders, out_dir=None, min_score=0.2, snap=0.9):
+def iter_result_records(folders, pattern="*.json"):
+    """The result records of every `pattern` file (sorted by name) of every folder, in that order, skipping `prediction*`
+    files; a video id seen before is skipped (first occurrence wins, like the notebook)."""
     seen = set()
-    probs, segs = [], {}
     for folder in folders:
-        for path in sorted(glob.glob(os.path.join(folder, "*.json"))):
+        for path in sorted(glob.glob(os.path.join(folder, pattern))):
             if os.path.basename(path).startswith("prediction"):
                 continue
             with open(path, "r", encoding="utf-8") as f:
@@ -37,8 +38,15 @@ def merge_results(folders, out_dir=None, min_score=0.2, snap=0.9):
                 if vid in seen:
                     continue
                 seen.add(vid)
-                probs.append([vid, str(video_probability(item["video_cls"], snap))])
-                segs[vid] = filter_segments(item["scores"], item["segments"], min_score)
+                yield item
+
+
+def merge_results(folders, out_dir=None, min_score=0.2, snap=0.9):
+    probs, segs = [], {}
+    for item in iter_result_records(folders):
+        vid = item["video_id"]
+        probs.append([vid, str(video_probability(item["video_cls"], snap))])
+        segs[vid] = filter_segments(item["scores"], item["segments"], min_score)
     probs.sort(key=lambda x: x[0])
     if out_dir is not None:
         os.makedirs(out_dir, exist_ok=True)

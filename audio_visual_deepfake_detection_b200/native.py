@@ -8,7 +8,7 @@ signatures below take raw device pointers.
 """
 import ctypes
 import os
-from ctypes import POINTER, Structure, c_char_p, c_float, c_int32, c_int64, c_size_t, c_uint8, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_double, c_float, c_int32, c_int64, c_size_t, c_uint8, c_void_p
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AVDF_LIB_PATH") or os.path.join(HERE, "csrc", "libavdf_sm100.so")      # (override: kernel experiments)
@@ -26,7 +26,7 @@ EXPORTS = [
     "avdf_conv_gemm_workspace_bytes", "avdf_conv_gemm", "avdf_mlp_fused", "avdf_ln_dwconv_ln", "avdf_attention",
     "avdf_ln_rows", "avdf_instnorm_lrelu", "avdf_fpn_fuse", "avdf_head_final", "avdf_head_combine",
     "avdf_vcls_exp12", "avdf_vcls_exp13", "avdf_host_pack", "avdf_host_all_pinned", "avdf_h2d_gather",
-    "avdf_logmel", "avdf_byola_conv1_pool", "avdf_byola_pool",
+    "avdf_logmel", "avdf_byola_conv1_pool", "avdf_byola_pool", "avdf_eval_workspace_bytes", "avdf_eval_detection",
 ]
 
 
@@ -92,6 +92,19 @@ class MlpFusedArgs(Structure):
     ]
 
 
+class EvalArgs(Structure):
+    _fields_ = [
+        ("n_pred", c_int64), ("n_video", c_int32), ("n_gt", c_int32),
+        ("pred_off", c_void_p), ("pred_seg", c_void_p), ("pred_score", c_void_p), ("gt_off", c_void_p), ("gt_seg", c_void_p),
+        ("thresholds", POINTER(c_double)), ("n_thr", c_int32), ("top_k", POINTER(c_int32)), ("n_topk", c_int32),
+        ("ap", c_void_p), ("recall_hits", c_void_p), ("tp_mask", c_void_p), ("pred_rank", c_void_p), ("status", c_void_p),
+        ("workspace", c_void_p), ("workspace_bytes", c_size_t),
+    ]
+
+
+# status bits of avdf_eval_detection (AVDF_EVAL_*)
+EVAL_PRED_LIMIT, EVAL_GT_LIMIT, EVAL_BAD_OFFSETS = 1, 2, 4
+
 _lib = None
 
 
@@ -139,10 +152,13 @@ def lib():
     L.avdf_logmel.argtypes = [c_void_p] * 4 + [c_int32] * 3 + [c_void_p] * 5 + [c_int32, c_float, c_float, c_void_p, c_void_p]
     L.avdf_byola_conv1_pool.argtypes = [c_void_p] * 6 + [c_int32, c_void_p, c_int32, c_void_p, c_void_p]
     L.avdf_byola_pool.argtypes = [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p]
+    L.avdf_eval_workspace_bytes.restype = c_size_t
+    L.avdf_eval_workspace_bytes.argtypes = [c_int64, c_int32]
+    L.avdf_eval_detection.argtypes = [POINTER(EvalArgs), c_void_p]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("avdf_last_error", "avdf_nms_workspace_bytes", "avdf_postprocess_workspace_bytes",
-                        "avdf_conv_gemm_workspace_bytes", "avdf_abi_version"):
+                        "avdf_conv_gemm_workspace_bytes", "avdf_eval_workspace_bytes", "avdf_abi_version"):
             fn.restype = c_int32
     if L.avdf_abi_version() != 3:
         raise AvdfError("libavdf_sm100.so ABI version mismatch")

@@ -446,3 +446,50 @@ def byola_pool(x, clip_step_in, clip_of_step, t_of_step, out, *, mel_in, pad_out
     assert out.numel() == n_steps * (mel_in // 2 + 2 * pad_out) * 64
     _call("avdf_byola_pool", L.avdf_byola_pool, (nv.ptr(x), _dt(x), mel_in, nv.ptr(clip_step_in), nv.ptr(clip_of_step), nv.ptr(t_of_step), n_steps,
           int(pad_out), nv.ptr(out), nv.ptr(mask_out) if mask_out is not None else None, _stream(),), launches=1, work={"bytes": _nbytes(x, out)})
+
+
+# ---------------------------------------------------------------------------- detection evaluation (one class)
+def eval_detection(pred_off, pred_seg, pred_score, gt_off, gt_seg, thresholds, top_k, *, tp_mask=None, pred_rank=None,
+                   workspace=None, check_status=True):
+    """ActivityNet AP per tIoU threshold + Recall@kx hit counts of one class, videos in CSR form (include/avdf.h
+    avdf_eval_detection): pred_off int64 [V+1], pred_seg fp64 [N, 2], pred_score fp64 [N], gt_off int32 [V+1],
+    gt_seg fp64 [G, 2] (G >= 1); thresholds / top_k host sequences. tp_mask: optional uint16 [N] output. pred_rank:
+    optional int32 [N] permutation that orders equal scores instead of the CSR position.
+    Returns (ap fp64 [n_thr], hits int64 [n_thr, n_topk], status int32 [1]) on the device. check_status reads the status
+    word (a synchronisation) and raises AvdfError when a per-video limit was exceeded (no results were written)."""
+    L = nv.lib()
+    _chk(pred_off, torch.int64, "pred_off"); _chk(pred_seg, torch.float64, "pred_seg"); _chk(pred_score, torch.float64, "pred_score")
+    _chk(gt_off, torch.int32, "gt_off"); _chk(gt_seg, torch.float64, "gt_seg"); _chk(tp_mask, torch.uint16, "tp_mask")
+    _chk(pred_rank, torch.int32, "pred_rank")
+    n, n_video, n_gt = pred_score.numel(), pred_off.numel() - 1, gt_seg.shape[0]
+    assert pred_seg.shape == (n, 2) and gt_seg.shape == (n_gt, 2) and gt_off.numel() == n_video + 1
+    assert tp_mask is None or tp_mask.numel() == n
+    dev = pred_off.device
+    thr = [float(t) for t in thresholds]
+    ks = [int(k) for k in top_k]
+    ap = torch.empty(len(thr), dtype=torch.float64, device=dev)
+    hits = torch.empty((len(thr), len(ks)), dtype=torch.int64, device=dev)
+    status = torch.empty(1, dtype=torch.int32, device=dev)
+    need = L.avdf_eval_workspace_bytes(n, n_video)
+    if workspace is None or workspace.numel() * workspace.element_size() < need:
+        workspace = torch.empty(need, dtype=torch.uint8, device=dev)
+    a = nv.EvalArgs()
+    a.n_pred, a.n_video, a.n_gt = n, n_video, n_gt
+    a.pred_off, a.pred_seg, a.pred_score = pred_off.data_ptr(), pred_seg.data_ptr() if n else None, pred_score.data_ptr() if n else None
+    a.gt_off, a.gt_seg = gt_off.data_ptr(), gt_seg.data_ptr()
+    thr_arr, k_arr = (ctypes.c_double * max(1, len(thr)))(*thr), (c_int32 * max(1, len(ks)))(*ks)
+    a.thresholds, a.n_thr, a.top_k, a.n_topk = thr_arr, len(thr), k_arr, len(ks)
+    a.ap, a.recall_hits, a.status = ap.data_ptr(), hits.data_ptr(), status.data_ptr()
+    a.tp_mask = tp_mask.data_ptr() if tp_mask is not None and n else None
+    a.pred_rank = pred_rank.data_ptr() if pred_rank is not None and n else None
+    a.workspace, a.workspace_bytes = workspace.data_ptr(), workspace.numel() * workspace.element_size()
+    _call("avdf_eval_detection", L.avdf_eval_detection, (ctypes.byref(a), _stream(),), launches=1,
+          work={"bytes": n * (16 + 8) + n_gt * 16})
+    if check_status:
+        st = int(status.item())
+        if st:
+            why = [w for b, w in ((nv.EVAL_PRED_LIMIT, "a video has more than 8192 predictions"),
+                                  (nv.EVAL_GT_LIMIT, "a video has more than 64 ground-truth rows"),
+                                  (nv.EVAL_BAD_OFFSETS, "malformed CSR offsets")) if st & b]
+            raise nv.AvdfError("avdf_eval_detection: %s (status %d); no results were written" % ("; ".join(why), st))
+    return ap, hits, status

@@ -39,6 +39,8 @@
  *   avdf_fpn_fuse                   FPN1D top-down sum + depthwise conv + LN (necks.py:75-93)
  *   avdf_head_final                 last conv of the cls / reg heads + Scale + ReLU (av_fd_no_recon.py:82-89,152-159)
  *   avdf_vcls_exp12 / _exp13        video-level classifier tails (blocks.py:1608-1626, 1682-1700)
+ *   avdf_eval_detection             libs/utils/metrics.py ANETdetection (AP and Recall@kx of one class), the evaluator
+ *                                   valid_one_epoch calls (libs/utils/train_utils.py)
  */
 #ifndef AVDF_H_
 #define AVDF_H_
@@ -333,6 +335,41 @@ AVDF_API int avdf_byola_conv1_pool(const float* lms, const int32_t* clip_frame_o
 AVDF_API int avdf_byola_pool(const void* in, int32_t dtype, int32_t mel_in, const int32_t* clip_step_in,
                 const int32_t* clip_of_step, const int32_t* t_of_step, int32_t n_steps_out, int32_t pad_out, void* out,
                 uint8_t* mask_out, void* stream);
+
+/* ---- detection evaluation of ONE class: ActivityNet AP per tIoU threshold + Recall@kx (ActionFormer / UMMAFormer
+ * libs/utils/metrics.py ANETdetection: compute_average_precision_detection, compute_topkx_recall_detection) ----
+ * Videos in CSR form: video v owns predictions [pred_off[v], pred_off[v+1]) and GT rows [gt_off[v], gt_off[v+1]).
+ * Prediction order is score descending, ties by smaller input index; within a video the GT rows are tried in tIoU-descending
+ * order, ties by larger GT index. tIoU is fp64 in numpy's operation order. AP is the area under the monotone precision
+ * envelope over npos = n_gt; recall_hits[t * n_topk + q] counts the GT rows whose best tIoU over their video's top
+ * top_k[q] * n_gt(video) predictions is >= thresholds[t] (divide by n_gt for Recall@kx). Limits: n_thr <= 16, n_topk <= 4,
+ * <= 8192 predictions and <= 64 GT rows per video. Per-video limits are checked on the device: a violation sets bits of
+ * *status (AVDF_EVAL_*) and the call then writes none of ap / recall_hits / tp_mask. Deterministic (bit-identical runs). */
+enum { AVDF_EVAL_PRED_LIMIT = 1, AVDF_EVAL_GT_LIMIT = 2, AVDF_EVAL_BAD_OFFSETS = 4 };
+typedef struct avdf_eval_args {
+  int64_t n_pred;                /* predictions (< 2^31) */
+  int32_t n_video;               /* videos with GT or predictions of this class */
+  int32_t n_gt;                  /* GT rows (npos >= 1) */
+  const int64_t* pred_off;       /* [n_video + 1] */
+  const double* pred_seg;        /* [n_pred, 2] (start, end), 16-byte aligned */
+  const double* pred_score;      /* [n_pred] */
+  const int32_t* gt_off;         /* [n_video + 1] */
+  const double* gt_seg;          /* [n_gt, 2], 16-byte aligned */
+  const double* thresholds;      /* HOST [n_thr] tIoU thresholds */
+  int32_t n_thr;
+  const int32_t* top_k;          /* HOST [n_topk] */
+  int32_t n_topk;
+  double* ap;                    /* [n_thr] */
+  int64_t* recall_hits;          /* [n_thr * n_topk] */
+  uint16_t* tp_mask;             /* [n_pred] or NULL: bit t = TP at thresholds[t], at the prediction's input position */
+  const int32_t* pred_rank;      /* [n_pred] or NULL: a permutation of 0 .. n_pred - 1 that breaks score ties instead of the
+                                  * position (must increase with the position inside every video); lets a caller whose
+                                  * predictions are not grouped by video keep its own row order for the ties */
+  int32_t* status;               /* [1] 0 on success, else AVDF_EVAL_* bits */
+  void* workspace; size_t workspace_bytes;   /* 256-byte aligned */
+} avdf_eval_args;                 /* host struct */
+AVDF_API size_t avdf_eval_workspace_bytes(int64_t n_pred, int32_t n_video);
+AVDF_API int avdf_eval_detection(const avdf_eval_args* args, void* stream);
 
 /* ---- HOST: gather n byte spans (src[i] -> dst[i], nbytes[i] bytes; all HOST pointers, any alignment; dst is normally
  * a slice of a pinned staging buffer) with up to n_threads threads of a pool that lives inside the library
