@@ -20,6 +20,10 @@
 //              over blocks, then sum_{i TP} max_{j >= i, j TP} prec_j per block and a fixed-order sum: AP = sum / npos.
 //              The envelope max_{j>=i} prec_j of the reference's interpolated_prec_rec is attained at a TP row, so
 //              only TP rows compute a precision. No floating-point atomics: bit-identical across runs.
+//
+// Proposal evaluation (ActivityNet eval_proposal.py `average_recall_vs_avg_nr_proposals`, avdf_eval_proposal) shares the
+// per-video validation, the score key, the shared-memory sort and seg_tiou: one warp per GT video walks its first keep[v]
+// proposals and turns each GT row's first rank at each threshold into one integer count (see eval_prop_match_kernel).
 #include <algorithm>
 
 #include "common.cuh"
@@ -71,8 +75,9 @@ __device__ __forceinline__ double seg_tiou(double ps, double pe, double gs, doub
 }
 
 // ---------------------------------------------------------------------------------------------
+// keep (proposal evaluation, else nullptr): the walked prefix of every video, 0 <= keep[v] <= its row count
 __global__ void eval_validate_kernel(const int64_t* __restrict__ pred_off, const int32_t* __restrict__ gt_off, int n_video,
-                                     int64_t n_pred, int n_gt, int32_t* status) {
+                                     int64_t n_pred, int n_gt, int32_t* status, const int32_t* __restrict__ keep = nullptr) {
   int v = blockIdx.x * blockDim.x + threadIdx.x;
   if (v > n_video) return;
   int bad = 0;
@@ -84,6 +89,7 @@ __global__ void eval_validate_kernel(const int64_t* __restrict__ pred_off, const
     if (np < 0 || ng < 0) bad |= AVDF_EVAL_BAD_OFFSETS;
     if (np > EVAL_MAX_PRED) bad |= AVDF_EVAL_PRED_LIMIT;
     if (ng > EVAL_MAX_GT) bad |= AVDF_EVAL_GT_LIMIT;
+    if (keep && (keep[v] < 0 || keep[v] > np)) bad |= AVDF_EVAL_BAD_KEEP;
   }
   if (bad) atomicOr(status, bad);
 }
@@ -203,8 +209,35 @@ __global__ void __launch_bounds__(MATCH_WARPS * 32) eval_match_kernel(
   flush_hits(P, acc, hits_sm, hits);
 }
 
-// Videos whose predictions are out of order: one CTA sorts the (score key, row) pairs in shared memory (bitonic, unique
-// keys, so the order is exactly the stable one), then its first warp walks them.
+// Block-wide: row[0 .. n) = the local rows of one video's n <= EVAL_MAX_PRED entries of `score`, score descending, equal
+// scores by smaller row (bitonic sort of the unique (score key, row) pairs in shared memory, so the order is exactly the
+// stable one). Starts and ends with a barrier.
+__device__ void sort_video_rows(const double* __restrict__ score, int n, uint64_t* key, uint16_t* row) {
+  int m = 1;
+  while (m < n) m <<= 1;
+  __syncthreads();
+  for (int i = threadIdx.x; i < m; i += blockDim.x) {
+    key[i] = i < n ? score_key(score[i]) : ~0ull;
+    row[i] = (uint16_t)(i < n ? i : 0xffff);
+  }
+  for (int size = 2; size <= m; size <<= 1)
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      __syncthreads();
+      for (int i = threadIdx.x; i < m; i += blockDim.x) {
+        const int j = i ^ stride;
+        if (j > i) {
+          const bool up = (i & size) == 0;
+          const uint64_t ki = key[i], kj = key[j];
+          const uint16_t ri = row[i], rj = row[j];
+          const bool gt_ = ki > kj || (ki == kj && ri > rj);
+          if (gt_ == up) { key[i] = kj; key[j] = ki; row[i] = rj; row[j] = ri; }
+        }
+      }
+    }
+  __syncthreads();
+}
+
+// Videos whose predictions are out of order: one CTA sorts them (sort_video_rows), then its first warp walks them.
 __global__ void __launch_bounds__(SORTV_THREADS) eval_match_sorted_kernel(
     EvalParams P, const int64_t* __restrict__ pred_off, const double2* __restrict__ seg, const double* __restrict__ score,
     const int32_t* __restrict__ gt_off, const double2* __restrict__ gt, uint16_t* __restrict__ tp_mask,
@@ -224,28 +257,7 @@ __global__ void __launch_bounds__(SORTV_THREADS) eval_match_sorted_kernel(
     const int v = unsorted[k];
     const int64_t p0 = pred_off[v];
     const int n = (int)(pred_off[v + 1] - p0);
-    int m = 1;
-    while (m < n) m <<= 1;
-    __syncthreads();
-    for (int i = threadIdx.x; i < m; i += blockDim.x) {
-      key[i] = i < n ? score_key(score[p0 + i]) : ~0ull;
-      row[i] = (uint16_t)(i < n ? i : 0xffff);
-    }
-    for (int size = 2; size <= m; size <<= 1)
-      for (int stride = size >> 1; stride > 0; stride >>= 1) {
-        __syncthreads();
-        for (int i = threadIdx.x; i < m; i += blockDim.x) {
-          const int j = i ^ stride;
-          if (j > i) {
-            const bool up = (i & size) == 0;
-            const uint64_t ki = key[i], kj = key[j];
-            const uint16_t ri = row[i], rj = row[j];
-            const bool gt_ = ki > kj || (ki == kj && ri > rj);
-            if (gt_ == up) { key[i] = kj; key[j] = ki; row[i] = rj; row[j] = ri; }
-          }
-        }
-      }
-    __syncthreads();
+    sort_video_rows(score + p0, n, key, row);
     if (threadIdx.x < 32) {
       const int g0 = gt_off[v], n_gt = gt_off[v + 1] - g0;
       walk_video(P, seg, tp_mask, p0, n, gt, g0, n_gt, row, tiou_sm, acc);
@@ -618,6 +630,166 @@ __global__ void eval_finish_kernel(const double* __restrict__ blk_sum, int n_blk
 }
 
 // ---------------------------------------------------------------------------------------------
+// Proposal evaluation (ActivityNet eval_proposal.py, average_recall_vs_avg_nr_proposals), class-agnostic: per tIoU
+// threshold t and point j, the number of GT rows matched by their video's first cut_j(c) proposals in walk order, where
+// c = keep[v] (the video's walked prefix) or 1 for a video without proposals (upstream's zeros((n_gt, 1)) column) and
+// cut_j(c) = min(int(c * an_frac[j]), c). cut_j does not decrease in j, so a GT row whose first rank reaching t is r is
+// matched at exactly the points j >= j0, j0 = the first point with cut_j > r: one integer count into hist[t][j0], and a
+// prefix over j gives the matches. The walk stops once every (row, threshold) has its first rank, or at cut_99.
+constexpr int PROP_POINTS = 100;
+
+struct PropParams {
+  double thr[EVAL_MAX_THR];
+  double frac[PROP_POINTS];      // the host's pcn: one fp64 product c * frac[j] per cut, never recomputed here
+  int32_t n_thr, n_video;
+};
+
+// cut[j] = min(int(c * frac[j]), c) (one fp64 product truncated toward zero, numpy's astype(int)); returns cut[99], the
+// most ranks any point looks at. Warp-collective; the first barrier lets the warp's previous walk finish reading cut.
+__device__ __forceinline__ int prop_cuts(const PropParams& P, int c, int32_t* cut) {
+  __syncwarp();
+  for (int j = threadIdx.x & 31; j < PROP_POINTS; j += 32)
+    cut[j] = (int)min(__double2ll_rz(__dmul_rn((double)c, P.frac[j])), (long long)c);
+  __syncwarp();
+  return cut[PROP_POINTS - 1];
+}
+
+// The walk of one video by one warp over its first lim proposals (order == nullptr: input order, else order[r] is the
+// local row of rank r; virt: no proposals, the one column is a tIoU of 0). Lane l owns GT rows l and l + 32 and, per row,
+// the bit set of thresholds not reached yet. A rank whose tIoU does not exceed the row's running maximum reaches nothing
+// new, so the thresholds are only tried when the maximum grows.
+__device__ __forceinline__ void walk_proposals(const PropParams& P, const double2* __restrict__ seg, int64_t p0, int lim,
+                                               bool virt, const double2* __restrict__ gt, int g0, int n_gt,
+                                               const uint16_t* order, const int32_t* cut, uint32_t* hist_sm) {
+  const int lane = threadIdx.x & 31;
+  const uint32_t all = (1u << P.n_thr) - 1u;
+  double ga_s = 0, ga_e = 0, gb_s = 0, gb_e = 0;
+  uint32_t pend_a = 0, pend_b = 0;
+  if (lane < n_gt) { double2 g = gt[g0 + lane]; ga_s = g.x; ga_e = g.y; pend_a = all; }
+  if (lane + 32 < n_gt) { double2 g = gt[g0 + lane + 32]; gb_s = g.x; gb_e = g.y; pend_b = all; }
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  double run_a = nan, run_b = nan;         // NaN: the first rank is always tried; a NaN tIoU reaches nothing
+  auto reach = [&](uint32_t& pend, double& run, double u, int r) {
+    if (u <= run) return;
+    run = fmax(run, u);
+    for (uint32_t m = pend; m; m &= m - 1) {
+      const int t = __ffs(m) - 1;
+      if (u >= P.thr[t]) {
+        pend &= ~(1u << t);
+        int lo = 0, hi = PROP_POINTS - 1;      // first j with cut[j] > r; cut[99] = lim > r
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (cut[mid] > r) hi = mid; else lo = mid + 1; }
+        atomicAdd(&hist_sm[t * PROP_POINTS + lo], 1u);
+      }
+    }
+  };
+  for (int base = 0; base < lim; base += 32) {
+    if (!__any_sync(0xffffffffu, pend_a | pend_b)) break;
+    const int cnt = min(32, lim - base);
+    double ps = 0, pe = 0;
+    if (lane < cnt && !virt) {
+      const double2 s = seg[p0 + (order ? (int)order[base + lane] : base + lane)];
+      ps = s.x; pe = s.y;
+    }
+    for (int j = 0; j < cnt; ++j) {
+      const double s = __shfl_sync(0xffffffffu, ps, j), e = __shfl_sync(0xffffffffu, pe, j);
+      if (pend_a) reach(pend_a, run_a, virt ? 0.0 : seg_tiou(s, e, ga_s, ga_e), base + j);
+      if (pend_b) reach(pend_b, run_b, virt ? 0.0 : seg_tiou(s, e, gb_s, gb_e), base + j);
+    }
+  }
+}
+
+__device__ __forceinline__ void prop_flush(const PropParams& P, const uint32_t* hist_sm, unsigned long long* hist) {
+  __syncthreads();
+  for (int i = threadIdx.x; i < P.n_thr * PROP_POINTS; i += blockDim.x)
+    if (hist_sm[i]) atomicAdd(&hist[i], (unsigned long long)hist_sm[i]);
+}
+
+__global__ void __launch_bounds__(MATCH_WARPS * 32) eval_prop_match_kernel(
+    PropParams P, const int64_t* __restrict__ prop_off, const double2* __restrict__ seg, const double* __restrict__ score,
+    const int32_t* __restrict__ keep, const int32_t* __restrict__ gt_off, const double2* __restrict__ gt,
+    int32_t* __restrict__ unsorted, int32_t* __restrict__ n_unsorted, unsigned long long* __restrict__ hist,
+    const int32_t* __restrict__ status) {
+  __shared__ int32_t cut_sm[MATCH_WARPS][PROP_POINTS];
+  __shared__ uint32_t hist_sm[EVAL_MAX_THR * PROP_POINTS];
+  if (*status) return;
+  for (int i = threadIdx.x; i < EVAL_MAX_THR * PROP_POINTS; i += blockDim.x) hist_sm[i] = 0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  for (int v = blockIdx.x * MATCH_WARPS + w; v < P.n_video; v += gridDim.x * MATCH_WARPS) {
+    const int64_t p0 = prop_off[v];
+    const int n = (int)(prop_off[v + 1] - p0);
+    const int g0 = gt_off[v], n_gt = gt_off[v + 1] - g0;
+    if (n_gt == 0) continue;
+    const int lim = prop_cuts(P, n ? keep[v] : 1, cut_sm[w]);
+    if (lim == 0) continue;
+    bool ok = true;                       // walk order = input order iff the scores do not increase
+    for (int i = lane; i + 1 < n && ok; i += 32) ok = score[p0 + i] >= score[p0 + i + 1];
+    if (!__all_sync(0xffffffffu, ok)) {
+      if (lane == 0) unsorted[atomicAdd(n_unsorted, 1)] = v;
+      continue;
+    }
+    walk_proposals(P, seg, p0, lim, n == 0, gt, g0, n_gt, nullptr, cut_sm[w], hist_sm);
+  }
+  prop_flush(P, hist_sm, hist);
+}
+
+// the videos eval_prop_match_kernel queued: one CTA sorts one video's rows (sort_video_rows), its first warp walks them
+__global__ void __launch_bounds__(SORTV_THREADS) eval_prop_match_sorted_kernel(
+    PropParams P, const int64_t* __restrict__ prop_off, const double2* __restrict__ seg, const double* __restrict__ score,
+    const int32_t* __restrict__ keep, const int32_t* __restrict__ gt_off, const double2* __restrict__ gt,
+    const int32_t* __restrict__ unsorted, const int32_t* __restrict__ n_unsorted, unsigned long long* __restrict__ hist,
+    const int32_t* __restrict__ status) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  uint64_t* key = reinterpret_cast<uint64_t*>(smem_raw);                        // [EVAL_MAX_PRED]
+  uint16_t* row = reinterpret_cast<uint16_t*>(key + EVAL_MAX_PRED);             // [EVAL_MAX_PRED]
+  __shared__ int32_t cut_sm[PROP_POINTS];
+  __shared__ uint32_t hist_sm[EVAL_MAX_THR * PROP_POINTS];
+  if (*status) return;
+  const int count = *n_unsorted;
+  if ((int)blockIdx.x >= count) return;
+  for (int i = threadIdx.x; i < EVAL_MAX_THR * PROP_POINTS; i += blockDim.x) hist_sm[i] = 0;
+  for (int k = blockIdx.x; k < count; k += gridDim.x) {
+    const int v = unsorted[k];
+    const int64_t p0 = prop_off[v];
+    sort_video_rows(score + p0, (int)(prop_off[v + 1] - p0), key, row);
+    if (threadIdx.x < 32) {
+      const int g0 = gt_off[v], n_gt = gt_off[v + 1] - g0;
+      const int lim = prop_cuts(P, keep[v], cut_sm);
+      walk_proposals(P, seg, p0, lim, false, gt, g0, n_gt, row, cut_sm, hist_sm);
+    }
+  }
+  prop_flush(P, hist_sm, hist);
+}
+
+// matches[t][j] = sum over j' <= j of hist[t][j']. Nothing is written on a bad status.
+__global__ void eval_prop_finish_kernel(const unsigned long long* __restrict__ hist, int n_thr, int64_t* __restrict__ matches,
+                                        const int32_t* status) {
+  if (*status) return;
+  const int t = threadIdx.x;
+  if (t >= n_thr) return;
+  unsigned long long run = 0;
+  for (int j = 0; j < PROP_POINTS; ++j) {
+    run += hist[t * PROP_POINTS + j];
+    matches[t * PROP_POINTS + j] = (int64_t)run;
+  }
+}
+
+struct PropWs {
+  int32_t* unsorted; int32_t* n_unsorted; unsigned long long* hist;
+  size_t bytes;
+};
+
+static PropWs prop_layout(char* base, int32_t n_video) {
+  PropWs w;
+  size_t off = 0;
+  auto take = [&](size_t bytes) { char* p = base ? base + off : nullptr; off += (bytes + 255) & ~size_t(255); return p; };
+  w.unsorted = (int32_t*)take(4 * (size_t)(n_video > 0 ? n_video : 1)); w.n_unsorted = (int32_t*)take(4);
+  w.hist = (unsigned long long*)take(8 * EVAL_MAX_THR * PROP_POINTS);
+  w.bytes = off;
+  return w;
+}
+
+// ---------------------------------------------------------------------------------------------
 struct EvalWs {
   uint64_t* keys[2]; uint16_t* pay[2]; uint16_t* tp;
   uint32_t* hist; SortPlan* plan; uint32_t* tile_cnt; int32_t* unsorted; int32_t* n_unsorted;
@@ -736,4 +908,55 @@ extern "C" AVDF_API int avdf_eval_detection(const avdf_eval_args* a, void* strea
   eval_finish_kernel<<<1, 32 * EVAL_MAX_THR, 0, st>>>(w.blk_sum, n > 0 ? n_blk : 0, a->n_thr, a->n_topk, a->n_gt, w.hits, a->ap,
                                                    a->recall_hits, a->status);
   return check_launch("avdf_eval_detection");
+}
+
+extern "C" AVDF_API size_t avdf_eval_proposal_workspace_bytes(int32_t n_video) {
+  if (n_video < 0) return 0;
+  return prop_layout(nullptr, n_video).bytes;
+}
+
+extern "C" AVDF_API int avdf_eval_proposal(const avdf_eval_proposal_args* a, void* stream) {
+  AVDF_CHECK_ARG(a != nullptr, "args is NULL");
+  AVDF_CHECK_ARG(a->n_thr >= 1 && a->n_thr <= EVAL_MAX_THR, "n_thr must be 1..16");
+  AVDF_CHECK_ARG(a->thresholds != nullptr && a->an_frac != nullptr, "thresholds / an_frac are NULL");
+  for (int t = 0; t < a->n_thr; ++t) AVDF_CHECK_ARG(a->thresholds[t] == a->thresholds[t], "threshold is NaN");
+  for (int j = 0; j < PROP_POINTS; ++j)
+    AVDF_CHECK_ARG(a->an_frac[j] >= 0.0 && a->an_frac[j] <= 1e12 && (j == 0 || a->an_frac[j] >= a->an_frac[j - 1]),
+                   "an_frac must be non-decreasing values in [0, 1e12]");
+  AVDF_CHECK_ARG(a->n_video >= 0 && a->n_prop >= 0 && a->n_gt >= 0, "n_video, n_prop and n_gt must be >= 0");
+  AVDF_CHECK_ARG(a->prop_off && a->gt_off && a->keep, "CSR offsets / keep are NULL");
+  AVDF_CHECK_ARG(a->n_prop == 0 || (a->prop_seg && a->prop_score), "proposal arrays are NULL");
+  AVDF_CHECK_ARG(a->n_gt == 0 || a->gt_seg, "GT segments are NULL");
+  AVDF_CHECK_ARG(a->matches && a->status, "outputs are NULL");
+  AVDF_CHECK_ARG(((uintptr_t)a->prop_seg & 15) == 0 && ((uintptr_t)a->gt_seg & 15) == 0, "segments must be 16-byte aligned");
+  const PropWs need = prop_layout(nullptr, a->n_video);
+  AVDF_CHECK_ARG(a->workspace && a->workspace_bytes >= need.bytes && ((uintptr_t)a->workspace & 255) == 0,
+                 "workspace too small or not 256-byte aligned (avdf_eval_proposal_workspace_bytes)");
+
+  cudaStream_t st = (cudaStream_t)stream;
+  PropWs w = prop_layout((char*)a->workspace, a->n_video);
+  PropParams P = {};
+  for (int t = 0; t < a->n_thr; ++t) P.thr[t] = a->thresholds[t];
+  for (int j = 0; j < PROP_POINTS; ++j) P.frac[j] = a->an_frac[j];
+  P.n_thr = a->n_thr; P.n_video = a->n_video;
+  const double2* seg = reinterpret_cast<const double2*>(a->prop_seg);
+  const double2* gt = reinterpret_cast<const double2*>(a->gt_seg);
+  const int sms = device_sm_count();
+
+  AVDF_CUDA(cudaMemsetAsync(a->status, 0, sizeof(int32_t), st));
+  AVDF_CUDA(cudaMemsetAsync(w.n_unsorted, 0, 4, st));
+  AVDF_CUDA(cudaMemsetAsync(w.hist, 0, 8 * EVAL_MAX_THR * PROP_POINTS, st));
+  eval_validate_kernel<<<(a->n_video + 1 + 255) / 256, 256, 0, st>>>(a->prop_off, a->gt_off, a->n_video, a->n_prop, a->n_gt,
+                                                                     a->status, a->keep);
+  if (a->n_video > 0) {
+    const int grid = (int)std::min<int64_t>((a->n_video + MATCH_WARPS - 1) / MATCH_WARPS, (int64_t)sms * 8);
+    eval_prop_match_kernel<<<grid, MATCH_WARPS * 32, 0, st>>>(P, a->prop_off, seg, a->prop_score, a->keep, a->gt_off, gt,
+                                                             w.unsorted, w.n_unsorted, w.hist, a->status);
+    const size_t smem = (size_t)EVAL_MAX_PRED * (8 + 2);
+    AVDF_SMEM_ATTR_ONCE(eval_prop_match_sorted_kernel, smem);
+    eval_prop_match_sorted_kernel<<<std::min(a->n_video, 2 * sms), SORTV_THREADS, smem, st>>>(
+        P, a->prop_off, seg, a->prop_score, a->keep, a->gt_off, gt, w.unsorted, w.n_unsorted, w.hist, a->status);
+  }
+  eval_prop_finish_kernel<<<1, 32, 0, st>>>(w.hist, a->n_thr, a->matches, a->status);
+  return check_launch("avdf_eval_proposal");
 }

@@ -42,7 +42,8 @@ def _frame(vids, starts, stops, labels):
 
 def load_gt_seg_from_json(json_file, split=None, label="label", label_offset=0):
     """ActivityNet-format ground truth (`database -> video id -> {subset, annotations: [{segment, <label>}]}`) ->
-    DataFrame (video-id, t-start, t-end, label). `split` keeps the videos whose `subset` equals it (case-insensitive)."""
+    DataFrame (video-id, t-start, t-end, label). `split` keeps the videos whose `subset` equals it (case-insensitive).
+    label=None reads no label (every row gets 0): the class-agnostic proposal task, whose labels may be names."""
     with open(json_file, "r", encoding="utf8") as f:
         json_db = json.load(f)["database"]
     vids, starts, stops, labels = [], [], [], []
@@ -53,7 +54,9 @@ def load_gt_seg_from_json(json_file, split=None, label="label", label_offset=0):
             vids.append(k)
             starts.append(float(event["segment"][0]))
             stops.append(float(event["segment"][1]))
-            if isinstance(event[label], (tuple, list)):
+            if label is None:
+                label_id = 0
+            elif isinstance(event[label], (tuple, list)):
                 label_id = 0              # the reference's folding of a label tuple with label_offset
                 for i, x in enumerate(event[label][::-1]):
                     label_id += label_offset ** i + int(x)
@@ -117,6 +120,42 @@ def prediction_columns(preds):
             _np(cols["label"], np.int64), score)
 
 
+def video_codes(vids, rows, gt):
+    """One code per video id: prediction ids first (in order of appearance, so grouped records stay in order), then the
+    ids only GT rows have. -> (code per prediction row, code per GT row, number of codes)."""
+    import pandas as pd
+    codes, _ = pd.factorize(np.concatenate([vids, gt["video-id"].values.astype(object)]))
+    n_codes = int(codes.max()) + 1 if codes.size else 0
+    return np.repeat(codes[:vids.size], rows), codes[vids.size:], n_codes
+
+
+def video_csr(p_code, g_code, n_codes, gt_videos_only=False):
+    """Prediction rows and GT rows (video codes p_code, g_code) -> the CSR of the videos that have GT rows or predictions
+    (gt_videos_only: GT rows), in code order: (p_rows, order, pred_off int64 [V+1], g_rows, gt_off int32 [V+1]).
+    p_rows / g_rows index the inputs in CSR order; predictions of the other videos are left out. The kept rows keep their
+    order inside each video; order is their regrouping permutation (None when they already come grouped)."""
+    present = np.zeros(n_codes, dtype=bool)
+    present[g_code] = True
+    p_rows = np.arange(p_code.size)
+    if gt_videos_only:
+        p_rows = p_rows[present[p_code]]
+    else:
+        present[p_code] = True
+    local = np.cumsum(present) - 1
+    n_video = int(present.sum())
+    p_loc = local[p_code[p_rows]]
+    order = None if (p_loc.size < 2 or (np.diff(p_loc) >= 0).all()) else np.argsort(p_loc, kind="stable")
+    if order is not None:
+        p_rows, p_loc = p_rows[order], p_loc[order]
+    g_loc = local[g_code]
+    g_rows = np.argsort(g_loc, kind="stable")
+    pred_off = np.zeros(n_video + 1, dtype=np.int64)
+    pred_off[1:] = np.cumsum(np.bincount(p_loc, minlength=n_video))
+    gt_off = np.zeros(n_video + 1, dtype=np.int32)
+    gt_off[1:] = np.cumsum(np.bincount(g_loc, minlength=n_video))
+    return p_rows, order, pred_off, g_rows, gt_off
+
+
 class ANETdetection(object):
     """The reference's evaluator. ant_file: ActivityNet-format JSON or AV-Deepfake1M metadata JSON (or a ground-truth
     DataFrame from one of the loaders). num_workers is accepted for compatibility and unused."""
@@ -165,7 +204,6 @@ class ANETdetection(object):
     def evaluate_classes(self, preds, want_tp=False):
         """-> (ap [n_thr, n_cls], recall [n_thr, n_topk, n_cls], tp_mask): tp_mask (want_tp) is a uint16 array over the
         prediction rows in input order, bit t = TP at threshold t within the row's class."""
-        import pandas as pd
         dev = _device()
         vids, rows, t0, t1, label, score = prediction_columns(preds)
         if np.isnan(t0).any() or np.isnan(t1).any() or np.isnan(score).any():
@@ -174,11 +212,7 @@ class ANETdetection(object):
             u, inv = np.unique(label, return_inverse=True)
             label = np.array([self.activity_index.get(int(x), int(x)) for x in u], dtype=np.int64)[inv.reshape(-1)]
         gt = self.ground_truth
-        # one code per video id: prediction ids first (in order of appearance), so grouped records stay in order
-        codes, _ = pd.factorize(np.concatenate([vids, gt["video-id"].values.astype(object)]))
-        n_codes = int(codes.max()) + 1 if codes.size else 0
-        p_code = np.repeat(codes[:vids.size], rows)
-        g_code = codes[vids.size:]
+        p_code, g_code, n_codes = video_codes(vids, rows, gt)
         g_lab = gt["label"].values.astype(np.int64)
         g_se = np.stack([gt["t-start"].values, gt["t-end"].values], 1).astype(np.float64)
         n_thr, n_k, n_cls = len(self.tiou_thresholds), len(self.top_k), len(self.activity_index)
@@ -189,30 +223,17 @@ class ANETdetection(object):
         for c in range(n_cls):
             gsel = np.nonzero(g_lab == c)[0]
             psel = np.nonzero(label == c)[0]
-            present = np.zeros(n_codes, dtype=bool)
-            present[g_code[gsel]] = True
-            present[p_code[psel]] = True
-            local = np.cumsum(present) - 1
-            n_video = int(present.sum())
-            p_loc = local[p_code[psel]]
-            order = None if (p_loc.size < 2 or (np.diff(p_loc) >= 0).all()) else np.argsort(p_loc, kind="stable")
-            rank = None
-            if order is not None:       # rows not grouped by video: the CSR regroups them, equal scores keep the input order
-                psel, p_loc = psel[order], p_loc[order]
-                rank = torch.from_numpy(order.astype(np.int32)).to(dev)
-            g_loc = local[g_code[gsel]]
-            gorder = np.argsort(g_loc, kind="stable")
-            pred_off = np.zeros(n_video + 1, dtype=np.int64)
-            pred_off[1:] = np.cumsum(np.bincount(p_loc, minlength=n_video))
-            gt_off = np.zeros(n_video + 1, dtype=np.int32)
-            gt_off[1:] = np.cumsum(np.bincount(g_loc, minlength=n_video))
+            p_rows, order, pred_off, g_rows, gt_off = video_csr(p_code[psel], g_code[gsel], n_codes)
+            psel = psel[p_rows]
+            # rows not grouped by video: the CSR regroups them, equal scores keep the input order
+            rank = None if order is None else torch.from_numpy(order.astype(np.int32)).to(dev)
             seg = np.stack([t0[psel], t1[psel]], 1)
             tp = torch.empty(psel.size, dtype=torch.uint16, device=dev) if want_tp else None
             if ws is None:
                 ws = torch.empty(ops.nv.lib().avdf_eval_workspace_bytes(score.size, n_codes), dtype=torch.uint8, device=dev)
             a, h, _ = ops.eval_detection(torch.from_numpy(pred_off).to(dev), torch.from_numpy(seg).to(dev),
                                          torch.from_numpy(score[psel]).to(dev), torch.from_numpy(gt_off).to(dev),
-                                         torch.from_numpy(np.ascontiguousarray(g_se[gsel[gorder]])).to(dev),
+                                         torch.from_numpy(np.ascontiguousarray(g_se[gsel[g_rows]])).to(dev),
                                          self.tiou_thresholds, self.top_k, tp_mask=tp, pred_rank=rank, workspace=ws)
             ap[:, c] = a.cpu().numpy()
             recall[:, :, c] = h.cpu().numpy() / float(gsel.size)

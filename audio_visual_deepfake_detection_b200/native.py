@@ -27,6 +27,7 @@ EXPORTS = [
     "avdf_ln_rows", "avdf_instnorm_lrelu", "avdf_fpn_fuse", "avdf_head_final", "avdf_head_combine",
     "avdf_vcls_exp12", "avdf_vcls_exp13", "avdf_host_pack", "avdf_host_all_pinned", "avdf_h2d_gather",
     "avdf_logmel", "avdf_byola_conv1_pool", "avdf_byola_pool", "avdf_eval_workspace_bytes", "avdf_eval_detection",
+    "avdf_eval_proposal_workspace_bytes", "avdf_eval_proposal",
 ]
 
 
@@ -102,8 +103,19 @@ class EvalArgs(Structure):
     ]
 
 
-# status bits of avdf_eval_detection (AVDF_EVAL_*)
-EVAL_PRED_LIMIT, EVAL_GT_LIMIT, EVAL_BAD_OFFSETS = 1, 2, 4
+class EvalProposalArgs(Structure):
+    _fields_ = [
+        ("n_video", c_int32), ("n_prop", c_int64), ("n_gt", c_int32),
+        ("prop_off", c_void_p), ("prop_seg", c_void_p), ("prop_score", c_void_p), ("keep", c_void_p),
+        ("gt_off", c_void_p), ("gt_seg", c_void_p),
+        ("thresholds", POINTER(c_double)), ("n_thr", c_int32), ("an_frac", POINTER(c_double)),
+        ("matches", c_void_p), ("status", c_void_p),
+        ("workspace", c_void_p), ("workspace_bytes", c_size_t),
+    ]
+
+
+# status bits of avdf_eval_detection / avdf_eval_proposal (AVDF_EVAL_*)
+EVAL_PRED_LIMIT, EVAL_GT_LIMIT, EVAL_BAD_OFFSETS, EVAL_BAD_KEEP = 1, 2, 4, 8
 
 _lib = None
 
@@ -155,10 +167,14 @@ def lib():
     L.avdf_eval_workspace_bytes.restype = c_size_t
     L.avdf_eval_workspace_bytes.argtypes = [c_int64, c_int32]
     L.avdf_eval_detection.argtypes = [POINTER(EvalArgs), c_void_p]
+    L.avdf_eval_proposal_workspace_bytes.restype = c_size_t
+    L.avdf_eval_proposal_workspace_bytes.argtypes = [c_int32]
+    L.avdf_eval_proposal.argtypes = [POINTER(EvalProposalArgs), c_void_p]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("avdf_last_error", "avdf_nms_workspace_bytes", "avdf_postprocess_workspace_bytes",
-                        "avdf_conv_gemm_workspace_bytes", "avdf_eval_workspace_bytes", "avdf_abi_version"):
+                        "avdf_conv_gemm_workspace_bytes", "avdf_eval_workspace_bytes", "avdf_eval_proposal_workspace_bytes",
+                        "avdf_abi_version"):
             fn.restype = c_int32
     if L.avdf_abi_version() != 3:
         raise AvdfError("libavdf_sm100.so ABI version mismatch")

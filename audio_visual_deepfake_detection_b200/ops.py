@@ -493,3 +493,49 @@ def eval_detection(pred_off, pred_seg, pred_score, gt_off, gt_seg, thresholds, t
                                   (nv.EVAL_BAD_OFFSETS, "malformed CSR offsets")) if st & b]
             raise nv.AvdfError("avdf_eval_detection: %s (status %d); no results were written" % ("; ".join(why), st))
     return ap, hits, status
+
+
+def eval_proposal(prop_off, prop_seg, prop_score, keep, gt_off, gt_seg, thresholds, an_frac, *, matches=None, workspace=None,
+                  check_status=True):
+    """ActivityNet proposal matches per tIoU threshold and point of the AR-AN curve, videos in CSR form (include/avdf.h
+    avdf_eval_proposal): prop_off int64 [V+1], prop_seg fp64 [N, 2], prop_score fp64 [N], keep int32 [V] (proposals walked
+    per video), gt_off int32 [V+1], gt_seg fp64 [G, 2]; thresholds and an_frac (100 values) host sequences. matches: optional
+    int64 [n_thr, 100] output. Returns (matches, status int32 [1]) on the device; check_status reads the status word (a
+    synchronisation) and raises AvdfError when a per-video check failed (matches was not written)."""
+    L = nv.lib()
+    _chk(prop_off, torch.int64, "prop_off"); _chk(prop_seg, torch.float64, "prop_seg"); _chk(prop_score, torch.float64, "prop_score")
+    _chk(keep, torch.int32, "keep"); _chk(gt_off, torch.int32, "gt_off"); _chk(gt_seg, torch.float64, "gt_seg")
+    _chk(matches, torch.int64, "matches")
+    n, n_video, n_gt = prop_score.numel(), prop_off.numel() - 1, gt_seg.shape[0]
+    assert prop_seg.shape == (n, 2) and gt_seg.shape == (n_gt, 2) and gt_off.numel() == n_video + 1 and keep.numel() == n_video
+    dev = prop_off.device
+    thr = [float(t) for t in thresholds]
+    frac = [float(f) for f in an_frac]
+    assert len(frac) == 100, "an_frac must hold the 100 points of the AR-AN curve"
+    if matches is None:
+        matches = torch.empty((len(thr), 100), dtype=torch.int64, device=dev)
+    assert matches.numel() == len(thr) * 100
+    status = torch.empty(1, dtype=torch.int32, device=dev)
+    need = L.avdf_eval_proposal_workspace_bytes(n_video)
+    if workspace is None or workspace.numel() * workspace.element_size() < need:
+        workspace = torch.empty(need, dtype=torch.uint8, device=dev)
+    a = nv.EvalProposalArgs()
+    a.n_video, a.n_prop, a.n_gt = n_video, n, n_gt
+    a.prop_off, a.keep, a.gt_off = prop_off.data_ptr(), keep.data_ptr(), gt_off.data_ptr()
+    a.prop_seg, a.prop_score = (prop_seg.data_ptr(), prop_score.data_ptr()) if n else (None, None)
+    a.gt_seg = gt_seg.data_ptr() if n_gt else None
+    thr_arr, frac_arr = (ctypes.c_double * max(1, len(thr)))(*thr), (ctypes.c_double * 100)(*frac)
+    a.thresholds, a.n_thr, a.an_frac = thr_arr, len(thr), frac_arr
+    a.matches, a.status = matches.data_ptr(), status.data_ptr()
+    a.workspace, a.workspace_bytes = workspace.data_ptr(), workspace.numel() * workspace.element_size()
+    _call("avdf_eval_proposal", L.avdf_eval_proposal, (ctypes.byref(a), _stream(),), launches=1,
+          work={"bytes": n * (16 + 8) + n_gt * 16})
+    if check_status:
+        st = int(status.item())
+        if st:
+            why = [w for b, w in ((nv.EVAL_PRED_LIMIT, "a video has more than 8192 proposals"),
+                                  (nv.EVAL_GT_LIMIT, "a video has more than 64 ground-truth rows"),
+                                  (nv.EVAL_BAD_OFFSETS, "malformed CSR offsets"),
+                                  (nv.EVAL_BAD_KEEP, "keep is outside 0 .. proposals of its video")) if st & b]
+            raise nv.AvdfError("avdf_eval_proposal: %s (status %d); no results were written" % ("; ".join(why), st))
+    return matches, status

@@ -41,6 +41,7 @@
  *   avdf_vcls_exp12 / _exp13        video-level classifier tails (blocks.py:1608-1626, 1682-1700)
  *   avdf_eval_detection             libs/utils/metrics.py ANETdetection (AP and Recall@kx of one class), the evaluator
  *                                   valid_one_epoch calls (libs/utils/train_utils.py)
+ *   avdf_eval_proposal              libs/utils/Evaluation/eval_proposal.py ANETproposal (ActivityNet AR vs. AN)
  */
 #ifndef AVDF_H_
 #define AVDF_H_
@@ -370,6 +371,37 @@ typedef struct avdf_eval_args {
 } avdf_eval_args;                 /* host struct */
 AVDF_API size_t avdf_eval_workspace_bytes(int64_t n_pred, int32_t n_video);
 AVDF_API int avdf_eval_detection(const avdf_eval_args* args, void* stream);
+
+/* ---- proposal evaluation: ActivityNet average recall vs. average number of proposals (eval_proposal.py
+ * average_recall_vs_avg_nr_proposals, ANETproposal), class-agnostic ----
+ * Videos in CSR form, normally the videos that have GT rows: video v owns proposals [prop_off[v], prop_off[v+1]) and GT rows
+ * [gt_off[v], gt_off[v+1]). Walk order is score descending, ties by smaller row; a video walks its first keep[v] proposals
+ * (the host's min(int(n_p * ratio), n_p)). With c = keep[v], or c = 1 and a tIoU of 0 for a video without proposals, point
+ * j looks at the first cut_j = min(int(c * an_frac[j]), c) proposals (one fp64 product, truncated; an_frac = the host's
+ * 100 pcn values, non-decreasing). matches[t * 100 + j] counts the GT rows with a proposal among those whose tIoU (fp64,
+ * numpy's operation order) is >= thresholds[t]; recall = matches / n_gt. Limits: n_thr <= 16, <= 8192 proposals and <= 64 GT
+ * rows per video, 0 <= keep[v] <= proposals of v; checked on the device: a violation sets bits of *status (AVDF_EVAL_*) and
+ * the call then writes nothing to matches. Integer counts only: bit-identical runs. */
+enum { AVDF_EVAL_BAD_KEEP = 8 };
+typedef struct avdf_eval_proposal_args {
+  int32_t n_video;               /* videos */
+  int64_t n_prop;                /* proposal rows in the CSR */
+  int32_t n_gt;                  /* GT rows */
+  const int64_t* prop_off;       /* [n_video + 1] */
+  const double* prop_seg;        /* [n_prop, 2] (start, end), 16-byte aligned */
+  const double* prop_score;      /* [n_prop] */
+  const int32_t* keep;           /* [n_video] proposals walked per video */
+  const int32_t* gt_off;         /* [n_video + 1] */
+  const double* gt_seg;          /* [n_gt, 2], 16-byte aligned */
+  const double* thresholds;      /* HOST [n_thr] tIoU thresholds */
+  int32_t n_thr;
+  const double* an_frac;         /* HOST [100] */
+  int64_t* matches;              /* [n_thr * 100] */
+  int32_t* status;               /* [1] 0 on success, else AVDF_EVAL_* bits */
+  void* workspace; size_t workspace_bytes;   /* 256-byte aligned */
+} avdf_eval_proposal_args;        /* host struct */
+AVDF_API size_t avdf_eval_proposal_workspace_bytes(int32_t n_video);
+AVDF_API int avdf_eval_proposal(const avdf_eval_proposal_args* args, void* stream);
 
 /* ---- HOST: gather n byte spans (src[i] -> dst[i], nbytes[i] bytes; all HOST pointers, any alignment; dst is normally
  * a slice of a pinned staging buffer) with up to n_threads threads of a pool that lives inside the library
