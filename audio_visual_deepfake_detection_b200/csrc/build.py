@@ -14,7 +14,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["runtime.cu", "interp.cu", "nms.cu", "gemm_simt.cu", "gemm_tc.cu", "mlp_fused.cu", "blocks.cu", "host_pack.cu", "attention_mma.cu", "byola.cu", "eval.cu"]
+SOURCES = ["runtime.cu", "interp.cu", "nms.cu", "gemm_simt.cu", "gemm_tc.cu", "mlp_fused.cu", "blocks.cu", "host_pack.cu", "attention_mma.cu", "byola.cu", "eval.cu", "window.cu"]
 LIB = os.path.join(HERE, "libavdf_sm100.so")
 OBJ_DIR = os.path.join(HERE, "build")
 
@@ -23,7 +23,7 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler",
           "--expt-relaxed-constexpr", "-Xptxas", "-v"]
 # nms.cu restates g++-compiled float code: no fused multiply-add contraction, IEEE div/sqrt; eval.cu restates numpy's fp64
 # segment_iou, whose TP / FP decisions must come out bit-identical
-PER_FILE = {"nms.cu": ["-fmad=false", "-prec-div=true", "-prec-sqrt=true"], "eval.cu": ["-fmad=false"],"gemm_tc.cu": (["-DAVDF_GEMM_TIMELINE"] if os.environ.get("AVDF_GEMM_TIMELINE") else []),
+PER_FILE = {"nms.cu": ["-fmad=false", "-prec-div=true", "-prec-sqrt=true"], "eval.cu": ["-fmad=false"], "window.cu": ["-fmad=false", "-prec-div=true"],"gemm_tc.cu": (["-DAVDF_GEMM_TIMELINE"] if os.environ.get("AVDF_GEMM_TIMELINE") else []),
             "blocks.cu": os.environ.get("AVDF_BLOCKS_FLAGS", "").split()}
 
 

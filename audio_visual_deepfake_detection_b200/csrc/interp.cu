@@ -14,13 +14,17 @@
 // per NEW source row, one 16 B (bf16) or two 16 B (fp32) stores per output row); the threads of a warp are
 // contiguous in C so every access is a fully coalesced 128 B+ line. Algorithmic bytes per video:
 // 4 * sum_s(T_s * C_s) read + T_out * C_total * sizeof(out) written.
+//
+// avdf_interp_concat_ranges runs the same kernel on (start, count) row ranges instead of CSR offsets: the overlapping
+// windows of a long recording (libs/modeling/windows.py) read one device copy of it.
 #include "common.cuh"
 
 namespace avdf {
 
 struct InterpParams {
   const void* src[3];          // packed rows of all videos, per stream: [sum_b T_s(b), C_s], fp32 or bf16 (16-bit feature shards)
-  const int* row_off[3];       // [B+1] prefix offsets (rows) per stream
+  const int* row_off[3];       // [B+1] prefix offsets (rows) per stream, or with row_cnt: [B] first rows
+  const int* row_cnt[3];       // null: CSR (rows of video b = [row_off[b], row_off[b+1])); else [B] row counts
   int c[3];                    // channels per stream (0 = stream absent)
   int c_off[3];                // channel offset in the concatenated output
   int c_total, t_out, B;
@@ -48,7 +52,7 @@ __global__ void __launch_bounds__(256) interp_concat_kernel(const InterpParams p
     const int s = (ch >= p.c_off[2] && p.c[2] > 0) ? 2 : ((ch >= p.c_off[1] && p.c[1] > 0) ? 1 : 0);
     const int cs = ch - p.c_off[s];
     const int r0 = p.row_off[s][b];
-    const int t_in = p.row_off[s][b + 1] - r0;
+    const int t_in = p.row_cnt[s] ? p.row_cnt[s][b] : p.row_off[s][b + 1] - r0;
     const int cstride = p.c[s];
     const InT* base = static_cast<const InT*>(p.src[s]) + (size_t)r0 * cstride + cs;
     OutT* orow = out + ((size_t)b * p.t_out + t_first) * p.c_total + ch;
@@ -139,27 +143,8 @@ extern "C" int avdf_interp_concat(const float* video, const float* byola, const 
                                out, out_dtype, stream);
 }
 
-extern "C" int avdf_interp_concat_in(const void* video, const void* byola, const void* emo, int32_t in_dtype,
-                                     const int32_t* video_off, const int32_t* byola_off, const int32_t* emo_off,
-                                     int32_t batch, int32_t c_video, int32_t c_byola, int32_t c_emo, int32_t t_out,
-                                     void* out, int32_t out_dtype, void* stream) {
-  AVDF_CHECK_ARG(batch >= 0 && t_out > 0, "bad batch / t_out");
-  AVDF_CHECK_ARG(in_dtype == AVDF_DTYPE_F32 || in_dtype == AVDF_DTYPE_BF16, "in_dtype must be F32 or BF16");
-  AVDF_CHECK_ARG(c_video >= 0 && c_byola >= 0 && c_emo >= 0, "negative channel count");
-  AVDF_CHECK_ARG((c_video % 8 | c_byola % 8 | c_emo % 8) == 0, "channel counts must be multiples of 8");
-  AVDF_CHECK_ARG(c_video + c_byola + c_emo > 0, "no stream");
-  AVDF_CHECK_DTYPE(out_dtype, "out_dtype");
-  AVDF_CHECK_ARG((c_video == 0 || (video && video_off)) && (c_byola == 0 || (byola && byola_off)) &&
-                 (c_emo == 0 || (emo && emo_off)), "null stream pointer");
-  AVDF_CHECK_ARG(out != nullptr, "out is null");
-  if (batch == 0) return AVDF_OK;
-  InterpParams p{};
-  p.src[0] = video; p.src[1] = byola; p.src[2] = emo;
-  p.row_off[0] = video_off; p.row_off[1] = byola_off; p.row_off[2] = emo_off;
-  p.c[0] = c_video; p.c[1] = c_byola; p.c[2] = c_emo;
-  p.c_off[0] = 0; p.c_off[1] = c_video; p.c_off[2] = c_video + c_byola;
-  p.c_total = c_video + c_byola + c_emo; p.t_out = t_out; p.B = batch;
-  const long long total = (long long)batch * ((t_out + INTERP_ROWS - 1) / INTERP_ROWS) * (p.c_total / 8);
+static int launch_interp(InterpParams& p, int32_t in_dtype, void* out, int32_t out_dtype, void* stream) {
+  const long long total = (long long)p.B * ((p.t_out + INTERP_ROWS - 1) / INTERP_ROWS) * (p.c_total / 8);
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -173,4 +158,50 @@ extern "C" int avdf_interp_concat_in(const void* video, const void* byola, const
     AVDF_DISPATCH_DTYPE(out_dtype, OutT, (interp_concat_kernel<__nv_bfloat16, OutT><<<grid, 256, 0, st>>>(p, reinterpret_cast<OutT*>(out))));
   }
   return check_launch("interp_concat_kernel");
+}
+
+static int interp_params(InterpParams& p, const void* video, const void* byola, const void* emo, int32_t in_dtype,
+                         int32_t batch, int32_t c_video, int32_t c_byola, int32_t c_emo, int32_t t_out, void* out, int32_t out_dtype) {
+  AVDF_CHECK_ARG(batch >= 0 && t_out > 0, "bad batch / t_out");
+  AVDF_CHECK_ARG(in_dtype == AVDF_DTYPE_F32 || in_dtype == AVDF_DTYPE_BF16, "in_dtype must be F32 or BF16");
+  AVDF_CHECK_ARG(c_video >= 0 && c_byola >= 0 && c_emo >= 0, "negative channel count");
+  AVDF_CHECK_ARG((c_video % 8 | c_byola % 8 | c_emo % 8) == 0, "channel counts must be multiples of 8");
+  AVDF_CHECK_ARG(c_video + c_byola + c_emo > 0, "no stream");
+  AVDF_CHECK_DTYPE(out_dtype, "out_dtype");
+  AVDF_CHECK_ARG((c_video == 0 || video) && (c_byola == 0 || byola) && (c_emo == 0 || emo), "null stream pointer");
+  AVDF_CHECK_ARG(out != nullptr, "out is null");
+  p.src[0] = video; p.src[1] = byola; p.src[2] = emo;
+  p.c[0] = c_video; p.c[1] = c_byola; p.c[2] = c_emo;
+  p.c_off[0] = 0; p.c_off[1] = c_video; p.c_off[2] = c_video + c_byola;
+  p.c_total = c_video + c_byola + c_emo; p.t_out = t_out; p.B = batch;
+  return AVDF_OK;
+}
+
+extern "C" int avdf_interp_concat_in(const void* video, const void* byola, const void* emo, int32_t in_dtype,
+                                     const int32_t* video_off, const int32_t* byola_off, const int32_t* emo_off,
+                                     int32_t batch, int32_t c_video, int32_t c_byola, int32_t c_emo, int32_t t_out,
+                                     void* out, int32_t out_dtype, void* stream) {
+  InterpParams p{};
+  const int rc = interp_params(p, video, byola, emo, in_dtype, batch, c_video, c_byola, c_emo, t_out, out, out_dtype);
+  if (rc != AVDF_OK) return rc;
+  AVDF_CHECK_ARG((c_video == 0 || video_off) && (c_byola == 0 || byola_off) && (c_emo == 0 || emo_off), "null stream pointer");
+  if (batch == 0) return AVDF_OK;
+  p.row_off[0] = video_off; p.row_off[1] = byola_off; p.row_off[2] = emo_off;
+  return launch_interp(p, in_dtype, out, out_dtype, stream);
+}
+
+extern "C" int avdf_interp_concat_ranges(const void* video, const void* byola, const void* emo, int32_t in_dtype,
+                                         const int32_t* start, const int32_t* count,
+                                         int32_t batch, int32_t c_video, int32_t c_byola, int32_t c_emo, int32_t t_out,
+                                         void* out, int32_t out_dtype, void* stream) {
+  InterpParams p{};
+  const int rc = interp_params(p, video, byola, emo, in_dtype, batch, c_video, c_byola, c_emo, t_out, out, out_dtype);
+  if (rc != AVDF_OK) return rc;
+  AVDF_CHECK_ARG(start != nullptr && count != nullptr, "null start / count");
+  if (batch == 0) return AVDF_OK;
+  for (int s = 0; s < 3; ++s) {
+    p.row_off[s] = start + (size_t)s * batch;
+    p.row_cnt[s] = count + (size_t)s * batch;
+  }
+  return launch_interp(p, in_dtype, out, out_dtype, stream);
 }

@@ -17,6 +17,7 @@ and `forward_streams`, which takes the RAW per-stream features and runs the
 dataset-side resampling (libs/datasets/deepfake_video_audio.py:513-547) on the
 GPU as the first kernel of the pass.
 """
+import gc
 from collections import OrderedDict
 
 import numpy as np
@@ -197,22 +198,35 @@ class _LocalizationBase(nn.Module):
         return logits.cpu(), offsets.cpu(), vcls.cpu()
 
     @torch.no_grad()
-    def forward_streams(self, batch):
+    def forward_streams(self, batch, window=None, hop=None):
         """batch: list of dicts {video_id, duration, streams: {'video'?: [T_v,256], 'byola': [T_b,2048],
         'emo': [T_e,768]} fp32 numpy/torch, time-major like the `.npy` files}. Runs the dataset's resampling to
         max_seq_len + concat (deepfake_video_audio.py:513-547) on the GPU, then the model; returns the same list
-        of dicts as forward(). Host buffers in, host tensors out (pinned staging + CUDA graph inside)."""
+        of dicts as forward(). Host buffers in, host tensors out (pinned staging + CUDA graph inside).
+
+        window / hop (seconds, hop defaults to window / 2): recordings longer than `window` are cut into overlapping
+        windows that each run at the model's trained time scale, and their results are merged on the GPU into one
+        result per recording (libs/modeling/windows.py). Recordings no longer than `window` give exactly the
+        result they give without it."""
         runner = self.runner()
+        if window is not None:
+            return runner.run_windows(batch, window, hop)
         out = []
         for i in range(0, len(batch), self.max_batch):
             out.extend(runner.run(batch[i:i + self.max_batch]))
         return out
 
     @torch.no_grad()
-    def stream(self, batches):
+    def stream(self, batches, window=None, hop=None):
         """Pipelined variant for serving loops: `for results in model.stream(iterable_of_batches)` overlaps the
-        host-side packing of batch i+1 with the copies and GPU work of batch i (two pinned staging slots)."""
-        yield from self.runner().stream(batches)
+        host-side packing of batch i+1 with the copies and GPU work of batch i (two pinned staging slots).
+        window / hop: as forward_streams; each batch's recordings are windowed and merged, one result per recording."""
+        if window is None:
+            yield from self.runner().stream(batches)
+            return
+        runner = self.runner()
+        for chunk in batches:
+            yield runner.run_windows(chunk, window, hop)
 
     def runner(self):
         if getattr(self, "_runner", None) is None or self._runner.eng is not self.engine():
@@ -278,7 +292,10 @@ class _LocalizationBase(nn.Module):
         eng.lane = lane
         B, L = staged["B"], eng.max_seq_len
         x = eng.buf("x_in_%d" % L, (B, L, eng.c_in), eng.in_dt)
-        ops.interp_concat(staged["streams"], staged["offs"], L, x)
+        if staged.get("ranges") is not None:      # sliding windows: (start, count) [3, B] rows into the group's staging
+            ops.interp_concat_ranges(staged["streams"], *staged["ranges"], L, x)
+        else:
+            ops.interp_concat(staged["streams"], staged["offs"], L, x)
         logits, offsets, vcls, masks, lens = eng.forward_dense(x, [L] * B)
         rec = staged.get("records")      # (ring, counter): result records for the multi-GPU gather, written by the kernel
         if rec is not None:
@@ -306,12 +323,19 @@ class _LocalizationBase(nn.Module):
         # may call the CUDA allocator while this thread records; in the default global mode that invalidates the capture
         eng = self.engine()
         eng._capture_refs = []
+        # no cyclic garbage collection while recording: collecting a discarded model frees its captured graphs, a call
+        # this thread may not make during a capture (it invalidates the capture)
+        gc_on = gc.isenabled()
+        gc.collect()
+        gc.disable()
         try:
             with torch.cuda.graph(graph, capture_error_mode="thread_local"):
                 res = self.run_staged(staged, lane)
             keep = eng._capture_refs
         finally:
             eng._capture_refs = None
+            if gc_on:
+                gc.enable()
         return GraphedPass(graph, res, native.LAUNCHES["n"] - n0, staged, keep)
 
     @staticmethod

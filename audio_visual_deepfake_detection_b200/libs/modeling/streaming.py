@@ -20,7 +20,7 @@ import threading
 import numpy as np
 import torch
 
-from ... import native
+from ... import native, ops
 
 STREAMS = ("video", "byola", "emo")
 
@@ -279,6 +279,178 @@ class StreamRunner:
         empty_labels = torch.zeros(segs.shape[1], dtype=torch.long)
         return [{"video_id": vid, "segments": segs[b, :n], "scores": scores[b, :n], "labels": empty_labels[:n],
                  "video_cls": vcls[b:b + 1]} for b, (vid, n) in enumerate(zip(slot.ids, counts))]
+
+    # ---------------------------------------------------------------- sliding windows (libs/modeling/windows.py)
+    # A group of recordings is copied to the device ONCE (one pinned pack, one copy per stream); its windows - and its
+    # recordings no longer than the window, as single windows - are packed in order into batches of max_batch that
+    # read their rows through avdf_interp_concat_ranges, full batches by replaying a captured graph. Every window's
+    # result is copied aside on the device, and avdf_window_merge turns them into one result (and optionally one
+    # record) per recording. The only host synchronisation of a group is the final copy of its results.
+    GROUP_BYTES = 1 << 30             # raw-stream bytes per group (at least one recording): bounds the pinned / device staging
+
+    def run_windows(self, items, window, hop=None, feat_stride=1, num_frames=1):
+        from ...native import AvdfError
+        from .windows import check_window
+        check_window(window, hop)
+        if self.model.test_nms_method == "none":
+            raise AvdfError("nms_method 'none' returns every decoded candidate: windows need hard or soft NMS to merge")
+        for c in items:
+            if "streams" not in c:
+                raise AvdfError("sliding windows need raw streams; 'feats' items are already resampled to max_seq_len")
+        out, group, nbytes = [], [], 0
+        for c in items:
+            b = sum(np.asarray(a).nbytes if not torch.is_tensor(a) else a.numel() * a.element_size() for a in c["streams"].values())
+            if group and nbytes + b > self.GROUP_BYTES:
+                out.extend(self._run_group(group, window, hop, feat_stride, num_frames))
+                group, nbytes = [], 0
+            group.append(c)
+            nbytes += b
+        if group:
+            out.extend(self._run_group(group, window, hop, feat_stride, num_frames))
+        return out
+
+    def _win_stage(self, rows, chans, dtype, device):
+        """Group staging, grown x1.5 when a group does not fit; growing drops the graphs that captured the old buffers."""
+        if not hasattr(self, "win_cap"):
+            self.win_cap, self.win_host, self.win_dev, self.win_graphs = [0, 0, 0], [None] * 3, [None] * 3, {}
+        for s in range(3):
+            if chans[s] == 0:
+                continue
+            t = self.win_host[s]
+            if t is None or rows[s] > self.win_cap[s] or t.dtype != dtype or t.shape[1] != chans[s]:
+                self.win_cap[s] = max(rows[s], int(self.win_cap[s] * 1.5)) + 64
+                self.win_host[s] = torch.empty((self.win_cap[s], chans[s]), dtype=dtype, pin_memory=True)
+                self.win_dev[s] = torch.empty((self.win_cap[s], chans[s]), dtype=dtype, device=device)
+                self.win_graphs.clear()
+
+    def _run_group(self, items, window, hop, feat_stride, num_frames):
+        from .windows import window_meta, window_plan
+        eng, L, MB = self.eng, self.eng.max_seq_len, self.eng.max_batch
+        K = int(self.model.test_max_seg_num)
+        present = [n in items[0]["streams"] for n in STREAMS]
+        arrs = [[np.ascontiguousarray(_stream_array(c["streams"][n])) for c in items] if p else None for n, p in zip(STREAMS, present)]
+        np_dt = next(al[0].dtype for al in arrs if al)
+        item = np_dt.itemsize
+        chans = [al[0].shape[1] if al else 0 for al in arrs]
+        if sum(chans) != eng.c_in:
+            raise ValueError("streams carry %d channels, the model expects %d" % (sum(chans), eng.c_in))
+        for al in arrs:
+            for a in al or ():
+                if a.dtype != np_dt:
+                    raise ValueError("a batch mixes fp32 streams and 16-bit shards")
+        rows = [sum(a.shape[0] for a in al) if al else 0 for al in arrs]
+        first = 0 if present[0] else 1
+        # ---- plan: one unit per window (a recording no longer than the window is one unit with its own meta)
+        rec_win, starts, counts, metas, s_k = [0], [], [], [], []
+        base = [0, 0, 0]
+        for r, c in enumerate(items):
+            lens = [al[r].shape[0] if al else None for al in arrs]
+            plan = window_plan(c["duration"], lens, window, hop)
+            for s0, rng in plan:
+                starts.append([base[s] + a for s, (a, _) in enumerate(rng)])
+                counts.append([m for _, m in rng])
+                metas.append(video_meta(c, lens[first], L, feat_stride, num_frames) if len(plan) == 1
+                             else window_meta(rng[first][1], window, L, feat_stride, num_frames))
+                s_k.append(np.float32(s0))
+            rec_win.append(len(starts))
+            base = [b + (l or 0) for b, l in zip(base, lens)]
+        n_units, R = len(starts), len(items)
+        slot = self.slots[0]                     # lane 0 and its stream: the window batches run one after the other
+        with torch.cuda.device(eng.device):
+            if slot.busy:
+                self._collect(slot)
+            with self.cuda_lock:
+                self._win_stage(rows, chans, torch.float32 if item == 4 else torch.bfloat16, eng.device)
+            # ---- pack the group's rows once (library thread pool), then one host -> device copy per stream
+            src, dst, nb = [], [], []
+            for s in range(3):
+                if arrs[s] is None:
+                    continue
+                hb, row_bytes, off = self.win_host[s].data_ptr(), chans[s] * item, 0
+                for a in arrs[s]:
+                    if a.shape[1] != chans[s]:
+                        raise ValueError("stream %s: recordings differ in channel count" % STREAMS[s])
+                    src.append(a.ctypes.data); dst.append(hb + off * row_bytes); nb.append(a.nbytes)
+                    off += a.shape[0]
+            n = len(src)
+            native.check(native.lib().avdf_host_pack((ctypes.c_void_p * n)(*src), (ctypes.c_void_p * n)(*dst),
+                                                     (ctypes.c_size_t * n)(*nb), n, self.n_threads), "avdf_host_pack")
+            # per-batch (start [3, b], count [3, b], meta [4, b]) blocks, one after the other, in one pinned buffer
+            batches = [(u, min(MB, n_units - u)) for u in range(0, n_units, MB)]
+            par = np.zeros(10 * n_units, np.float32)
+            for u0, b in batches:
+                blk = par[10 * u0: 10 * (u0 + b)]
+                blk[:6 * b].view(np.int32)[:] = np.concatenate([np.asarray(starts[u0:u0 + b], np.int32).T,
+                                                                np.asarray(counts[u0:u0 + b], np.int32).T]).reshape(-1)
+                blk[6 * b:] = np.asarray(metas[u0:u0 + b], np.float32).T.reshape(-1)
+            h_par = torch.from_numpy(par).pin_memory()
+            h_idx = torch.tensor(rec_win + [int(c.get("index", r)) for r, c in enumerate(items)], dtype=torch.int32).pin_memory()
+            h_start = torch.from_numpy(np.asarray(s_k, np.float32)).pin_memory()
+            slot.stream.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(slot.stream):
+                for s in range(3):
+                    if chans[s]:
+                        self.win_dev[s][:rows[s]].copy_(self.win_host[s][:rows[s]], non_blocking=True)
+                d_par = h_par.to(eng.device, non_blocking=True)
+                d_idx = h_idx.to(eng.device, non_blocking=True)
+                d_start = h_start.to(eng.device, non_blocking=True)
+                self.h2d_bytes += sum(rows[s] * chans[s] * item for s in range(3)) + 4 * (par.size + h_idx.numel() + n_units)
+                w_segs = torch.empty((n_units, K, 2), dtype=torch.float32, device=eng.device)
+                w_scores = torch.empty((n_units, K), dtype=torch.float32, device=eng.device)
+                w_count = torch.empty((n_units,), dtype=torch.int32, device=eng.device)
+                w_cls = torch.empty((n_units,), dtype=torch.float32, device=eng.device)
+                streams = [self.win_dev[s] if chans[s] else None for s in range(3)]
+                for u0, b in batches:
+                    blk = d_par[10 * u0: 10 * (u0 + b)]
+                    ranges = (blk[:6 * b].view(torch.int32)[:3 * b].view(3, b), blk[:6 * b].view(torch.int32)[3 * b:].view(3, b))
+                    meta = blk[6 * b:].view(4, b)
+                    if self.use_graph and b == MB:
+                        key = (b, self.model.test_key(), item)
+                        g = self.win_graphs.get(key)
+                        if g is None:
+                            fixed = {"start": torch.empty((3, b), dtype=torch.int32, device=eng.device),
+                                     "count": torch.empty((3, b), dtype=torch.int32, device=eng.device),
+                                     "meta": torch.empty((4, b), dtype=torch.float32, device=eng.device)}
+                            fixed["start"].copy_(ranges[0]); fixed["count"].copy_(ranges[1]); fixed["meta"].copy_(meta)
+                            staged = {"ids": [None] * b, "B": b, "meta": fixed["meta"], "streams": streams, "offs": None,
+                                      "ranges": (fixed["start"], fixed["count"])}
+                            with self.cuda_lock:
+                                g = self.model.capture(staged, lane=slot.index)
+                            self.win_graphs[key] = g
+                        st = g.staged
+                        st["ranges"][0].copy_(ranges[0], non_blocking=True)
+                        st["ranges"][1].copy_(ranges[1], non_blocking=True)
+                        st["meta"].copy_(meta, non_blocking=True)
+                        res = g.replay()
+                    else:
+                        staged = {"ids": [None] * b, "B": b, "meta": meta, "streams": streams, "offs": None, "ranges": ranges}
+                        res = self.model.run_staged(staged, lane=slot.index)
+                    w_segs[u0:u0 + b].copy_(res["segs"], non_blocking=True)
+                    w_scores[u0:u0 + b].copy_(res["scores"], non_blocking=True)
+                    w_count[u0:u0 + b].copy_(res["counts"], non_blocking=True)
+                    w_cls[u0:u0 + b].copy_(res["vcls"], non_blocking=True)
+                # ---- merge: one result per recording
+                cap = K * max(rec_win[r + 1] - rec_win[r] for r in range(R))
+                o_segs = torch.empty((R, K, 2), dtype=torch.float32, device=eng.device)
+                o_scores = torch.empty((R, K), dtype=torch.float32, device=eng.device)
+                o_count = torch.empty((R,), dtype=torch.int32, device=eng.device)
+                o_cls = torch.empty((R,), dtype=torch.float32, device=eng.device)
+                m = self.model
+                rec = None if self.records is None else (self.records[0], self.records[1], d_idx[R + 1:])
+                ops.window_merge(d_idx[:R + 1], d_start, w_segs, w_scores, w_count, w_cls, cand_cap=cap,
+                                 iou_threshold=m.test_iou_threshold, min_score=m.test_min_score, sigma=m.test_nms_sigma,
+                                 voting_thresh=0.0 if m.test_multiclass_nms else m.test_voting_thresh,
+                                 use_soft_nms=m.test_nms_method == "soft", out_segs=o_segs, out_scores=o_scores,
+                                 out_count=o_count, out_cls=o_cls, records=rec)
+                res = [t.to("cpu", non_blocking=True) for t in (o_segs, o_scores, o_count, o_cls)]
+                self.d2h_bytes += R * (3 * K + 2) * 4
+                done = torch.cuda.Event()
+                done.record()
+            done.synchronize()
+        segs, scores, cnt, vcls = res
+        empty_labels = torch.zeros(K, dtype=torch.long)
+        return [{"video_id": c["video_id"], "segments": segs[r, :int(cnt[r])], "scores": scores[r, :int(cnt[r])],
+                 "labels": empty_labels[:int(cnt[r])], "video_cls": vcls[r:r + 1]} for r, c in enumerate(items)]
 
     # ---------------------------------------------------------------- public
     def run(self, chunk):

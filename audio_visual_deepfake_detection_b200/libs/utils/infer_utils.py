@@ -110,13 +110,17 @@ def valid_one_epoch(val_loader, model, curr_epoch, ext_score_file=None, evaluato
     return mAP
 
 
-def inference_sharded(dataset, model, output_folder, batch_size=32, rank=0, world=1, print_freq=0):
+def inference_sharded(dataset, model, output_folder, batch_size=32, rank=0, world=1, print_freq=0, window=None, hop=None):
     """Multi-GPU form of inference_one_epoch: one process per GPU (torchrun), rank r takes videos r, r + world, ... of the
     dataset (the reference splits its list into 7 files run as 7 processes, libs/datasets/deepfake_video_audio.py:420-431,
     inference.py:116-124); each rank streams its shard through `model.stream` (pinned staging, H2D, CUDA graph), the
     postprocess kernel appends one fixed-size record per video to a device ring, and ONE all-gather of those records
     (NCCL) is the path's only exchange. Rank 0 writes `data_left.json` in dataset order, exactly the records
-    inference_one_epoch writes for the same list. Returns the records on rank 0, None elsewhere."""
+    inference_one_epoch writes for the same list. Returns the records on rank 0, None elsewhere.
+
+    window / hop (seconds): recordings longer than `window` run as overlapping windows merged on the GPU
+    (model.forward_streams(..., window, hop)); still one record per recording. Per-window metadata uses the dataset's
+    feat_stride / num_frames."""
     from .sharding import gather_records, shard_indices, unpack_records
     model.eval()
     n = len(dataset)
@@ -135,9 +139,14 @@ def inference_sharded(dataset, model, output_folder, batch_size=32, rank=0, worl
                 item["index"] = j
                 chunk.append(item)
             yield chunk
+    if window is None:
+        outs = model.stream(batches())
+    else:
+        fs, nf = getattr(dataset, "feat_stride", 1), getattr(dataset, "num_frames", 1)
+        outs = (runner.run_windows(chunk, window, hop, fs, nf) for chunk in batches())
     done = 0
     try:
-        for out in model.stream(batches()):
+        for out in outs:
             done += len(out)
             if print_freq and rank == 0 and (done // batch_size) % print_freq == 0:
                 print("Test: [{0:05d}/{1:05d}]".format(done, len(mine)))

@@ -27,7 +27,8 @@ EXPORTS = [
     "avdf_ln_rows", "avdf_instnorm_lrelu", "avdf_fpn_fuse", "avdf_head_final", "avdf_head_combine",
     "avdf_vcls_exp12", "avdf_vcls_exp13", "avdf_host_pack", "avdf_host_all_pinned", "avdf_h2d_gather",
     "avdf_logmel", "avdf_byola_conv1_pool", "avdf_byola_pool", "avdf_eval_workspace_bytes", "avdf_eval_detection",
-    "avdf_eval_proposal_workspace_bytes", "avdf_eval_proposal",
+    "avdf_eval_proposal_workspace_bytes", "avdf_eval_proposal", "avdf_interp_concat_ranges",
+    "avdf_window_merge_workspace_bytes", "avdf_window_merge",
 ]
 
 
@@ -50,6 +51,19 @@ class PostprocessArgs(Structure):
         ("workspace", c_void_p), ("workspace_bytes", c_size_t),
         ("rec_ring", c_void_p), ("rec_counter", c_void_p), ("rec_cap", c_int32), ("vid_index", c_void_p), ("vid_cls", c_void_p),
         ("out_index", c_void_p),
+    ]
+
+
+class WindowMergeArgs(Structure):
+    _fields_ = [
+        ("n_rec", c_int32), ("rec_win", c_void_p), ("win_start", c_void_p),
+        ("win_segs", c_void_p), ("win_scores", c_void_p), ("win_count", c_void_p), ("win_cls", c_void_p),
+        ("cand_cap", c_int32),
+        ("iou_threshold", c_float), ("min_score", c_float), ("sigma", c_float), ("voting_thresh", c_float),
+        ("max_seg_num", c_int32), ("use_soft_nms", c_int32),
+        ("out_segs", c_void_p), ("out_scores", c_void_p), ("out_count", c_void_p), ("out_cls", c_void_p),
+        ("workspace", c_void_p), ("workspace_bytes", c_size_t),
+        ("rec_ring", c_void_p), ("rec_counter", c_void_p), ("rec_cap", c_int32), ("vid_index", c_void_p),
     ]
 
 
@@ -135,6 +149,10 @@ def lib():
     L.avdf_device_info.argtypes = [POINTER(c_int32)] * 3
     L.avdf_interp_concat.argtypes = [c_void_p] * 6 + [c_int32] * 5 + [c_void_p, c_int32, c_void_p]
     L.avdf_interp_concat_in.argtypes = [c_void_p] * 3 + [c_int32] + [c_void_p] * 3 + [c_int32] * 5 + [c_void_p, c_int32, c_void_p]
+    L.avdf_interp_concat_ranges.argtypes = [c_void_p] * 3 + [c_int32] + [c_void_p] * 2 + [c_int32] * 5 + [c_void_p, c_int32, c_void_p]
+    L.avdf_window_merge_workspace_bytes.restype = c_size_t
+    L.avdf_window_merge_workspace_bytes.argtypes = [c_int32, c_int32]
+    L.avdf_window_merge.argtypes = [POINTER(WindowMergeArgs), c_void_p]
     L.avdf_pack_feats.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_void_p]
     L.avdf_nms_workspace_bytes.restype = c_size_t
     L.avdf_nms_workspace_bytes.argtypes = [c_int32]
@@ -174,7 +192,7 @@ def lib():
         fn = getattr(L, name)
         if name not in ("avdf_last_error", "avdf_nms_workspace_bytes", "avdf_postprocess_workspace_bytes",
                         "avdf_conv_gemm_workspace_bytes", "avdf_eval_workspace_bytes", "avdf_eval_proposal_workspace_bytes",
-                        "avdf_abi_version"):
+                        "avdf_window_merge_workspace_bytes", "avdf_abi_version"):
             fn.restype = c_int32
     if L.avdf_abi_version() != 3:
         raise AvdfError("libavdf_sm100.so ABI version mismatch")

@@ -108,6 +108,29 @@ def interp_concat(streams, offsets, t_out, out):
     return out
 
 
+def interp_concat_ranges(streams, start, count, t_out, out):
+    """Row-range form of interp_concat: video b of stream s is rows [start[s, b], start[s, b] + count[s, b]) of
+    streams[s]; start / count: int32 [3, B] device tensors (rows of absent streams are ignored). Overlapping ranges
+    read the same source rows: the windows of one recording share its one device copy."""
+    L = nv.lib()
+    cs = [0 if s is None else s.shape[1] for s in streams]
+    in_dt = next(s.dtype for s in streams if s is not None)
+    if in_dt not in (torch.float32, torch.bfloat16):
+        raise TypeError("streams must be fp32 or bf16")
+    for s in streams:
+        if s is not None:
+            _chk(s, in_dt, "stream")
+    _chk(start, torch.int32, "start"); _chk(count, torch.int32, "count"); _chk(out, None, "out")
+    batch = start.shape[1]
+    assert start.shape == (3, batch) and count.shape == (3, batch), (start.shape, count.shape)
+    assert out.shape == (batch, t_out, sum(cs)), (out.shape, batch, t_out, cs)
+    _call("avdf_interp_concat_ranges", L.avdf_interp_concat_ranges,
+          (nv.ptr(streams[0]), nv.ptr(streams[1]), nv.ptr(streams[2]), DTYPE_F32 if in_dt == torch.float32 else DTYPE_BF16,
+           nv.ptr(start), nv.ptr(count), batch, cs[0], cs[1], cs[2], t_out, nv.ptr(out), _dt(out), _stream(),),
+          launches=1, work=None)
+    return out
+
+
 def pack_feats(feats_ct, out):
     """feats_ct [C, T] fp32 (device) -> out [L, C] token-major, zero-padded rows T..L."""
     L = nv.lib()
@@ -191,6 +214,41 @@ def postprocess(batch, *, logits=None, offsets=None, mask=None, level_len=(), le
             workspace = torch.empty(need, dtype=torch.uint8, device=out_segs.device)
         a.workspace, a.workspace_bytes = workspace.data_ptr(), need
     _call("avdf_postprocess", L.avdf_postprocess, (ctypes.byref(a), _stream(),), launches=1, work=None)
+
+
+def window_merge(rec_win, win_start, win_segs, win_scores, win_count, win_cls, *, cand_cap, iou_threshold, min_score, sigma,
+                 voting_thresh, use_soft_nms, out_segs, out_scores, out_count, out_cls, workspace=None, records=None):
+    """Cross-window merge (csrc/window.cu): rec_win int32 [R+1] windows per recording (CSR), win_start fp32 [W] seconds,
+    window outputs win_segs [W, K, 2] / win_scores [W, K] / win_count [W] / win_cls [W] -> out_* [R, ...].
+    records: optional (ring [cap, 3 + 3K] f32, counter [1] i32, vid_index [R] i32)."""
+    L = nv.lib()
+    a = nv.WindowMergeArgs()
+    R = rec_win.numel() - 1
+    K = win_scores.shape[1]
+    for t, dt, name in ((rec_win, torch.int32, "rec_win"), (win_start, torch.float32, "win_start"), (win_segs, torch.float32, "win_segs"),
+                        (win_scores, torch.float32, "win_scores"), (win_count, torch.int32, "win_count"), (win_cls, torch.float32, "win_cls"),
+                        (out_segs, torch.float32, "out_segs"), (out_scores, torch.float32, "out_scores"),
+                        (out_count, torch.int32, "out_count"), (out_cls, torch.float32, "out_cls")):
+        _chk(t, dt, name)
+    a.n_rec, a.rec_win, a.win_start = R, rec_win.data_ptr(), win_start.data_ptr()
+    a.win_segs, a.win_scores, a.win_count, a.win_cls = win_segs.data_ptr(), win_scores.data_ptr(), win_count.data_ptr(), win_cls.data_ptr()
+    a.cand_cap = int(cand_cap)
+    a.iou_threshold, a.min_score, a.sigma, a.voting_thresh = float(iou_threshold), float(min_score), float(sigma), float(voting_thresh)
+    a.max_seg_num, a.use_soft_nms = K, int(bool(use_soft_nms))
+    a.out_segs, a.out_scores, a.out_count, a.out_cls = out_segs.data_ptr(), out_scores.data_ptr(), out_count.data_ptr(), out_cls.data_ptr()
+    if records is not None:
+        ring, counter, vidx = records
+        _chk(ring, torch.float32, "rec_ring"); _chk(counter, torch.int32, "rec_counter"); _chk(vidx, torch.int32, "vid_index")
+        if ring.shape[1] != 3 + 3 * K:
+            raise ValueError("record rows must hold 3 + 3 * max_seg_num floats")
+        a.rec_ring, a.rec_counter, a.rec_cap = ring.data_ptr(), counter.data_ptr(), ring.shape[0]
+        a.vid_index = vidx.data_ptr() if vidx is not None else None
+    need = L.avdf_window_merge_workspace_bytes(R, a.cand_cap)
+    if need and (workspace is None or workspace.numel() * workspace.element_size() < need):
+        workspace = torch.empty(need, dtype=torch.uint8, device=out_segs.device)
+    if need:
+        a.workspace, a.workspace_bytes = workspace.data_ptr(), need
+    _call("avdf_window_merge", L.avdf_window_merge, (ctypes.byref(a), _stream(),), launches=3, work=None)
 
 
 def postprocess_workspace_bytes(batch, cand_cap):

@@ -20,6 +20,8 @@
  *                                   postprocessing) + libs/utils/nms.py:8-190 (NMSop, SoftNMSop,
  *                                   seg_voting, batched_nms)
  *   avdf_interp_concat              libs/datasets/deepfake_video_audio.py:513-547 (F.interpolate x3 + cat)
+ *   avdf_interp_concat_ranges,      new: sliding windows over recordings longer than the training clips (the same
+ *   avdf_window_merge               resampling on row ranges; the windows' results merged with batched_nms)
  *   avdf_host_pack                  HOST: DataLoader collate + pin of the raw stream arrays,
  *                                   libs/datasets/deepfake_video_audio.py:547-558 (dataset item) and the
  *                                   per-video `.to(device)` of libs/modeling/av_fd_no_recon.py:476-477
@@ -89,6 +91,16 @@ AVDF_API int avdf_interp_concat_in(const void* video, const void* byola, const v
                           int32_t batch, int32_t c_video, int32_t c_byola, int32_t c_emo, int32_t t_out,
                           void* out, int32_t out_dtype, void* stream);
 
+/* Row-range form (sliding windows over long recordings): video b of stream s is rows [start[s*batch + b],
+ * start[s*batch + b] + count[s*batch + b]) of that stream's packed source; start / count are device int32 [3, batch]
+ * (rows of absent streams are ignored). Windows may overlap and share rows, so overlapping windows of one recording
+ * read one device copy of it. Every count must be >= 1 and every range inside the source. The arithmetic is
+ * avdf_interp_concat's: a range equal to a video's CSR rows gives the same bits. */
+AVDF_API int avdf_interp_concat_ranges(const void* video, const void* byola, const void* emo, int32_t in_dtype,
+                              const int32_t* start, const int32_t* count,
+                              int32_t batch, int32_t c_video, int32_t c_byola, int32_t c_emo, int32_t t_out,
+                              void* out, int32_t out_dtype, void* stream);
+
 /* ---- preprocessing (av_fd_no_recon.py:431-479): one video's feats [channels, t] fp32 (dataset item layout)
  * -> token-major rows out[t_padded, channels], zero-padded from t to t_padded. */
 AVDF_API int avdf_pack_feats(const float* feats_ct, int32_t channels, int32_t t, int32_t t_padded, void* out,
@@ -152,6 +164,36 @@ typedef struct avdf_postprocess_args {
 } avdf_postprocess_args;          /* host struct */
 AVDF_API size_t avdf_postprocess_workspace_bytes(int32_t batch, int32_t cand_cap);
 AVDF_API int avdf_postprocess(const avdf_postprocess_args* args, void* stream);
+
+/* ---- cross-window merge of the sliding-window path (csrc/window.cu) ----
+ * Recording r owns window rows [rec_win[r], rec_win[r+1]) of the window outputs (the per-window postprocess results:
+ * seconds within the window, sorted, win_count[w] <= max_seg_num of them). For a recording with more than one window:
+ * candidates = fp32(win_start[w]) + segment (round to nearest) over its windows in ascending order, each window's
+ * segments in output order; then the class-agnostic batched_nms of libs/utils/nms.py over that list (hard, or soft
+ * method 2; seg_voting over the whole list when voting_thresh > 0, in the summation order of oracle/nms_ref.c; stable
+ * sort by score; cap at max_seg_num); out_cls = max window logit. A recording with one window gets that window's
+ * output unchanged. All of it is three launches on `stream`, no host synchronisation. Optional records: one row per
+ * recording in the avdf_postprocess record layout. cand_cap >= max windows per recording * max_seg_num. */
+typedef struct avdf_window_merge_args {
+  int32_t n_rec;
+  const int32_t* rec_win;        /* [n_rec + 1] device */
+  const float* win_start;        /* [n_win] window start, seconds (fp32) */
+  const float* win_segs;         /* [n_win, max_seg_num, 2] */
+  const float* win_scores;       /* [n_win, max_seg_num] */
+  const int32_t* win_count;      /* [n_win] */
+  const float* win_cls;          /* [n_win] video-level logit of every window */
+  int32_t cand_cap;
+  float iou_threshold, min_score, sigma, voting_thresh;
+  int32_t max_seg_num, use_soft_nms;   /* 0 hard, 1 soft */
+  float* out_segs;               /* [n_rec, max_seg_num, 2] */
+  float* out_scores;             /* [n_rec, max_seg_num] */
+  int32_t* out_count;            /* [n_rec] */
+  float* out_cls;                /* [n_rec] */
+  void* workspace; size_t workspace_bytes;   /* avdf_window_merge_workspace_bytes(n_rec, cand_cap) */
+  float* rec_ring; uint32_t* rec_counter; int32_t rec_cap; const int32_t* vid_index;   /* optional, as avdf_postprocess */
+} avdf_window_merge_args;        /* host struct */
+AVDF_API size_t avdf_window_merge_workspace_bytes(int32_t n_rec, int32_t cand_cap);
+AVDF_API int avdf_window_merge(const avdf_window_merge_args* args, void* stream);
 
 /* ---- conv-as-GEMM with fused epilogue ----
  * out[b, seg_o_row + t, n] = epi( sum_{j<taps} sum_{c<c_in} W[n, j*c_in + c] * A[b, seg_a_row + stride*t + j - taps/2, c] )

@@ -8,6 +8,10 @@ loads the yaml with the reference's DEFAULTS merge, builds the inference dataset
 `module.` keys accepted) and writes `<ckpt dir>/<sub_index>/data_left*.json` exactly like inference_one_epoch does.
 New: `-b` videos per model call (default 32; the reference is fixed to 1) and `--merge` to also write the challenge's
 prediction.txt / prediction.json (generate_results.ipynb) for this shard.
+`--window SEC [--hop SEC]` (hop defaults to window / 2): recordings longer than SEC seconds run as overlapping windows at
+the model's trained time scale, merged into one result per recording on the GPU (libs/modeling/windows.py); such runs
+always go through inference_sharded, single-process and torchrun alike. The window is a user choice: no setting of it
+has been validated for detection quality.
 
 Multi-GPU: launched under torchrun, one process per GPU,
 
@@ -57,8 +61,9 @@ def main(args):
     model.to(device).eval()
     out_dir = os.path.join(os.path.dirname(args.ckpt), str(args.sub_index))
     start = time.time()
-    if world > 1:
-        inference_sharded(dataset, model, out_dir, batch_size=args.batch, rank=rank, world=world, print_freq=args.print_freq)
+    if world > 1 or args.window is not None:
+        inference_sharded(dataset, model, out_dir, batch_size=args.batch, rank=rank, world=world, print_freq=args.print_freq,
+                          window=args.window, hop=args.hop)
     else:
         inference_one_epoch(loader, model, -1, output_folder=out_dir, print_freq=args.print_freq, dataset_name=cfg["dataset_name"])
     if rank == 0:
@@ -80,4 +85,6 @@ if __name__ == "__main__":
     parser.add_argument("-p", "--print-freq", default=10, type=int, help="print frequency")
     parser.add_argument("-b", "--batch", default=32, type=int, help="videos per model call")
     parser.add_argument("--merge", action="store_true", help="also write prediction.txt / prediction.json for this shard")
+    parser.add_argument("--window", type=float, default=None, help="sliding window (seconds) for recordings longer than it")
+    parser.add_argument("--hop", type=float, default=None, help="hop between windows (seconds, default: window / 2)")
     main(parser.parse_args())
