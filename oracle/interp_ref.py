@@ -26,11 +26,12 @@ import numpy as np
 f32 = np.float32
 
 
-def linear_resize_tc(x_tc: np.ndarray, t_out: int) -> np.ndarray:
-    """[T_in, C] -> [t_out, C] (time-major in and out)."""
+def linear_resize_tc(x_tc: np.ndarray, t_out: int, out_dtype=f32) -> np.ndarray:
+    """[T_in, C] -> [t_out, C] (time-major in and out). out_dtype=np.float64: the same fp32 index / weight math, the
+    blend l0 * x[i0] + l1 * x[i1] exact in float64 (no fp32 rounding of the product or the sum)."""
     t_in = x_tc.shape[0]
     if t_in == t_out:
-        return x_tc.astype(f32, copy=True)
+        return x_tc.astype(out_dtype, copy=True)
     scale = f32(t_in) / f32(t_out)
     t = np.arange(t_out, dtype=f32)
     src = (np.float64(scale) * np.float64(t + f32(0.5)) - 0.5).astype(f32)
@@ -39,7 +40,10 @@ def linear_resize_tc(x_tc: np.ndarray, t_out: int) -> np.ndarray:
     i1 = i0 + (i0 < t_in - 1)
     l1 = (src - i0.astype(f32)).astype(f32)
     l0 = (f32(1.0) - l1).astype(f32)
-    b = (l1[:, None] * x_tc[i1]).astype(f32)
+    if out_dtype == np.float64:
+        x64 = x_tc.astype(np.float64)
+        return np.float64(l0[:, None]) * x64[i0] + np.float64(l1[:, None]) * x64[i1]
+    b =(l1[:, None] * x_tc[i1]).astype(f32)
     return (np.float64(l0[:, None]) * np.float64(x_tc[i0]) + np.float64(b)).astype(f32)
 
 

@@ -84,7 +84,7 @@ def max_pool_3_2_1(x: Tensor) -> Tensor:
     max(x[2t-1], x[2t], x[2t+1]) with out-of-range taps ignored (-inf)."""
     T = x.shape[-1]
     xp = F.pad(x, (1, 1), value=float("-inf"))
-    idx = torch.arange(0, T, 2)
+    idx = torch.arange(0, T, 2, device=x.device)
     return torch.maximum(torch.maximum(xp[..., idx], xp[..., idx + 1]), xp[..., idx + 2])
 
 
@@ -92,7 +92,7 @@ def nearest_resample(x: Tensor, t_out: int) -> Tensor:
     """F.interpolate(mode='nearest') with an integer up/down factor
     (backbones.py:487, 490; necks.py:78): out[t] = in[floor(t * T_in / T_out)]."""
     t_in = x.shape[-1]
-    idx = (torch.arange(t_out) * t_in) // t_out
+    idx = (torch.arange(t_out, device=x.device) * t_in) // t_out
     return x[..., idx]
 
 
@@ -112,7 +112,7 @@ def banded_attention(q: Tensor, k: Tensor, v: Tensor, kv_mask: Tensor,
     kh = k.view(B, n_head, d, T).transpose(2, 3)
     vh = v.view(B, n_head, d, T).transpose(2, 3)
     s = qh @ kh.transpose(-1, -2)                               # [B, H, T, T]
-    i = torch.arange(T)
+    i = torch.arange(T, device=q.device)
     band = (i[:, None] - i[None, :]).abs() <= half_window
     s = s + (~kv_mask).to(s.dtype).view(B, 1, 1, T) * (-1e4)
     s = s.masked_fill(~band.view(1, 1, T, T), float("-inf"))

@@ -15,6 +15,7 @@ import torch
 import torch.nn.functional as F
 
 import interp_ref
+import launch_ref
 import model_ref
 import nms_ref
 from make_golden import sweep_inputs
@@ -340,9 +341,21 @@ def _ln_params(rng, C=256):
     return (torch.from_numpy(rng.uniform(0.5, 1.5, C).astype(np.float32)), torch.from_numpy(rng.normal(0, 0.2, C).astype(np.float32)))
 
 
+LDL_CASES = [pytest.param(*c, 3, torch.float32, id="%d-%d-%d-%d" % c)
+             for c in [(1, 0, 96, 96), (2, 0, 96, 96), (1, 2, 24, 96), (1, -3, 192, 24), (1, 0, 20, 20)]]
+LDL_CASES += [pytest.param(*c, id="%d-%d-%d-%d-%dstreams-%s" % (c[:5] + (str(c[5])[6:],)))
+              for c in [(1, 2, 24, 96, 2, torch.float32), (1, -3, 192, 24, 2, torch.float16),      # the cross-modal K / V
+                        (1, 1, 48, 96, 1, torch.float32), (1, -1, 192, 96, 1, torch.float16),
+                        (2, 0, 96, 96, 2, torch.float32), (2, 0, 96, 96, 1, torch.float16),       # stride 2 without skip_out
+                        (1, 0, 96, 96, 3, torch.float16), (2, 0, 96, 96, 3, torch.float16)]]
+
+
 @pytest.mark.parametrize("tile_rows", [0, 2, 4, 8])
-@pytest.mark.parametrize("stride,shift,T_src,T_virt", [(1, 0, 96, 96), (2, 0, 96, 96), (1, 2, 24, 96), (1, -3, 192, 24), (1, 0, 20, 20)])
-def test_ln_dwconv_ln(stride, shift, T_src, T_virt, tile_rows):
+@pytest.mark.parametrize("stride,shift,T_src,T_virt,n_streams,out_dt", LDL_CASES)
+def test_ln_dwconv_ln(stride, shift, T_src, T_virt, tile_rows, n_streams, out_dt):
+    """tile_rows 0 is the automatic choice: two or three streams take the second-layout kernel (the K / V of every
+    cross-modal block: two streams, shift != 0), one stream the first layout with automatic tile rows. Stride 2 with
+    fewer than three streams runs without skip_out."""
     rng = np.random.RandomState(7)
     B, C = 3, 256
     To = T_virt // stride
@@ -352,16 +365,19 @@ def test_ln_dwconv_ln(stride, shift, T_src, T_virt, tile_rows):
     dws = [torch.from_numpy(rng.normal(0, 0.6, (C, 3)).astype(np.float32)) for _ in range(3)]
     valid = np.array([To, To // 2, To - 1])
     mask = np.arange(To)[None] < valid[:, None]
-    outs = [torch.zeros((B, To, C), device=DEV) for _ in range(3)]
-    skip = torch.zeros((B, To, C), device=DEV) if (stride == 2) else None
-    ops.ln_dwconv_ln(dev(x), batch=B, t_src=T_src, t_virt=T_virt, shift=shift, stride=stride, mask_out=dev(mask.astype(np.uint8)),
-                     ln_in=[(dev(a), dev(b)) for a, b in lni], dw=[dev(d) for d in dws],
-                     ln_out=[(dev(a), dev(b)) for a, b in lno], outs=outs, skip_out=skip, tile_rows=tile_rows)
+    outs = [torch.full((B, To, C), float("nan"), dtype=out_dt, device=DEV) for _ in range(n_streams)]
+    skip = torch.full((B, To, C), float("nan"), device=DEV) if (stride == 2 and n_streams == 3) else None
+    kw = dict(batch=B, t_src=T_src, t_virt=T_virt, shift=shift, stride=stride, mask_out=dev(mask.astype(np.uint8)),
+              ln_in=[(dev(a), dev(b)) for a, b in lni[:n_streams]], dw=[dev(d) for d in dws[:n_streams]],
+              ln_out=[(dev(a), dev(b)) for a, b in lno[:n_streams]], outs=outs, skip_out=skip, tile_rows=tile_rows)
+    ops.ln_dwconv_ln(dev(x), **kw)
+    ref = launch_ref.ln_dwconv_ln(dev(x), **kw)
+    for s in range(n_streams):
+        launch_ref.check(outs[s], ref["outs.%d" % s], C, 5e-5, "stream %d" % s)
     xc = x.permute(0, 2, 1)
     idx = (torch.arange(T_virt) >> shift) if shift >= 0 else (torch.arange(T_virt) << -shift)
     xv = xc[..., idx]                                                  # nearest resample (backbones.py:487,490)
-    m_in = torch.ones(B, 1, T_virt, dtype=torch.bool)
-    for s in range(3):
+    for s in range(n_streams if out_dt == torch.float32 else 0):
         u = model_ref.channel_ln(xv, *lni[s])
         y = F.conv1d(u, dws[s].view(C, 1, 3), None, stride=stride, padding=1, groups=C) * torch.from_numpy(mask)[:, None, :].float()
         y = model_ref.channel_ln(y, *lno[s]).permute(0, 2, 1)
@@ -369,53 +385,83 @@ def test_ln_dwconv_ln(stride, shift, T_src, T_virt, tile_rows):
     if skip is not None:
         want = model_ref.max_pool_3_2_1(xc).permute(0, 2, 1)
         assert torch.equal(skip.cpu(), want.contiguous())
-    del m_in
 
 
-@pytest.mark.parametrize("window,T", [(7, 96), (7, 5), (-1, 24), (-1, 48)])
+ATT_CASES = [pytest.param(w, t, "plain", id="%d-%d" % (w, t)) for w, t in [(7, 96), (7, 5), (-1, 24), (-1, 48), (7, 17), (7, 33),
+                                                                         (7, 100), (7, 768), (-1, 17), (-1, 100)]]
+ATT_CASES += [pytest.param(w, t, v, id="%d-%d-%s" % (w, t, v)) for w, t, v in [(7, 96, "out16"), (-1, 48, "out16"), (7, 768, "out16"),
+                                                                               (7, 96, "no_mask"), (-1, 24, "no_mask"),
+                                                                               (7, 768, "sm_batch"), (7, 192, "sm_batch")]]
+
+
+@pytest.mark.parametrize("window,T,variant", ATT_CASES)
 @pytest.mark.parametrize("in_dt", [torch.float32, torch.bfloat16, torch.float16])
-def test_attention(window, T, in_dt):
+def test_attention(window, T, in_dt, variant):
+    """plain: the fp32 output; out16: the 16-bit output the engine writes in mixed precision; no_mask: kv_mask=None;
+    sm_batch: a batch that gives the tensor-core kernel its 64-row CTAs (as batch 32 does at T = 768). Video 1 ends
+    after one row: its later query rows have their whole band masked."""
+    if variant == "sm_batch" and (window != 7 or in_dt == torch.float32):
+        pytest.skip("the 64-row CTAs belong to the 16-bit window-7 kernel")
     rng = np.random.RandomState(9)
-    B, C, H = 3, 256, 4
+    C, H = 256, 4
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    B = 3 if variant != "sm_batch" else max(3, -(-sms // -(-T // 64)))          # batch * ceil(T / 64) >= SM count
     q, k, v = (torch.from_numpy(rng.standard_normal((B, T, C)).astype(np.float32)).to(in_dt) for _ in range(3))
-    valid = np.array([T, max(1, T // 2), T - 1])
+    valid = np.array([T, 1, T - 1] + [int(x) for x in rng.randint(1, T + 1, B - 3)])
     mask = torch.from_numpy(np.arange(T)[None] < valid[:, None])
-    out = torch.zeros((B, T, C), device=DEV)
-    ops.attention(dev(q), dev(k), dev(v), dev(mask.to(torch.uint8)), out, batch=B, t=T, n_head=H, window=window)
-    qc, kc, vc = (t.float().permute(0, 2, 1).contiguous() for t in (q, k, v))
-    if window > 1:
-        want = model_ref.banded_attention(qc, kc, vc, mask[:, None, :], H, window // 2)
-    else:
-        want = model_ref.global_attention(qc, kc, vc, mask[:, None, :], H)
-        want = want * mask[:, None, :].float()          # masked query rows are zeroed by the proj mask downstream
-        out = out * dev(mask.float())[:, :, None]
-    assert rel_err(out.cpu(), want.permute(0, 2, 1)) < 2e-5
+    out_dt = torch.float16 if variant == "out16" else torch.float32
+    out = torch.full((B, T, C), float("nan"), dtype=out_dt, device=DEV)
+    km = None if variant == "no_mask" else dev(mask.to(torch.uint8))
+    ops.attention(dev(q), dev(k), dev(v), km, out, batch=B, t=T, n_head=H, window=window)
+    ref = launch_ref.attention(dev(q), dev(k), dev(v), km, out, batch=B, t=T, n_head=H, window=window)["out"]
+    launch_ref.check(out, ref, C, 5e-5, "attention")
+    if variant == "plain" and B == 3:
+        qc, kc, vc = (t.float().permute(0, 2, 1).contiguous() for t in (q, k, v))
+        if window > 1:
+            want = model_ref.banded_attention(qc, kc, vc, mask[:, None, :], H, window // 2)
+        else:
+            want = model_ref.global_attention(qc, kc, vc, mask[:, None, :], H)
+            want = want * mask[:, None, :].float()          # masked query rows are zeroed by the proj mask downstream
+            out = out * dev(mask.float())[:, :, None]
+        assert rel_err(out.cpu(), want.permute(0, 2, 1)) < 2e-5
 
 
-@pytest.mark.parametrize("C", [256, 1024])
+@pytest.mark.parametrize("C", [256, 512, 1024])
 def test_ln_rows(C):
     rng = np.random.RandomState(1)
     x = torch.from_numpy(rng.standard_normal((777, C)).astype(np.float32) * 3 + 1)
     w, b = _ln_params(rng, C)
     want = model_ref.channel_ln(x.t()[None], w, b)[0].t()
     for dt in (torch.float32, torch.bfloat16, torch.float16):
-        out = torch.zeros((777, C), dtype=dt, device=DEV)
+        out = torch.full((777, C), float("nan"), dtype=dt, device=DEV)
         ops.ln_rows(dev(x), dev(w), dev(b), out, 777)
         assert rel_err(out.float().cpu(), want) < (2e-6 if dt == torch.float32 else 5e-3)
+        launch_ref.check(out, launch_ref.ln_rows(dev(x), dev(w), dev(b), out, 777)["out"], C, 5e-5, "ln_rows")
 
 
 def test_instnorm_lrelu():
+    """T / 16 rows per thread pick the register kernel (3, 6, 12, 24, 48 rows: T = 24 .. 768); T = 1000 runs the
+    general kernel. 96 / 192 are exp12's contraction levels, 6 / 12 rows the exp5 expansion's. fp32 and the 16-bit
+    outputs of mixed precision."""
     rng = np.random.RandomState(2)
-    for B, T, C in ((3, 384, 256), (2, 24, 2048), (2, 768, 64)):
+    cases = ((3, 384, 256), (2, 24, 2048), (2, 768, 64), (2, 96, 512), (3, 192, 256), (2, 1000, 64), (2, 5, 32))
+    for (B, T, C), out_dt in [(c, dt) for dt in (torch.float32, torch.float16, torch.bfloat16) for c in cases]:
         x = torch.from_numpy(rng.standard_normal((B, T, C)).astype(np.float32) * 2 + 0.3)
         want = F.leaky_relu(model_ref.instance_norm_t(x.permute(0, 2, 1)), 0.2).permute(0, 2, 1)
-        out = torch.zeros((B, T, C), device=DEV)
+        out = torch.full((B, T, C), float("nan"), dtype=out_dt, device=DEV)
         ops.instnorm_lrelu(dev(x), out, batch=B, t=T, channels=C)
-        assert rel_err(out.cpu(), want) < 5e-6
+        if out_dt == torch.float32:
+            assert rel_err(out.cpu(), want) < 5e-6
+        ref = launch_ref.instnorm_lrelu(dev(x), out, batch=B, t=T, channels=C)["out"]
+        launch_ref.check(out, ref, C, 5e-5, "instnorm T=%d" % T)
 
 
-@pytest.mark.parametrize("lens", [[96, 48, 24, 12, 6, 3], [768, 384, 192, 96, 48, 24], [40, 20, 10, 5]])
-def test_fpn_fuse_and_head_final(lens):
+FPN_LENS = [[96, 48, 24, 12, 6, 3], [768, 384, 192, 96, 48, 24], [40, 20, 10, 5]]
+
+
+@pytest.mark.parametrize("lens,out_dt", [pytest.param(l, torch.float32, id="lens%d" % i) for i, l in enumerate(FPN_LENS)] +
+                         [pytest.param(l, torch.float16, id="lens%d-f16" % i) for i, l in enumerate(FPN_LENS)])
+def test_fpn_fuse_and_head_final(lens, out_dt):
     """[96..3] / [768..24]: the column-blocked fpn kernel (level 0 divisible by 32); [40..5]: the row-per-warp kernel."""
     rng = np.random.RandomState(4)
     B, C = 2, 256
@@ -425,8 +471,11 @@ def test_fpn_fuse_and_head_final(lens):
     mask = rng.rand(B, P) > 0.15
     dw = torch.from_numpy(rng.normal(0, 0.6, (L, C, 3)).astype(np.float32))
     lw = torch.from_numpy(rng.uniform(0.5, 1.5, (L, C)).astype(np.float32)); lb = torch.from_numpy(rng.normal(0, 0.2, (L, C)).astype(np.float32))
-    out = torch.zeros((B, P, C), device=DEV)
+    out = torch.full((B, P, C), float("nan"), dtype=out_dt, device=DEV)
     ops.fpn_fuse(dev(lat), dev(mask.astype(np.uint8)), dev(dw), dev(lw), dev(lb), out, batch=B, level_len=lens)
+    ref = launch_ref.fpn_fuse(dev(lat), dev(mask.astype(np.uint8)), dev(dw), dev(lw), dev(lb), out, batch=B, level_len=lens)["out"]
+    launch_ref.check(out, ref, C, 5e-5, "fpn_fuse")
+    out = out.float()
     lats = [lat[:, offs[l]:offs[l + 1]].permute(0, 2, 1).clone() for l in range(L)]
     for l in range(L - 1, 0, -1):
         lats[l - 1] = lats[l - 1] + model_ref.nearest_resample(lats[l], lens[l - 1])
@@ -435,13 +484,13 @@ def test_fpn_fuse_and_head_final(lens):
         m = torch.from_numpy(mask[:, offs[l]:offs[l + 1]])[:, None, :].float()
         z = F.conv1d(lats[l], dw[l].view(C, 1, 3), None, padding=1, groups=C) * m
         fpn.append(model_ref.channel_ln(z, lw[l], lb[l]))
-        assert rel_err(out[:, offs[l]:offs[l + 1]].cpu(), fpn[l].permute(0, 2, 1)) < 2e-5, l
+        assert rel_err(out[:, offs[l]:offs[l + 1]].cpu(), fpn[l].permute(0, 2, 1)) < (2e-5 if out_dt == torch.float32 else 1e-3), l
     # head_final on top
     cw = torch.from_numpy((rng.standard_normal((1, C, 3)) / 10).astype(np.float32)); cb = torch.tensor([-1.0])
     rw = torch.from_numpy((rng.standard_normal((2, C, 3)) / 10).astype(np.float32)); rb = torch.tensor([0.3, -0.2])
     scales = [0.8, 0.9, 1.0, 1.1, 1.2, 1.3][:L]
     cf = torch.from_numpy(rng.standard_normal((B, P, C)).astype(np.float32)); rf = torch.from_numpy(rng.standard_normal((B, P, C)).astype(np.float32))
-    logits = torch.zeros((B, P), device=DEV); offsets = torch.zeros((B, P, 2), device=DEV)
+    logits = torch.full((B, P), float("nan"), device=DEV); offsets = torch.full((B, P, 2), float("nan"), device=DEV)
     ops.head_final(dev(cf), dev(rf), dev(mask.astype(np.uint8)), dev(cw.permute(0, 2, 1).reshape(1, -1)), dev(cb),
                    dev(rw.permute(0, 2, 1).reshape(2, -1)), dev(rb), scales, logits, offsets, batch=B, level_len=lens)
     for l in range(L):
@@ -453,31 +502,42 @@ def test_fpn_fuse_and_head_final(lens):
 
 
 def test_vcls_tails():
+    """exp12 / exp13 video-level tails, with the fp32 z and the 16-bit z the engine feeds them in mixed precision;
+    exp13 with 64 and 32 channels."""
+    for z_dt in (torch.float32, torch.float16, torch.bfloat16):
+        _check_vcls_tails(z_dt)
+
+
+def _check_vcls_tails(z_dt):
     rng = np.random.RandomState(6)
     B, T, C = 3, 24, 256
-    z = torch.from_numpy(rng.standard_normal((B, T, C)).astype(np.float32))
+    z = torch.from_numpy(rng.standard_normal((B, T, C)).astype(np.float32)).to(z_dt)
     w0 = torch.from_numpy((rng.standard_normal((C, C)) / 16).astype(np.float32))
     w1 = torch.from_numpy((rng.standard_normal((C, 2 * C)) / 22).astype(np.float32))
     lw, lb = _ln_params(rng)
     w2 = torch.from_numpy((rng.standard_normal(C) / 16).astype(np.float32)); b2 = torch.tensor([0.1])
-    g = F.leaky_relu(model_ref.instance_norm_t(torch.einsum("oc,btc->bot", w0, z)), 0.2)
+    g = F.leaky_relu(model_ref.instance_norm_t(torch.einsum("oc,btc->bot", w0, z.float())), 0.2)
     pooled = torch.cat([g.max(dim=2).values, g.mean(dim=2)], dim=1)
     h = torch.relu(model_ref.channel_ln((pooled @ w1.t()).unsqueeze(-1), lw, lb).squeeze(-1))
     want = h @ w2 + b2
-    out = torch.zeros(B, device=DEV)
-    ops.vcls_exp12(dev(z), dev(w0.t().contiguous()), dev(w1.t().contiguous()), dev(lw), dev(lb), dev(w2), dev(b2), out, batch=B, t=T)
+    out = torch.full((B,), float("nan"), device=DEV)
+    args = (dev(z), dev(w0.t().contiguous()), dev(w1.t().contiguous()), dev(lw), dev(lb), dev(w2), dev(b2), out)
+    ops.vcls_exp12(*args, batch=B, t=T)
     assert rel_err(out.cpu(), want) < 2e-5
-    T, C = 768, 64
-    z = torch.from_numpy(rng.standard_normal((B, T, C)).astype(np.float32))
-    w0 = torch.from_numpy((rng.standard_normal((C, C)) / 8).astype(np.float32))
-    sw = torch.from_numpy((rng.standard_normal(C) / 8).astype(np.float32)); sb = torch.tensor([0.05])
-    cw = torch.tensor([0.7, -0.4]); cb = torch.tensor([0.2])
-    g = F.leaky_relu(model_ref.instance_norm_t(torch.einsum("oc,btc->bot", w0, z)), 0.2)
-    s = torch.einsum("bct,c->bt", g, sw) + sb
-    want = cw[0] * s.max(dim=1).values + cw[1] * s.mean(dim=1) + cb
-    out = torch.zeros(B, device=DEV)
-    ops.vcls_exp13(dev(z), dev(w0), dev(sw), dev(sb), dev(cw), dev(cb), out, batch=B, t=T)
-    assert rel_err(out.cpu(), want) < 2e-5
+    launch_ref.check(out, launch_ref.vcls_exp12(*args, batch=B, t=T)["out"], 1, 5e-5, "vcls_exp12")
+    for T, C in ((768, 64), (768, 32), (96, 32)):
+        z = torch.from_numpy(rng.standard_normal((B, T, C)).astype(np.float32)).to(z_dt)
+        w0 = torch.from_numpy((rng.standard_normal((C, C)) / 8).astype(np.float32))
+        sw = torch.from_numpy((rng.standard_normal(C) / 8).astype(np.float32)); sb = torch.tensor([0.05])
+        cw = torch.tensor([0.7, -0.4]); cb = torch.tensor([0.2])
+        g = F.leaky_relu(model_ref.instance_norm_t(torch.einsum("oc,btc->bot", w0, z.float())), 0.2)
+        s = torch.einsum("bct,c->bt", g, sw) + sb
+        want = cw[0] * s.max(dim=1).values + cw[1] * s.mean(dim=1) + cb
+        out = torch.full((B,), float("nan"), device=DEV)
+        args = (dev(z), dev(w0), dev(sw), dev(sb), dev(cw), dev(cb), out)
+        ops.vcls_exp13(*args, batch=B, t=T)
+        assert rel_err(out.cpu(), want) < 2e-5, (T, C)
+        launch_ref.check(out, launch_ref.vcls_exp13(*args, batch=B, t=T)["out"], 1, 5e-5, "vcls_exp13 T=%d C=%d" % (T, C))
 
 
 @pytest.mark.parametrize("mode", ["fp32", "fp16"])
