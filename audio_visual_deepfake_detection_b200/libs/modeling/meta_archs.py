@@ -338,6 +338,12 @@ class _LocalizationBase(nn.Module):
                 gc.enable()
         return GraphedPass(graph, res, native.LAUNCHES["n"] - n0, staged, keep)
 
+    def export_plan(self, path, batch_sizes=None, shards=False, max_seconds=36.0, items=None):
+        """Write the launch plan of the raw-stream pass (libs/modeling/plan.py): what libavdf_sm100.so's
+        avdf_session_run replays as a CUDA graph, with no Python in the process."""
+        from .plan import export_plan
+        return export_plan(self, path, batch_sizes=batch_sizes, shards=shards, max_seconds=max_seconds, items=items)
+
     @staticmethod
     def fetch(res):
         segs, scores, counts, vc = res["segs"].cpu(), res["scores"].cpu(), res["counts"].cpu(), res["vcls"].cpu()

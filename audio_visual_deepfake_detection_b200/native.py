@@ -29,6 +29,8 @@ EXPORTS = [
     "avdf_logmel", "avdf_byola_conv1_pool", "avdf_byola_pool", "avdf_eval_workspace_bytes", "avdf_eval_detection",
     "avdf_eval_proposal_workspace_bytes", "avdf_eval_proposal", "avdf_interp_concat_ranges",
     "avdf_window_merge_workspace_bytes", "avdf_window_merge",
+    "avdf_plan_open", "avdf_plan_get_info", "avdf_plan_upload", "avdf_plan_close",
+    "avdf_session_create", "avdf_session_get_io", "avdf_session_run", "avdf_session_destroy",
 ]
 
 
@@ -128,6 +130,22 @@ class EvalProposalArgs(Structure):
     ]
 
 
+class PlanInfo(Structure):
+    _fields_ = [
+        ("abi_version", c_int32), ("cc_major", c_int32), ("cc_minor", c_int32), ("sm_count", c_int32), ("max_batch", c_int32),
+        ("max_seg_num", c_int32), ("t_out", c_int32), ("in_dtype", c_int32),
+        ("channels", c_int32 * 3), ("stream_rows", c_int64 * 3), ("batch_mask", ctypes.c_uint64),
+        ("const_bytes", c_size_t), ("session_bytes", c_size_t), ("description", ctypes.c_char * 1024),
+    ]
+
+
+class SessionIO(Structure):
+    _fields_ = [
+        ("streams", c_void_p * 3), ("offsets", c_void_p), ("meta", c_void_p),
+        ("segs", c_void_p), ("scores", c_void_p), ("counts", c_void_p), ("video_cls", c_void_p),
+    ]
+
+
 # status bits of avdf_eval_detection / avdf_eval_proposal (AVDF_EVAL_*)
 EVAL_PRED_LIMIT, EVAL_GT_LIMIT, EVAL_BAD_OFFSETS, EVAL_BAD_KEEP = 1, 2, 4, 8
 
@@ -188,11 +206,21 @@ def lib():
     L.avdf_eval_proposal_workspace_bytes.restype = c_size_t
     L.avdf_eval_proposal_workspace_bytes.argtypes = [c_int32]
     L.avdf_eval_proposal.argtypes = [POINTER(EvalProposalArgs), c_void_p]
+    L.avdf_plan_open.argtypes = [c_char_p, POINTER(c_void_p)]
+    L.avdf_plan_get_info.argtypes = [c_void_p, POINTER(PlanInfo)]
+    L.avdf_plan_upload.argtypes = [c_void_p, c_void_p, c_size_t, c_void_p]
+    L.avdf_plan_close.argtypes = [c_void_p]
+    L.avdf_plan_close.restype = None
+    L.avdf_session_create.argtypes = [c_void_p, c_void_p, c_size_t, POINTER(c_void_p)]
+    L.avdf_session_get_io.argtypes = [c_void_p, POINTER(SessionIO)]
+    L.avdf_session_run.argtypes = [c_void_p, c_int32, POINTER(c_int64), c_void_p]
+    L.avdf_session_destroy.argtypes = [c_void_p]
+    L.avdf_session_destroy.restype = None
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("avdf_last_error", "avdf_nms_workspace_bytes", "avdf_postprocess_workspace_bytes",
                         "avdf_conv_gemm_workspace_bytes", "avdf_eval_workspace_bytes", "avdf_eval_proposal_workspace_bytes",
-                        "avdf_window_merge_workspace_bytes", "avdf_abi_version"):
+                        "avdf_window_merge_workspace_bytes", "avdf_abi_version", "avdf_plan_close", "avdf_session_destroy"):
             fn.restype = c_int32
     if L.avdf_abi_version() != 3:
         raise AvdfError("libavdf_sm100.so ABI version mismatch")

@@ -456,6 +456,67 @@ AVDF_API int avdf_host_all_pinned(const void* const* src, const size_t* nbytes, 
  * must stay alive and unchanged until the stream has passed the copies. */
 AVDF_API int avdf_h2d_gather(const void* const* src, void* const* dst, const size_t* nbytes, int32_t n, void* stream);
 
+/* ---- the whole model: launch plans (csrc/plan.cu) ----
+ * A plan file holds the launch sequence of the raw-stream pass (resampling -> model -> decode / NMS) of one model at one
+ * precision and test-time config, for a set of batch sizes, recorded by the Python side
+ * (audio_visual_deepfake_detection_b200/libs/modeling/plan.py, `model.export_plan`), together with the packed constants
+ * (weights, mask / positional-encoding tables). Replaying it calls the same entry points with the same arguments as the
+ * Python path, so results are bit-identical to `model.forward_streams` on the same inputs.
+ *
+ *   avdf_plan* plan;  avdf_plan_info info;
+ *   avdf_plan_open(path, &plan);  avdf_plan_get_info(plan, &info);          (host only, no CUDA call)
+ *   cudaMalloc(&consts, info.const_bytes);  avdf_plan_upload(plan, consts, info.const_bytes, stream);
+ *   cudaMalloc(&arena, info.session_bytes);  avdf_session_create(plan, arena, info.session_bytes, &s);
+ *   avdf_session_get_io(s, &io);
+ *   per batch: write io.streams / io.offsets / io.meta (cudaMemcpyAsync on `stream`), avdf_session_run(s, B, rows, stream),
+ *              read io.segs / io.scores / io.counts / io.video_cls
+ *   avdf_session_destroy(s);  avdf_plan_close(plan);  cudaFree(arena);  cudaFree(consts);
+ *
+ * Inputs (device, inside the session arena, sized for max_batch):
+ *   streams[s]   [rows, channels[s]] of stream s (0 video, 1 byola, 2 emo; NULL when channels[s] == 0), the batch's
+ *                recordings back to back, in_dtype (AVDF_DTYPE_F32, or AVDF_DTYPE_BF16 for 16-bit feature shards)
+ *   offsets      int32 [3, max_batch + 1]: offsets[s * (max_batch + 1) + b] = first row of recording b in streams[s],
+ *                offsets[s * (max_batch + 1) + B] = rows[s]
+ *   meta         fp32 [4, B] contiguous (row r at meta + r * B): feat_stride, 0.5 * feat_num_frames, fps, duration.
+ *                For a raw-stream item with T rows in its first stream (video if present, else byola), t_out = info.t_out
+ *                and its duration in seconds, computed in double and then rounded to float:
+ *                  feat_stride = (float)((double)T / t_out);  half_nframes = (float)(0.5 * ((double)T / t_out));
+ *                  fps = (float)((double)T / duration);       duration = (float)duration
+ * Outputs (device, at their max_batch allocations; rows b < B are written):
+ *   segs [B, max_seg_num, 2] seconds, scores [B, max_seg_num] (descending), counts int32 [B], video_cls [B] (logit).
+ * A session is one buffer set: it runs on one stream at a time. Concurrent batches use separate sessions of one plan
+ * (they share its constants). The plan must stay open while it has sessions. */
+typedef struct avdf_plan avdf_plan;          /* parsed plan (host); its constants once uploaded */
+typedef struct avdf_session avdf_session;    /* one buffer set = one batch in flight */
+typedef struct avdf_plan_info {
+  int32_t abi_version, cc_major, cc_minor, sm_count, max_batch, max_seg_num, t_out, in_dtype;
+  int32_t channels[3];  int64_t stream_rows[3];    /* video, byola, emo; 0 channels = absent; rows = staging capacity */
+  uint64_t batch_mask;                             /* bit b-1: a launch list for batch size b */
+  size_t const_bytes, session_bytes;               /* device bytes of avdf_plan_upload / avdf_session_create (256-aligned) */
+  char description[1024];                          /* model, precision, test config, switches */
+} avdf_plan_info;
+/* parse + validate the whole file; makes NO CUDA call. Fails (nothing allocated) on a bad magic / version, a truncated
+ * file, an unknown entry point, a scalar type-tag mismatch, a relocation outside its allocation, a struct-size mismatch. */
+AVDF_API int avdf_plan_open(const char* path, avdf_plan** out);
+AVDF_API int avdf_plan_get_info(const avdf_plan* p, avdf_plan_info* info);
+/* constants -> dev (const_bytes, 256-byte aligned) on `stream`, on the current device; refuses a device whose compute
+ * capability or SM count differs from the recording device's (launch configurations depend on the SM count). */
+AVDF_API int avdf_plan_upload(avdf_plan* p, void* dev, size_t bytes, void* stream);
+AVDF_API void avdf_plan_close(avdf_plan* p);
+/* dev: session_bytes of device memory (256-byte aligned) on the plan's device; zeroed here (synchronously). */
+AVDF_API int avdf_session_create(const avdf_plan* p, void* dev, size_t bytes, avdf_session** out);
+typedef struct avdf_session_io {
+  void* streams[3]; int32_t* offsets; float* meta;
+  float* segs; float* scores; int32_t* counts; float* video_cls;
+} avdf_session_io;
+AVDF_API int avdf_session_get_io(const avdf_session* s, avdf_session_io* io);
+/* One batch of `batch` recordings with rows[s] rows per stream (checked against the staging capacity; nothing is launched
+ * when a check fails). The first call for a batch size runs the launch list eagerly on `stream`, captures it (thread-local
+ * capture mode) into a CUDA graph and launches that; later calls launch the graph. `stream` must be a created stream
+ * (graph capture is not possible on the legacy default stream). Asynchronous; no host synchronisation. */
+AVDF_API int avdf_session_run(avdf_session* s, int32_t batch, const int64_t rows[3], void* stream);
+AVDF_API void avdf_session_destroy(avdf_session* s);
+
 #ifdef __cplusplus
 }
 #endif
