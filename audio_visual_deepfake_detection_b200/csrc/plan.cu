@@ -13,10 +13,12 @@
 //     u32 tag u32 0, then by tag: I32 / I64: i64 | F32: u32 bits u32 0 | PTR: u64 alloc (NULL: ~0) u64 byte offset |
 //     HOST_I32 / HOST_F32: u64 count, count * 4 bytes | STRUCT: u64 size, bytes, u64 n_relocs, per relocation:
 //     u64 field_offset u64 alloc u64 offset (alloc HOST_REF: offset = byte count of a host array that follows) | STREAM
+#include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <new>
 #include <string>
 #include <vector>
@@ -128,6 +130,15 @@ struct avdf_session {
   int device;
   std::vector<std::vector<uint8_t>> structs[kMaxBatch];   // per launch: its args struct with relocated pointers
   cudaGraphExec_t graph[kMaxBatch] = {};
+  // sliding windows (avdf_session_attach_windows): the caller's device block, the windowed graphs (first launch =
+  // avdf_interp_concat_ranges on the fixed start / count arrays), the pinned parameter buffer and its copy's event
+  uint8_t* win = nullptr;
+  int32_t max_windows = 0, max_per_rec = 0;
+  cudaGraphExec_t win_graph[kMaxBatch] = {};
+  uint8_t* pinned = nullptr;
+  cudaEvent_t copied = nullptr;
+  float iou_threshold = 0.f, min_score = 0.f, sigma = 0.f, voting_thresh = 0.f;   // of the recorded avdf_postprocess
+  int32_t use_soft_nms = 0;
 };
 
 namespace {
@@ -401,6 +412,209 @@ int run_list(const avdf_session& s, int batch, cudaStream_t st) {
   return AVDF_OK;
 }
 
+// The first call for a list runs it eagerly on `st` (lazy per-device setup happens outside the capture), then captures it
+// in thread-local mode; every call launches the graph.
+template <class Run>
+int launch_graph(cudaGraphExec_t& exec, Run run, cudaStream_t st, const char* who) {
+  if (!exec) {
+    if (int rc = run()) return rc;
+    AVDF_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+    const int rc = run();
+    cudaGraph_t g = nullptr;
+    const cudaError_t e = cudaStreamEndCapture(st, &g);
+    if (rc) {
+      if (g) cudaGraphDestroy(g);
+      return rc;
+    }
+    AVDF_CUDA(e);
+    const cudaError_t ei = cudaGraphInstantiate(&exec, g, 0);
+    cudaGraphDestroy(g);
+    if (ei != cudaSuccess) {
+      exec = nullptr;
+      avdf::set_error("%s: cudaGraphInstantiate -> %s", who, cudaGetErrorString(ei));
+      return AVDF_ERR_CUDA;
+    }
+  }
+  AVDF_CUDA(cudaGraphLaunch(exec, st));
+  return AVDF_OK;
+}
+
+// ---- sliding windows (libs/modeling/windows.py, the same double operations) ----
+#define WIN_FAIL(code, ...)         \
+  do {                              \
+    avdf::set_error(__VA_ARGS__);   \
+    return code;                    \
+  } while (0)
+
+// First stream of a window's meta: video if present, else byola, else emo.
+int first_stream(const avdf_plan& p) { return p.info.channels[0] > 0 ? 0 : p.info.channels[1] > 0 ? 1 : 2; }
+
+int check_window(const char* who, double W, double H) {
+  if (!(W > 0)) WIN_FAIL(AVDF_ERR_INVALID, "%s: window must be > 0 seconds, got %g", who, W);
+  if (!(H > 0 && H <= W)) WIN_FAIL(AVDF_ERR_INVALID, "%s: hop must satisfy 0 < hop <= window, got hop %g, window %g", who, H, W);
+  return AVDF_OK;
+}
+
+// Number of windows of one recording (window_plan), after every check of its inputs.
+int window_count(const avdf_plan& p, const char* who, double D, const int64_t rows[3], double W, double H, int64_t* n) {
+  if (int rc = check_window(who, W, H)) return rc;
+  if (!(D > 0) || !(D <= 1e300)) WIN_FAIL(AVDF_ERR_INVALID, "%s: duration must be a positive finite number of seconds, got %g", who, D);
+  for (int s = 0; s < 3; ++s) {
+    if (p.info.channels[s] == 0 && rows[s] != 0)
+      WIN_FAIL(AVDF_ERR_INVALID, "%s: stream %d is absent from the plan but has %lld rows", who, s, (long long)rows[s]);
+    if (p.info.channels[s] > 0 && (rows[s] < 1 || rows[s] > INT32_MAX))
+      WIN_FAIL(AVDF_ERR_INVALID, "%s: stream %d is present in the plan but has %lld rows", who, s, (long long)rows[s]);
+  }
+  if (D <= W) {
+    *n = 1;
+    return AVDF_OK;
+  }
+  for (int s = 0; s < 3; ++s)
+    if (p.info.channels[s] > 0 && floor(W * (double)rows[s] / D) < 1)
+      WIN_FAIL(AVDF_ERR_INVALID, "%s: a %.3f s window of a %.3f s recording holds no row of stream %d (%lld rows)", who, W, D,
+               s, (long long)rows[s]);
+  const double k = ceil((D - W) / H);
+  if (!(k < (double)(1 << 30)))
+    WIN_FAIL(AVDF_ERR_INVALID, "%s: %.3f s in %g s hops of a %g s window is more than 2^30 windows", who, D, H, W);
+  *n = (int64_t)k + 1;
+  return AVDF_OK;
+}
+
+// The meta formula of avdf_session_run (streaming.video_meta with feat_stride = num_frames = 1).
+void window_meta(const avdf_plan& p, int64_t T, double duration, float* m) {
+  const double fs = (double)T / p.info.t_out;
+  m[0] = (float)fs;
+  m[1] = (float)(0.5 * fs);
+  m[2] = (float)((double)T / duration);
+  m[3] = (float)duration;
+}
+
+// Window k of n (window_count's n) of one recording: rows relative to the recording, meta, fp32 start.
+void window_at(const avdf_plan& p, double D, const int64_t rows[3], double W, double H, int64_t n, int64_t k,
+               int32_t start[3], int32_t count[3], float meta[4], float* win_start) {
+  const int first = first_stream(p);
+  if (D <= W) {
+    for (int s = 0; s < 3; ++s) start[s] = 0, count[s] = (int32_t)rows[s];
+    window_meta(p, rows[first], D, meta);
+    *win_start = 0.f;
+    return;
+  }
+  const double sk = std::min((double)k * H, D - W);
+  for (int s = 0; s < 3; ++s) {
+    const bool on = p.info.channels[s] > 0;
+    start[s] = on ? (int32_t)floor(sk * (double)rows[s] / D) : 0;
+    count[s] = on ? (int32_t)floor(W * (double)rows[s] / D) : 0;
+  }
+  window_meta(p, count[first], W, meta);
+  *win_start = (float)sk;
+}
+
+// Can every launch list run windows? Its first launch is the CSR resampling reading the io offsets for its own batch size
+// (replaced by the range form in the windowed list), and it has one postprocess writing the io outputs without records.
+// Fills the NMS settings of the merge when `s` is given.
+int check_windowable(const avdf_plan& p, const char* who, avdf_session* s) {
+  const uint64_t off = (uint64_t)p.io[ROLE_OFFSETS];
+  for (int b = 1; b <= p.info.max_batch; ++b) {
+    if (!(p.info.batch_mask >> (b - 1) & 1)) continue;
+    const auto& list = p.lists[b - 1];
+    if (list.empty() || list[0].op != OP_INTERP)
+      WIN_FAIL(AVDF_ERR_UNSUPPORTED, "%s: the launch list for batch %d does not start with avdf_interp_concat_in (it starts "
+               "with %s)", who, b, list.empty() ? "nothing" : kOps[list[0].op].name);
+    const Launch& in = list[0];
+    for (int k = 0; k < 3; ++k) {
+      const Arg& a = in.args[4 + k];
+      if (p.info.channels[k] > 0 ? (a.alloc != off) : (a.alloc != kNull))
+        WIN_FAIL(AVDF_ERR_UNSUPPORTED, "%s: batch %d: the resampling's stream %d offsets are not the io offsets", who, b, k);
+    }
+    if (in.args[7].i != b)
+      WIN_FAIL(AVDF_ERR_UNSUPPORTED, "%s: batch %d: the resampling runs %lld recordings", who, b, (long long)in.args[7].i);
+    const Launch* post = nullptr;
+    for (const Launch& l : list)
+      if (l.op == OP_POSTPROCESS) {
+        if (post) WIN_FAIL(AVDF_ERR_UNSUPPORTED, "%s: batch %d: more than one avdf_postprocess", who, b);
+        post = &l;
+      }
+    if (!post) WIN_FAIL(AVDF_ERR_UNSUPPORTED, "%s: batch %d: no avdf_postprocess", who, b);
+    const Arg& a = post->args[0];
+    avdf_postprocess_args pa;
+    memcpy(&pa, a.bytes.data(), sizeof(pa));
+    const struct { size_t field; int role; } outs[3] = {{offsetof(avdf_postprocess_args, out_segs), ROLE_SEGS},
+                                                        {offsetof(avdf_postprocess_args, out_scores), ROLE_SCORES},
+                                                        {offsetof(avdf_postprocess_args, out_count), ROLE_COUNTS}};
+    for (const auto& o : outs) {
+      bool ok = false;
+      for (const Reloc& r : a.relocs) ok |= r.field == o.field && r.alloc == (uint64_t)p.io[o.role] && r.offset == 0;
+      if (!ok) WIN_FAIL(AVDF_ERR_UNSUPPORTED, "%s: batch %d: avdf_postprocess does not write the io outputs", who, b);
+    }
+    for (const Reloc& r : a.relocs)
+      if (r.field == offsetof(avdf_postprocess_args, rec_ring))
+        WIN_FAIL(AVDF_ERR_UNSUPPORTED, "%s: batch %d: avdf_postprocess keeps result records", who, b);
+    if (pa.use_soft_nms != 0 && !(pa.use_soft_nms == 1 && pa.soft_method == 2))
+      WIN_FAIL(AVDF_ERR_UNSUPPORTED, "%s: batch %d: avdf_postprocess runs use_soft_nms %d (method %d); windows merge with hard "
+               "or soft (method 2) NMS", who, b, pa.use_soft_nms, pa.soft_method);
+    if (s) {
+      s->iou_threshold = pa.iou_threshold, s->min_score = pa.min_score, s->sigma = pa.sigma;
+      s->voting_thresh = pa.voting_thresh, s->use_soft_nms = pa.use_soft_nms;
+    }
+  }
+  return AVDF_OK;
+}
+
+// The window block: byte offsets of its parts (avdf_session_window_bytes documents the sum).
+struct WinBlock {
+  size_t table, fixed, segs, scores, count, cls, ws, ws_bytes, total;
+};
+size_t table_bytes(const avdf_plan& p, int64_t W) { return 4 * (12 * W + 10 * (int64_t)p.info.max_batch); }
+WinBlock win_block(const avdf_plan& p, int64_t W, int64_t per_rec) {
+  const int64_t B = p.info.max_batch, K = p.info.max_seg_num;
+  WinBlock w{};
+  size_t o = 0;
+  w.table = o, o += align_up(table_bytes(p, W));
+  w.fixed = o, o += align_up(24 * B);
+  w.segs = o, o += align_up(8 * K * W);
+  w.scores = o, o += align_up(4 * K * W);
+  w.count = o, o += align_up(4 * W);
+  w.cls = o, o += align_up(4 * W);
+  w.ws = o, w.ws_bytes = avdf_window_merge_workspace_bytes((int32_t)W, (int32_t)(K * per_rec));
+  w.total = o + w.ws_bytes;
+  return w;
+}
+
+int check_limits(const avdf_plan& p, const char* who, int32_t max_windows, int32_t per_rec) {
+  if (max_windows < 1 || max_windows > (1 << 24) || per_rec < 1 || per_rec > max_windows)
+    WIN_FAIL(AVDF_ERR_INVALID, "%s: need 1 <= max_windows_per_recording (%d) <= max_windows (%d) <= 2^24", who, per_rec,
+             max_windows);
+  if ((int64_t)per_rec * p.info.max_seg_num > INT32_MAX)
+    WIN_FAIL(AVDF_ERR_INVALID, "%s: max_windows_per_recording %d * max_seg_num %d overflows int32", who, per_rec,
+             p.info.max_seg_num);
+  return AVDF_OK;
+}
+
+// Batch size whose list runs `b` windows: b itself when recorded, else the smallest recorded size above it.
+int run_size(const avdf_plan& p, int b) {
+  for (int r = b; r <= p.info.max_batch; ++r)
+    if (p.info.batch_mask >> (r - 1) & 1) return r;
+  return 0;
+}
+
+// The windowed list for batch B: the recorded list with its first launch as the range form, reading the fixed arrays.
+int run_windowed_list(const avdf_session& s, int batch, cudaStream_t st) {
+  const avdf_plan& p = *s.plan;
+  const auto& list = p.lists[batch - 1];
+  const Launch& l = list[0];
+  void* P[3];
+  for (int k = 0; k < 3; ++k) P[k] = resolve(p, s.arena, l.args[k].alloc, l.args[k].offset);
+  const int32_t* start = (const int32_t*)(s.win + win_block(p, s.max_windows, s.max_per_rec).fixed);
+  auto I = [&](int k) { return (int32_t)l.args[k].i; };
+  if (int rc = avdf_interp_concat_ranges(P[0], P[1], P[2], I(3), start, start + 3 * batch, I(7), I(8), I(9), I(10), I(11),
+                                         resolve(p, s.arena, l.args[12].alloc, l.args[12].offset), I(13), st))
+    return rc;
+  const auto& structs = s.structs[batch - 1];
+  for (size_t i = 1; i < list.size(); ++i)
+    if (int rc = call(s, list[i], structs[i], st)) return rc;
+  return AVDF_OK;
+}
+
 }  // namespace
 
 extern "C" int avdf_plan_open(const char* path, avdf_plan** out) {
@@ -528,33 +742,175 @@ extern "C" int avdf_session_run(avdf_session* s, int32_t batch, const int64_t ro
   AVDF_CHECK_ARG(stream != nullptr, "stream is the legacy default stream (graph capture needs a created stream)");
   AVDF_CHECK_ARG(avdf::current_device() == s->device, "the current device is not the plan's");
   cudaStream_t st = (cudaStream_t)stream;
-  cudaGraphExec_t& exec = s->graph[batch - 1];
-  if (!exec) {
-    if (int rc = run_list(*s, batch, st)) return rc;          // eager pass: lazy per-device setup happens outside the capture
-    AVDF_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    const int rc = run_list(*s, batch, st);
-    cudaGraph_t g = nullptr;
-    const cudaError_t e = cudaStreamEndCapture(st, &g);
-    if (rc) {
-      if (g) cudaGraphDestroy(g);
-      return rc;
-    }
-    AVDF_CUDA(e);
-    const cudaError_t ei = cudaGraphInstantiate(&exec, g, 0);
-    cudaGraphDestroy(g);
-    if (ei != cudaSuccess) {
-      exec = nullptr;
-      avdf::set_error("avdf_session_run: cudaGraphInstantiate -> %s", cudaGetErrorString(ei));
-      return AVDF_ERR_CUDA;
-    }
-  }
-  AVDF_CUDA(cudaGraphLaunch(exec, st));
-  return AVDF_OK;
+  return launch_graph(s->graph[batch - 1], [&] { return run_list(*s, batch, st); }, st, "avdf_session_run");
 }
 
 extern "C" void avdf_session_destroy(avdf_session* s) {
   if (!s) return;
   for (auto& g : s->graph)
     if (g) cudaGraphExecDestroy(g);
+  for (auto& g : s->win_graph)
+    if (g) cudaGraphExecDestroy(g);
+  if (s->copied) {
+    cudaEventSynchronize(s->copied);         // the last call's parameter copy still reads the pinned buffer
+    cudaEventDestroy(s->copied);
+  }
+  if (s->pinned) cudaFreeHost(s->pinned);
   delete s;
+}
+
+// ---- sliding windows ----
+extern "C" int32_t avdf_plan_window_layout(const avdf_plan* p, double duration, const int64_t rows[3], double window,
+                                           double hop, int32_t cap, int32_t* start, int32_t* count, float* meta,
+                                           float* win_start) {
+  AVDF_CHECK_ARG(p != nullptr && rows != nullptr, "plan / rows is NULL");
+  int64_t n = 0;
+  if (int rc = window_count(*p, "avdf_plan_window_layout", duration, rows, window, hop, &n)) return rc;
+  if (n > INT32_MAX) WIN_FAIL(AVDF_ERR_INVALID, "avdf_plan_window_layout: %lld windows", (long long)n);
+  if (cap >= n && start && count && meta && win_start)
+    for (int64_t k = 0; k < n; ++k)
+      window_at(*p, duration, rows, window, hop, n, k, start + 3 * k, count + 3 * k, meta + 4 * k, win_start + k);
+  return (int32_t)n;
+}
+
+extern "C" size_t avdf_session_window_bytes(const avdf_plan* p, int32_t max_windows, int32_t max_windows_per_recording) {
+  if (!p) {
+    avdf::set_error("avdf_session_window_bytes: plan is NULL");
+    return 0;
+  }
+  if (check_limits(*p, "avdf_session_window_bytes", max_windows, max_windows_per_recording) ||
+      check_windowable(*p, "avdf_session_window_bytes", nullptr))
+    return 0;
+  return win_block(*p, max_windows, max_windows_per_recording).total;
+}
+
+extern "C" int avdf_session_attach_windows(avdf_session* s, void* dev, size_t bytes, int32_t max_windows,
+                                           int32_t max_windows_per_recording) {
+  AVDF_CHECK_ARG(s != nullptr, "session is NULL");
+  AVDF_CHECK_ARG(s->win == nullptr, "the session already has a window block");
+  const avdf_plan& p = *s->plan;
+  const char* who = "avdf_session_attach_windows";
+  if (int rc = check_limits(p, who, max_windows, max_windows_per_recording)) return rc;
+  if (int rc = check_windowable(p, who, s)) return rc;
+  AVDF_CHECK_ARG(dev != nullptr && bytes >= win_block(p, max_windows, max_windows_per_recording).total,
+                 "device block smaller than avdf_session_window_bytes");
+  AVDF_CHECK_ARG((uintptr_t)dev % kAlign == 0, "device block is not 256-byte aligned");
+  AVDF_CHECK_ARG(avdf::current_device() == s->device, "the current device is not the plan's");
+  AVDF_CUDA(cudaHostAlloc((void**)&s->pinned, table_bytes(p, max_windows), cudaHostAllocDefault));
+  const cudaError_t e = cudaEventCreateWithFlags(&s->copied, cudaEventDisableTiming);
+  if (e != cudaSuccess) {
+    cudaFreeHost(s->pinned);
+    s->pinned = nullptr, s->copied = nullptr;
+    WIN_FAIL(AVDF_ERR_CUDA, "%s: cudaEventCreateWithFlags -> %s", who, cudaGetErrorString(e));
+  }
+  s->win = (uint8_t*)dev;
+  s->max_windows = max_windows, s->max_per_rec = max_windows_per_recording;
+  return AVDF_OK;
+}
+
+extern "C" int avdf_session_run_windows(avdf_session* s, const avdf_window_run_args* a, void* stream) {
+  AVDF_CHECK_ARG(s != nullptr && a != nullptr, "session / args is NULL");
+  const char* who = "avdf_session_run_windows";
+  if (!s->win) WIN_FAIL(AVDF_ERR_INVALID, "%s: the session has no window block (avdf_session_attach_windows)", who);
+  if (a->n_rec < 1) WIN_FAIL(AVDF_ERR_INVALID, "%s: n_rec is %d, needs >= 1 recording", who, a->n_rec);
+  AVDF_CHECK_ARG(a->duration && a->rows && a->out_segs && a->out_scores && a->out_count && a->out_cls,
+                 "duration / rows / an output is NULL");
+  const avdf_plan& p = *s->plan;
+  const int R = a->n_rec;
+  std::vector<int64_t> n_win(R);
+  int64_t total_win = 0, most = 0, total_rows[3] = {0, 0, 0};
+  for (int r = 0; r < R; ++r) {
+    const int64_t* rows = a->rows + 3 * r;
+    if (int rc = window_count(p, who, a->duration[r], rows, a->window, a->hop, &n_win[r])) return rc;
+    if (n_win[r] > s->max_per_rec)
+      WIN_FAIL(AVDF_ERR_INVALID, "%s: recording %d has %lld windows, the window block holds %d per recording", who, r,
+               (long long)n_win[r], s->max_per_rec);
+    total_win += n_win[r], most = std::max(most, n_win[r]);
+    for (int k = 0; k < 3; ++k) total_rows[k] += rows[k];
+  }
+  if (total_win > s->max_windows)
+    WIN_FAIL(AVDF_ERR_INVALID, "%s: %lld windows, the window block holds %d", who, (long long)total_win, s->max_windows);
+  for (int k = 0; k < 3; ++k)
+    if (total_rows[k] > p.info.stream_rows[k])
+      WIN_FAIL(AVDF_ERR_INVALID, "%s: stream %d: %lld rows, the staging holds %lld", who, k, (long long)total_rows[k],
+               (long long)p.info.stream_rows[k]);
+  AVDF_CHECK_ARG(stream != nullptr, "stream is the legacy default stream (graph capture needs a created stream)");
+  AVDF_CHECK_ARG(avdf::current_device() == s->device, "the current device is not the plan's");
+  cudaStream_t st = (cudaStream_t)stream;
+
+  // ---- the table: per batch [start 3B | count 3B | meta 4B] (B = the size its list runs), then win_start, rec_win
+  int step = 0;
+  for (int b = p.info.max_batch; b >= 1 && !step; --b)
+    if (p.info.batch_mask >> (b - 1) & 1) step = b;
+  struct Batch { int64_t u0; int b, run; size_t word; };
+  std::vector<Batch> batches;
+  size_t words = 0;
+  for (int64_t u0 = 0; u0 < total_win; u0 += step) {
+    const int b = (int)std::min<int64_t>(step, total_win - u0);
+    const int run = run_size(p, b);
+    batches.push_back({u0, b, run, words});
+    words += 10 * (size_t)run;
+  }
+  const size_t ws_word = words, rw_word = words + total_win, used = 4 * (rw_word + R + 1);
+  AVDF_CUDA(cudaEventSynchronize(s->copied));       // the previous call's copy has read the buffer
+  int32_t* wi = (int32_t*)s->pinned;
+  float* wf = (float*)s->pinned;
+  int64_t u = 0, row0[3] = {0, 0, 0};          // window index; first row of the recording in each stream's staging
+  for (int r = 0; r < R; ++r) {
+    const int64_t* rows = a->rows + 3 * r;
+    wi[rw_word + r] = (int32_t)u;
+    for (int64_t k = 0; k < n_win[r]; ++k, ++u) {
+      const Batch& bt = batches[u / step];
+      int32_t sa[3], ca[3];
+      float m[4];
+      window_at(p, a->duration[r], rows, a->window, a->hop, n_win[r], k, sa, ca, m, &wf[ws_word + u]);
+      const int j0 = (int)(u - bt.u0), j1 = j0 + 1 == bt.b ? bt.run : j0 + 1;   // the batch's last window fills its unused slots
+      for (int j = j0; j < j1; ++j) {
+        for (int q = 0; q < 3; ++q) {
+          wi[bt.word + q * bt.run + j] = (int32_t)(row0[q] + sa[q]);
+          wi[bt.word + (3 + q) * bt.run + j] = ca[q];
+        }
+        for (int q = 0; q < 4; ++q) wf[bt.word + (6 + q) * bt.run + j] = m[q];
+      }
+    }
+    for (int q = 0; q < 3; ++q) row0[q] += rows[q];
+  }
+  wi[rw_word + R] = (int32_t)u;
+  const WinBlock wb = win_block(p, s->max_windows, s->max_per_rec);
+  uint8_t* table = s->win + wb.table;
+  AVDF_CUDA(cudaMemcpyAsync(table, s->pinned, used, cudaMemcpyHostToDevice, st));
+  AVDF_CUDA(cudaEventRecord(s->copied, st));
+
+  // ---- the windows, batch by batch; every window's results set aside
+  avdf_session_io io;
+  avdf_session_get_io(s, &io);
+  const int64_t K = p.info.max_seg_num;
+  float* w_segs = (float*)(s->win + wb.segs);
+  float* w_scores = (float*)(s->win + wb.scores);
+  int32_t* w_count = (int32_t*)(s->win + wb.count);
+  float* w_cls = (float*)(s->win + wb.cls);
+  for (const Batch& bt : batches) {
+    const uint8_t* blk = table + 4 * bt.word;
+    AVDF_CUDA(cudaMemcpyAsync(s->win + wb.fixed, blk, 24 * (size_t)bt.run, cudaMemcpyDeviceToDevice, st));
+    AVDF_CUDA(cudaMemcpyAsync(io.meta, blk + 24 * (size_t)bt.run, 16 * (size_t)bt.run, cudaMemcpyDeviceToDevice, st));
+    const int run = bt.run;
+    if (int rc = launch_graph(s->win_graph[run - 1], [&] { return run_windowed_list(*s, run, st); }, st, who)) return rc;
+    AVDF_CUDA(cudaMemcpyAsync(w_segs + bt.u0 * K * 2, io.segs, 8 * K * bt.b, cudaMemcpyDeviceToDevice, st));
+    AVDF_CUDA(cudaMemcpyAsync(w_scores + bt.u0 * K, io.scores, 4 * K * bt.b, cudaMemcpyDeviceToDevice, st));
+    AVDF_CUDA(cudaMemcpyAsync(w_count + bt.u0, io.counts, 4 * (size_t)bt.b, cudaMemcpyDeviceToDevice, st));
+    AVDF_CUDA(cudaMemcpyAsync(w_cls + bt.u0, io.video_cls, 4 * (size_t)bt.b, cudaMemcpyDeviceToDevice, st));
+  }
+
+  // ---- one result per recording
+  avdf_window_merge_args m{};
+  m.n_rec = R;
+  m.rec_win = (const int32_t*)(table + 4 * rw_word);
+  m.win_start = (const float*)(table + 4 * ws_word);
+  m.win_segs = w_segs, m.win_scores = w_scores, m.win_count = w_count, m.win_cls = w_cls;
+  m.cand_cap = (int32_t)(K * most);
+  m.iou_threshold = s->iou_threshold, m.min_score = s->min_score, m.sigma = s->sigma, m.voting_thresh = s->voting_thresh;
+  m.max_seg_num = (int32_t)K, m.use_soft_nms = s->use_soft_nms;
+  m.out_segs = a->out_segs, m.out_scores = a->out_scores, m.out_count = a->out_count, m.out_cls = a->out_cls;
+  m.workspace = s->win + wb.ws, m.workspace_bytes = avdf_window_merge_workspace_bytes(R, m.cand_cap);
+  return avdf_window_merge(&m, stream);
 }

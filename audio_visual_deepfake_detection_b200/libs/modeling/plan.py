@@ -11,9 +11,11 @@ aborts the export. `engine.py` stays the only place that knows the launch sequen
 signatures.
 
     python -m audio_visual_deepfake_detection_b200.libs.modeling.plan CFG CKPT OUT [--precision mixed|fp32] [--shards]
-                                                                      [--batch-sizes 1 8 32]
+                                                                      [--batch-sizes 1 8 32] [--max-seconds 36]
 
-`Plan` / `PlanSession` drive a plan file from Python through ctypes (tests, scripts/plan_bench.py).
+`Plan` / `PlanSession` drive a plan file from Python through ctypes (tests, scripts/plan_bench.py);
+`PlanSession.run_windows` runs sliding windows over long recordings (avdf_session_run_windows), like
+`forward_streams(window=...)`.
 """
 import argparse
 import bisect
@@ -235,26 +237,33 @@ def _synthetic_items(dims, n, seed):
             for i, d in enumerate(durs)]
 
 
-def _stage_items(items, streams, offsets, meta, t_out):
-    """Raw-stream items -> the staging tensors (recordings back to back, row prefixes, meta [4, B]); returns rows."""
-    from .streaming import _stream_array, video_meta
+def _stage_streams(items, streams):
+    """Raw-stream items -> the stream staging, recordings back to back; returns the row offsets [3, B + 1]."""
+    from .streaming import _stream_array
     B = len(items)
-    mb1 = offsets.shape[1]
-    off = np.zeros((3, mb1), np.int32)
-    rows = [0, 0, 0]
+    off = np.zeros((3, B + 1), np.int64)
     for s, name in enumerate(STREAM_NAMES):
         if streams[s] is None:
             continue
         arrs = [_stream_array(c["streams"][name]) for c in items]
-        off[s, 1:B + 1] = np.cumsum([a.shape[0] for a in arrs])
-        rows[s] = int(off[s, B])
-        if rows[s] > streams[s].shape[0]:
-            raise AvdfError("%s: %d rows, the staging holds %d" % (name, rows[s], streams[s].shape[0]))
+        off[s, 1:] = np.cumsum([a.shape[0] for a in arrs])
+        if off[s, B] > streams[s].shape[0]:
+            raise AvdfError("%s: %d rows, the staging holds %d" % (name, off[s, B], streams[s].shape[0]))
         cat = np.concatenate(arrs, axis=0)
         host = torch.from_numpy(cat.view(np.int16)).view(torch.bfloat16) if cat.dtype == np.uint16 else torch.from_numpy(cat)
         if host.dtype != streams[s].dtype:
             raise AvdfError("%s: %s rows for %s staging" % (name, host.dtype, streams[s].dtype))
-        streams[s][:rows[s]].copy_(host, non_blocking=False)
+        streams[s][:int(off[s, B])].copy_(host, non_blocking=False)
+    return off
+
+
+def _stage_items(items, streams, offsets, meta, t_out):
+    """Raw-stream items -> the staging tensors (recordings back to back, row prefixes, meta [4, B]); returns rows."""
+    from .streaming import _stream_array, video_meta
+    B = len(items)
+    off = np.zeros((3, offsets.shape[1]), np.int32)
+    off[:, :B + 1] = _stage_streams(items, streams)
+    rows = [int(off[s, B]) for s in range(3)]
     m = np.empty((4, B), np.float32)
     for b, c in enumerate(items):
         first = c["streams"]["video"] if streams[0] is not None else c["streams"]["byola"]
@@ -449,6 +458,7 @@ class PlanSession:
         self.scores = self._view(io.scores, (mb, K), torch.float32)
         self.counts = self._view(io.counts, (mb,), torch.int32)
         self.vcls = self._view(io.video_cls, (mb,), torch.float32)
+        self.win_block = None                 # device block of attach_windows
 
     def _view(self, p, shape, dtype):
         off = p - self.arena.data_ptr()
@@ -482,10 +492,58 @@ class PlanSession:
         self.launch(len(items), rows, stream)
         return self.results([c["video_id"] for c in items])
 
+    def attach_windows(self, max_windows, max_windows_per_recording):
+        """Give the session a window block (a torch device tensor) for run_windows calls with at most `max_windows`
+        windows in all and `max_windows_per_recording` windows per recording."""
+        L, mw, per = self.plan.L, int(max_windows), int(max_windows_per_recording)
+        n = L.avdf_session_window_bytes(self.plan.h, mw, per)
+        if n == 0:
+            raise AvdfError("avdf_session_window_bytes failed: %s" % L.avdf_last_error().decode())
+        with torch.cuda.device(self.plan.device):
+            block = torch.empty(n, dtype=torch.uint8, device=self.plan.device)
+            nv.check(L.avdf_session_attach_windows(self.h, block.data_ptr(), n, mw, per), "avdf_session_attach_windows")
+        self.win_block = block
+        return n
+
+    def launch_windows(self, durations, rows, window, hop, outs, stream=None):
+        """avdf_session_run_windows over recordings already staged (rows: [n_rec][3]) into outs = (segs [R, K, 2],
+        scores [R, K], counts [R], video_cls [R]) on `stream` (default: the session's stream); asynchronous."""
+        R = len(durations)
+        a = nv.WindowRunArgs()
+        dur = (ctypes.c_double * max(R, 1))(*[float(d) for d in durations])
+        rws = (c_int64 * max(3 * R, 3))(*[int(v) for r in rows for v in r])
+        a.n_rec, a.duration, a.rows, a.window, a.hop = R, dur, rws, float(window), float(hop)
+        a.out_segs, a.out_scores, a.out_count, a.out_cls = (t.data_ptr() for t in outs)
+        st = stream if stream is not None else self.stream
+        with torch.cuda.device(self.plan.device):
+            rc = self.plan.L.avdf_session_run_windows(self.h, ctypes.byref(a), c_void_p(st.cuda_stream))
+        nv.check(rc, "avdf_session_run_windows")
+
+    def run_windows(self, items, window, hop=None):
+        """Sliding windows over raw-stream recordings of any length (hop defaults to window / 2): the same list of
+        dicts as model.forward_streams(items, window=window, hop=hop). All recordings go into the stream staging at
+        once, so their rows must fit it (export_plan's max_seconds); their windows may exceed max_batch."""
+        W = float(window)
+        H = W / 2.0 if hop is None else float(hop)
+        R, K = len(items), self.plan.info.max_seg_num
+        with torch.cuda.device(self.plan.device), torch.cuda.stream(self.stream):
+            off = _stage_streams(items, self.streams)
+        rows = (off[:, 1:] - off[:, :-1]).T.tolist()
+        dev = self.plan.device
+        outs = (torch.empty((R, K, 2), dtype=torch.float32, device=dev), torch.empty((R, K), dtype=torch.float32, device=dev),
+                torch.empty((R,), dtype=torch.int32, device=dev), torch.empty((R,), dtype=torch.float32, device=dev))
+        self.launch_windows([c["duration"] for c in items], rows, W, H, outs)
+        torch.cuda.synchronize(dev)
+        segs, scores, counts, vcls = (t.cpu() for t in outs)
+        return [{"video_id": c["video_id"], "segments": segs[r, :int(counts[r])], "scores": scores[r, :int(counts[r])],
+                 "labels": torch.zeros(int(counts[r]), dtype=torch.long), "video_cls": vcls[r:r + 1]}
+                for r, c in enumerate(items)]
+
     def close(self):
         if self.h:
             self.plan.L.avdf_session_destroy(self.h)
             self.h = c_void_p()
+        self.win_block = None
 
 
 # ---------------------------------------------------------------------------- CLI
@@ -501,6 +559,9 @@ def main(argv=None):
     p.add_argument("--shards", action="store_true", help="the plan takes bf16 streams (16-bit feature shards)")
     p.add_argument("--batch-sizes", type=int, nargs="+", default=None, help="default: 1 .. --max-batch")
     p.add_argument("--max-batch", type=int, default=32)
+    p.add_argument("--max-seconds", type=float, default=36.0,
+                   help="input staging: a full batch of recordings this long (sliding windows over long recordings "
+                        "stage all of a call's recordings at once)")
     a = p.parse_args(argv)
     cfg = load_config(a.config)
     model = make_meta_arch(cfg["model_name"], **cfg["model"], precision=a.precision, max_batch=a.max_batch)
@@ -508,7 +569,7 @@ def main(argv=None):
     model.load_state_dict(ckpt["state_dict_ema"])
     del ckpt
     model.to(torch.device(cfg["devices"][0])).eval()
-    export_plan(model, a.out, batch_sizes=a.batch_sizes, shards=a.shards)
+    export_plan(model, a.out, batch_sizes=a.batch_sizes, shards=a.shards, max_seconds=a.max_seconds)
     print("wrote %s (%d bytes)" % (a.out, os.path.getsize(a.out)))
     return 0
 

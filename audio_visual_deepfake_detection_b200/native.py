@@ -31,6 +31,7 @@ EXPORTS = [
     "avdf_window_merge_workspace_bytes", "avdf_window_merge",
     "avdf_plan_open", "avdf_plan_get_info", "avdf_plan_upload", "avdf_plan_close",
     "avdf_session_create", "avdf_session_get_io", "avdf_session_run", "avdf_session_destroy",
+    "avdf_plan_window_layout", "avdf_session_window_bytes", "avdf_session_attach_windows", "avdf_session_run_windows",
 ]
 
 
@@ -146,6 +147,13 @@ class SessionIO(Structure):
     ]
 
 
+class WindowRunArgs(Structure):
+    _fields_ = [
+        ("n_rec", c_int32), ("duration", POINTER(c_double)), ("rows", POINTER(c_int64)), ("window", c_double), ("hop", c_double),
+        ("out_segs", c_void_p), ("out_scores", c_void_p), ("out_count", c_void_p), ("out_cls", c_void_p),
+    ]
+
+
 # status bits of avdf_eval_detection / avdf_eval_proposal (AVDF_EVAL_*)
 EVAL_PRED_LIMIT, EVAL_GT_LIMIT, EVAL_BAD_OFFSETS, EVAL_BAD_KEEP = 1, 2, 4, 8
 
@@ -216,11 +224,18 @@ def lib():
     L.avdf_session_run.argtypes = [c_void_p, c_int32, POINTER(c_int64), c_void_p]
     L.avdf_session_destroy.argtypes = [c_void_p]
     L.avdf_session_destroy.restype = None
+    L.avdf_plan_window_layout.argtypes = [c_void_p, c_double, POINTER(c_int64), c_double, c_double, c_int32, POINTER(c_int32),
+                                          POINTER(c_int32), POINTER(c_float), POINTER(c_float)]
+    L.avdf_session_window_bytes.restype = c_size_t
+    L.avdf_session_window_bytes.argtypes = [c_void_p, c_int32, c_int32]
+    L.avdf_session_attach_windows.argtypes = [c_void_p, c_void_p, c_size_t, c_int32, c_int32]
+    L.avdf_session_run_windows.argtypes = [c_void_p, POINTER(WindowRunArgs), c_void_p]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("avdf_last_error", "avdf_nms_workspace_bytes", "avdf_postprocess_workspace_bytes",
                         "avdf_conv_gemm_workspace_bytes", "avdf_eval_workspace_bytes", "avdf_eval_proposal_workspace_bytes",
-                        "avdf_window_merge_workspace_bytes", "avdf_abi_version", "avdf_plan_close", "avdf_session_destroy"):
+                        "avdf_window_merge_workspace_bytes", "avdf_abi_version", "avdf_plan_close", "avdf_session_destroy",
+                        "avdf_session_window_bytes"):
             fn.restype = c_int32
     if L.avdf_abi_version() != 3:
         raise AvdfError("libavdf_sm100.so ABI version mismatch")

@@ -485,7 +485,8 @@ AVDF_API int avdf_h2d_gather(const void* const* src, void* const* dst, const siz
  * Outputs (device, at their max_batch allocations; rows b < B are written):
  *   segs [B, max_seg_num, 2] seconds, scores [B, max_seg_num] (descending), counts int32 [B], video_cls [B] (logit).
  * A session is one buffer set: it runs on one stream at a time. Concurrent batches use separate sessions of one plan
- * (they share its constants). The plan must stay open while it has sessions. */
+ * (they share its constants). The plan must stay open while it has sessions. Recordings longer than the model's
+ * training clips run as sliding windows on a session: avdf_session_attach_windows / avdf_session_run_windows below. */
 typedef struct avdf_plan avdf_plan;          /* parsed plan (host); its constants once uploaded */
 typedef struct avdf_session avdf_session;    /* one buffer set = one batch in flight */
 typedef struct avdf_plan_info {
@@ -515,7 +516,66 @@ AVDF_API int avdf_session_get_io(const avdf_session* s, avdf_session_io* io);
  * capture mode) into a CUDA graph and launches that; later calls launch the graph. `stream` must be a created stream
  * (graph capture is not possible on the legacy default stream). Asynchronous; no host synchronisation. */
 AVDF_API int avdf_session_run(avdf_session* s, int32_t batch, const int64_t rows[3], void* stream);
+/* Releases the session's graphs and, when a window block is attached, its pinned parameter buffer and event. */
 AVDF_API void avdf_session_destroy(avdf_session* s);
+
+/* ---- sliding windows on a session (csrc/plan.cu; the C form of forward_streams(window=W, hop=H),
+ * libs/modeling/windows.py) ----
+ * A recording of D seconds longer than W is cut into n = (int)ceil((D - W) / H) + 1 windows (all in double):
+ *   s_k = min(k * H, D - W); window k of stream s (T_s rows) covers rows [floor(s_k * T_s / D), + floor(W * T_s / D))
+ *   and its meta is the session-run formula above with T = rows of the window in its first stream and duration W;
+ *   win_start[k] = (float)s_k.
+ * D <= W: one window covering every row, its meta from the recording's own T and duration D, win_start 0.
+ * Every window runs through the plan's pass at the model's trained time scale (its first launch replaced by the row-range
+ * resampling avdf_interp_concat_ranges); avdf_window_merge then turns the window results into one result per recording.
+ * The first stream is video if present, else byola (else emo). */
+
+/* HOST only, no CUDA call: the windows of one recording as plan p runs them. Returns n >= 1, or < 0 on bad input
+ * (avdf_last_error: W not > 0 or NaN, hop not in (0, W], a duration that is not a positive finite number, rows for an
+ * absent stream or none for a present one, a window that holds no row of a present stream). When cap >= n (and the
+ * arrays are not NULL) it fills start / count [n][3] (rows relative to the recording, 0 for absent streams),
+ * meta [n][4] (feat_stride, 0.5 * feat_num_frames, fps, duration) and win_start [n]. */
+AVDF_API int32_t avdf_plan_window_layout(const avdf_plan* p, double duration, const int64_t rows[3], double window,
+                                         double hop, int32_t cap, int32_t* start, int32_t* count, float* meta,
+                                         float* win_start);
+/* HOST only: device bytes of a session's window block for calls with at most max_windows windows in all and at most
+ * max_windows_per_recording windows per recording (1 <= max_windows_per_recording <= max_windows <= 2^24). With
+ * B = info.max_batch, K = info.max_seg_num, W = max_windows it is the sum of
+ *   align256(4 * (12 W + 10 B))   window table (per batch [3, B] start, [3, B] count, [4, B] meta; win_start; rec_win)
+ *   align256(24 B)                the fixed [3, B] start and count arrays the windowed graphs read
+ *   align256(8 K W) + align256(4 K W) + align256(4 W) + align256(4 W)   every window's segs, scores, count, video_cls
+ *   avdf_window_merge_workspace_bytes(W, K * max_windows_per_recording)
+ * Returns 0 (avdf_last_error says why) when the limits are out of range or the plan cannot run windows: every launch
+ * list must start with avdf_interp_concat_in reading the io offsets for its own batch size, and hold exactly one
+ * avdf_postprocess that writes the io outputs, keeps no result records and runs hard or soft NMS. */
+AVDF_API size_t avdf_session_window_bytes(const avdf_plan* p, int32_t max_windows, int32_t max_windows_per_recording);
+/* dev: avdf_session_window_bytes of device memory (256-byte aligned) on the plan's device, owned by the caller and kept
+ * until the session is destroyed. Allocates a small pinned host buffer and an event for the per-call parameters.
+ * AVDF_ERR_UNSUPPORTED when the plan cannot run windows (see above); a session takes one window block. */
+AVDF_API int avdf_session_attach_windows(avdf_session* s, void* dev, size_t bytes, int32_t max_windows,
+                                         int32_t max_windows_per_recording);
+typedef struct avdf_window_run_args {
+  int32_t n_rec;                 /* recordings, >= 1 (may exceed max_batch) */
+  const double* duration;        /* host [n_rec] seconds */
+  const int64_t* rows;           /* host [n_rec][3]; the recordings lie back to back in io.streams, in this order */
+  double window, hop;            /* W > 0, 0 < hop <= W (seconds) */
+  float* out_segs;               /* [n_rec, max_seg_num, 2] seconds */
+  float* out_scores;             /* [n_rec, max_seg_num] descending */
+  int32_t* out_count;            /* [n_rec] */
+  float* out_cls;                /* [n_rec] video-level logit (the largest of the recording's windows) */
+} avdf_window_run_args;          /* host struct; out_* are device pointers */
+/* One call over n_rec recordings staged in io.streams (written as for avdf_session_run; the rows of each stream must fit
+ * its staging). Steps, all on `stream`: the windows of every recording (avdf_plan_window_layout) go up as one copy; they
+ * run in recording order in batches of the plan's largest batch size - the last batch, when the plan has no list of its
+ * size, as the smallest recorded size that holds it, its unused slots repeating its last window - each batch being a
+ * device-to-device copy of its ranges and meta, the windowed launch list (eager and captured on the first call for a
+ * size, a graph replay after that) and copies of its results aside; then avdf_window_merge with the NMS settings of the
+ * plan's recorded postprocess and cand_cap = max_seg_num * (most windows of any recording in this call). No host
+ * synchronisation (the pinned parameter buffer is rewritten after an event of the previous call's copy). Refused, with
+ * nothing launched and the outputs untouched: no window block attached, n_rec < 1, bad W / hop or a window without a
+ * row, rows for an absent stream or none for a present one, rows beyond the staging, more windows than max_windows or
+ * more for one recording than max_windows_per_recording, the legacy default stream, another device than the plan's. */
+AVDF_API int avdf_session_run_windows(avdf_session* s, const avdf_window_run_args* a, void* stream);
 
 #ifdef __cplusplus
 }
