@@ -1,5 +1,5 @@
-"""float64 references of the `ops` entry points the localization forward pass launches, one per entry point, with the
-entry point's own keyword arguments.
+"""float64 references of the `ops` entry points the localization forward pass and the BYOL-A extractor launch, one per
+entry point, with the entry point's own keyword arguments.
 
 TEST INFRASTRUCTURE (see oracle/model_ref.py's header).
 
@@ -12,10 +12,13 @@ device of its operands) and returns a dict {output path: Out}. The path names th
   mag      float64 magnitude of the terms the value was summed from, or None (= |ref|). Outputs that are a short
            contraction of long sums (head logits / offsets, row dots, the video-level scalar) are compared against it:
            their value can cancel to far below the size of the fp32 rounding of its terms.
+  tol      float64 per-element absolute error bound, or None (the row-wise bar). The log-mel spectrogram has one: its
+           smallest mel bins sit ~1e-6 below the row's largest, where the fp32 FFT's rounding is all the value holds.
 Operands are what the kernel saw: 16-bit tensors convert exactly to float64. Intermediate roundings are modelled only
 where the code documents them: the 16-bit hidden activations of mlp_fused (csrc/mlp_fused.cu: "-> 16-bit -> shared
 memory") and the 16-bit LN2 operand of the block tail (mlp_fused proj=: "writes the 16-bit x tile").
 """
+import math
 from collections import namedtuple
 
 import numpy as np
@@ -26,7 +29,7 @@ import model_ref
 
 F64 = torch.float64
 ACT_NONE, ACT_RELU, ACT_GELU = 0, 1, 2
-Out = namedtuple("Out", "ref written zero mag")
+Out = namedtuple("Out", "ref written zero mag tol", defaults=(None,))
 
 # a ReLU output counts as a structural zero when its pre-activation is below -RELU_MARGIN x the row's largest magnitude:
 # two orders of magnitude above the fp32 error of the values the kernels clamp
@@ -421,9 +424,114 @@ def vcls_exp13(z, conv0_w, seg_w, seg_b, cls_w, cls_b, out, *, batch, t):
     return {"out": Out(o.reshape(out.shape), ~_false(out), _false(out), mag.reshape(out.shape))}
 
 
+# --------------------------------------------------------------------------------------------------- BYOL-A extractor
+N_FFT, HOP, LOG_EPS, FP32_U = 1024, 160, 2.0 ** -23, 2.0 ** -24
+
+
+def mel_matrix(mel, n_bins=N_FFT // 2 + 1):
+    """The sparse mel triangles (lo [M], cnt [M], w [M, stride]) as a dense float64 [n_bins, M] filterbank."""
+    lo, cnt, w = (t.cpu() for t in mel)
+    fb = torch.zeros((n_bins, lo.numel()), dtype=F64)
+    for m in range(lo.numel()):
+        fb[int(lo[m]):int(lo[m]) + int(cnt[m]), m] = w[m, :int(cnt[m])].to(F64)
+    return fb
+
+
+def logmel(wav, clip_sample_off, clip_frame_off, clip_pair_off, total_pairs, window, twiddle, mel, lms, *, mean, std):
+    """torchaudio's MelSpectrogram (centre framing, reflect padding without edge repeat, power 2) through the `window` and
+    `mel` arguments, then (log(M + 2^-23) - mean) / std; frames of a clip are rows clip_frame_off[c] .. of lms.
+    tol bounds the fp32 FFT's rounding (1024 points, 10 passes): the two frames 2j, 2j + 1 of a clip share one complex
+    FFT and are separated by conjugate symmetry, so the error of either grows with the energy of both,
+        d_f = 2^-24 log2(1024) sqrt(|x_A|^2 + |x_B|^2)
+        tol = sum_k fb[k, m] (2 |X_k| d_f + d_f^2) / (M_m + 2^-23) / std + 8 2^-24 (|log(M_m + 2^-23)| + |mean|) / std
+    (the second term: power, mel accumulation, log and normalisation in fp32). An odd last frame pairs with zeros."""
+    dev = lms.device
+    so, fo = clip_sample_off.cpu().tolist(), clip_frame_off.cpu().tolist()
+    fb = mel_matrix(mel).to(dev)
+    win = _f(window).to(dev)
+    x = _f(wav).to(dev)
+    ref = torch.empty(lms.shape, dtype=F64, device=dev)
+    tol = torch.empty_like(ref)
+    for c in range(len(fo) - 1):
+        nf = fo[c + 1] - fo[c]
+        padded = torch.nn.functional.pad(x[so[c]:so[c + 1]][None, None], (N_FFT // 2, N_FFT // 2), mode="reflect")[0, 0]
+        frames = padded.unfold(0, N_FFT, HOP)[:nf] * win
+        X = torch.fft.rfft(frames, dim=1).abs()
+        M = (X * X) @ fb
+        lg = torch.log(M + LOG_EPS)
+        ref[fo[c]:fo[c + 1]] = (lg - mean) / std
+        e2 = frames.pow(2).sum(dim=1)
+        e2 = torch.cat([e2, e2.new_zeros(nf % 2)]).reshape(-1, 2).sum(dim=1).repeat_interleave(2)[:nf]
+        d = (FP32_U * math.log2(N_FFT) * e2.sqrt())[:, None]
+        tol[fo[c]:fo[c + 1]] = ((2 * X * d + d * d) @ fb) / (M + LOG_EPS) / std + 8 * FP32_U * (lg.abs() + abs(mean)) / std
+    return {"lms": Out(ref, ~_false(lms), _false(lms), None, tol)}
+
+
+def _clip_rows(clip_of_step, t_of_step, counts):
+    """Live steps of a grid (clip_of_step >= 0) and, for each, its row in the clips' outputs stacked in clip order
+    (clip c has counts[c] rows)."""
+    clip, t = clip_of_step.long(), t_of_step.long().to(clip_of_step.device)
+    live = clip >= 0
+    off = torch.cat([counts.new_zeros(1), counts.cumsum(0)[:-1]]).to(clip.device)
+    return live, off[clip.clamp_min(0)] + t
+
+
+def byola_conv1_pool(lms, clip_frame_off, w, b, clip_of_step, t_of_step, out, mask_out=None):
+    """features.0-3 (byol_a/models.py:54-57) into the level-1 grid layout: step s, mel slot 1..32 of a clip holds
+    ReLU(max over the 2x2 window of conv2d(lms_c zero-padded, w as [out, 1, mel tap, time tap]) + b); the two padding
+    slots of every step and every step of no clip are zero; mask_out = the live pattern."""
+    dev = out.device
+    fo = clip_frame_off.cpu().tolist()
+    W, B = _f(w).to(dev).reshape(64, 1, 3, 3), _f(b).to(dev)
+    L = _f(lms).to(dev)
+    pooled = []
+    for c in range(len(fo) - 1):
+        img = L[fo[c]:fo[c + 1]].t()[None, None]                     # (1, 1, mel, frame)
+        y = torch.nn.functional.max_pool2d(torch.nn.functional.conv2d(img, W, B, padding=1), 2)[0]
+        pooled.append(y.permute(2, 1, 0))                              # [frame // 2, 32, 64]
+    counts = torch.tensor([p.shape[0] for p in pooled])
+    live, row = _clip_rows(clip_of_step.to(dev), t_of_step, counts)
+    pre = torch.zeros((live.numel(), 34, 64), dtype=F64, device=dev)
+    pre[live, 1:33] = torch.cat(pooled)[row[live]]
+    slot = torch.zeros((live.numel(), 34), dtype=torch.bool, device=dev)
+    slot[live, 1:33] = True
+    ref, zero = _relu(pre, ~slot[..., None].expand(pre.shape))
+    outs = {"out": Out(ref.reshape(out.shape), ~_false(out), zero.reshape(out.shape), None)}
+    if mask_out is not None:
+        outs["mask_out"] = Out(slot.to(F64).reshape(mask_out.shape), ~_false(mask_out), _false(mask_out), None)
+    return outs
+
+
+def byola_pool(x, clip_step_in, clip_of_step, t_of_step, out, *, mel_in, pad_out, mask_out=None):
+    """MaxPool2d(2) of every clip's mel_in x time block of the input grid (clip c's steps start at clip_step_in[c]) into
+    the next grid (pad_out = 1: mel slot 1 .. mel_in / 2 of a step) or the fc rows (pad_out = 0: one row per step,
+    mel * 64 + channel, byol_a/models.py:80-81); every other element is zero. The values are stored values: exact."""
+    dev = out.device
+    mo, st = mel_in // 2, clip_step_in.cpu().tolist()
+    X = _f(x).to(dev).reshape(-1, mel_in + 2, 64)
+    clip = clip_of_step.to(dev).long()
+    counts = torch.bincount(clip[clip >= 0].cpu(), minlength=len(st))
+    pooled = []
+    for c, n in enumerate(counts.tolist()):
+        if n == 0:
+            pooled.append(X.new_zeros((0, mo, 64)))
+            continue
+        img = X[st[c]:st[c] + 2 * n, 1:mel_in + 1].permute(2, 1, 0)[None]        # (1, 64, mel, step)
+        pooled.append(torch.nn.functional.max_pool2d(img, 2)[0].permute(2, 1, 0))  # [n, mo, 64]
+    live, row = _clip_rows(clip, t_of_step, counts)
+    ref = torch.zeros((live.numel(), mo + 2 * pad_out, 64), dtype=F64, device=dev)
+    ref[live, pad_out:pad_out + mo] = torch.cat(pooled)[row[live]]
+    slot = torch.zeros(ref.shape[:2], dtype=torch.bool, device=dev)
+    slot[live, pad_out:pad_out + mo] = True
+    outs = {"out": Out(ref.reshape(out.shape), ~_false(out), (~slot[..., None]).expand(ref.shape).reshape(out.shape), None)}
+    if mask_out is not None:
+        outs["mask_out"] = Out(slot.to(F64).reshape(mask_out.shape), ~_false(mask_out), _false(mask_out), None)
+    return outs
+
+
 REFERENCES = {f.__name__: f for f in (interp_concat, interp_concat_ranges, pack_feats, conv_gemm, mlp_fused, ln_dwconv_ln,
                                       attention, ln_rows, instnorm_lrelu, fpn_fuse, head_final, head_combine, vcls_exp12,
-                                      vcls_exp13)}
+                                      vcls_exp13, logmel, byola_conv1_pool, byola_pool)}
 # entry points the forward pass launches that have no reference here, and why
 EXCLUDED = {"postprocess": "decode + NMS + seconds conversion: compared bit for bit with the C oracle (oracle/nms_ref.c) "
                            "in tests/test_gpu_kernels.py and tests/test_gpu_model.py"}
@@ -437,26 +545,37 @@ def ulp(x, dtype):
 
 
 def check(got, o, width, bar, what=""):
-    """Asserts a kernel output against its reference Out: structural zeros exactly 0, and the row-wise error
-    max|got - ref| / max(|ref|, mag) over rows of `width` values within `bar` (16-bit outputs: beyond one ulp of their
-    type at |ref|). Returns the worst row-wise error."""
+    """Asserts a kernel output against its reference Out: integer outputs equal; structural zeros exactly 0; with a
+    per-element bound o.tol, |got - ref| <= bar * tol everywhere; otherwise the row-wise error max|got - ref| /
+    max(|ref|, mag) over rows of `width` values within `bar` (16-bit outputs: beyond one ulp of their type at |ref|;
+    bar 0 asks for exact values, without that ulp). Returns the worst row-wise error (err / tol with a bound)."""
     ref, written = o.ref.to(got.device), o.written.to(got.device)
+    if not got.is_floating_point():
+        if not torch.equal(got[written].to(F64), ref[written]):
+            i = tuple(int(v) for v in ((got.to(F64) != ref) & written).nonzero()[0])
+            raise AssertionError("%s: element %s is %d, expected %d" % (what, i, int(got[i]), int(ref[i])))
+        return 0.0
     mag = ref.abs() if o.mag is None else o.mag.to(got.device)
     bad = o.zero.to(got.device) & written & (got != 0)
     if bool(bad.any()):
         i = tuple(int(v) for v in bad.nonzero()[0])
         raise AssertionError("%s: element %s must be exactly 0, got %r" % (what, i, float(got[i])))
     err = (got.to(F64) - ref).abs()
-    if got.dtype in (torch.float16, torch.bfloat16):
-        err = (err - ulp(ref, got.dtype)).clamp_min(0.0)
-    err = torch.where(written, err, torch.zeros_like(err)).reshape(-1, width)
-    denom = torch.maximum(ref.abs(), mag).reshape(-1, width).amax(dim=1, keepdim=True).clamp_min(1e-30)
-    rel = torch.nan_to_num(err / denom, nan=float("inf"))
+    if o.tol is not None:
+        rel = torch.where(written, torch.nan_to_num(err / o.tol.to(got.device), nan=float("inf")), torch.zeros_like(err))
+        kind = "error / bound"
+    else:
+        if got.dtype in (torch.float16, torch.bfloat16) and bar > 0:
+            err = (err - ulp(ref, got.dtype)).clamp_min(0.0)
+        err = torch.where(written, err, torch.zeros_like(err)).reshape(-1, width)
+        denom = torch.maximum(ref.abs(), mag).reshape(-1, width).amax(dim=1, keepdim=True).clamp_min(1e-30)
+        rel = torch.nan_to_num(err / denom, nan=float("inf"))
+        kind = "row-wise error"
     worst = float(rel.max())
     if worst > bar:
         idx = tuple(int(v) for v in torch.unravel_index(rel.reshape(-1).argmax().cpu(), ref.shape))
-        raise AssertionError("%s: row-wise error %.3g > bar %.1g at %s: got %r, float64 reference %r" %
-                             (what, worst, bar, idx, float(got[idx]), float(ref[idx])))
+        raise AssertionError("%s: %s %.3g > bar %.1g at %s: got %r, float64 reference %r" %
+                             (what, kind, worst, bar, idx, float(got[idx]), float(ref[idx])))
     return worst
 
 

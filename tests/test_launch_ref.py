@@ -1,6 +1,7 @@
 """CPU checks of the float64 per-launch references (oracle/launch_ref.py) against independent torch formulations
-(nn.Conv1d / ConvTranspose1d / Conv2d, nn.LayerNorm, nn.InstanceNorm1d, F.interpolate, a dense band-masked softmax),
-their mask semantics, and a static check that every `ops` entry point the forward pass calls has a reference."""
+(nn.Conv1d / ConvTranspose1d / Conv2d, nn.LayerNorm, nn.InstanceNorm1d, F.interpolate, a dense band-masked softmax,
+torch.stft, BatchNorm + MaxPool2d), their mask semantics and error bounds, and a static check that every `ops` entry
+point the forward pass and the BYOL-A extractor call has a reference."""
 import math
 import os
 import re
@@ -10,8 +11,11 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+import byola_ref
 import launch_ref as lr
+from audio_visual_deepfake_detection_b200.libs.features.byola import BatchPlan, LogMelSpectrogram
 from audio_visual_deepfake_detection_b200.libs.modeling.engine import up_weight
+from audio_visual_deepfake_detection_b200.libs.utils import synthetic as syn
 
 D = torch.float64
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -334,10 +338,186 @@ def test_interp_concat_and_pack_feats():
     assert torch.equal(p.ref[:5], f.t().to(D)) and bool((p.ref[5:] == 0).all()) and bool(p.zero[5:].all()) and not p.zero[:5].any()
 
 
+# --------------------------------------------------------------------------------------------------- BYOL-A extractor
+def _logmel_call(wavs, window=None):
+    """lr.logmel on the host with the extractor's own tables (LogMelSpectrogram) and plan (BatchPlan)."""
+    lm = LogMelSpectrogram("cpu")
+    plan = BatchPlan([w.shape[0] for w in wavs], "cpu")
+    o = lr.logmel(torch.from_numpy(np.concatenate(wavs)), plan.d_sample_off, plan.d_frame_off, plan.d_pair_off, plan.total_pairs,
+                  lm.window if window is None else window, lm.twiddle, lm.mel, torch.empty(plan.total_frames, 64),
+                  mean=lm.stats[0], std=lm.stats[1])["lms"]
+    return o, plan
+
+
+def _lms_of_frames(frames):
+    """The plain log-mel formula on float64 windowed frames [F, 1024]."""
+    fb = torch.from_numpy(byola_ref.mel_filterbank()).to(D)
+    M = torch.fft.rfft(frames, dim=1).abs().pow(2) @ fb
+    return (torch.log(M + lr.LOG_EPS) - byola_ref.NORM_STATS[0]) / byola_ref.NORM_STATS[1]
+
+
+def _logmel_clips():
+    onset = np.zeros(16000 * 2, np.float32)                     # digital silence, then a full-scale onset
+    onset[20000:] = np.clip(3.0 * syn.synthetic_wav(12000, 5), -1.0, 1.0)
+    return [syn.synthetic_wav(9000, 11), syn.synthetic_wav(1279, 12), onset]
+
+
+def test_logmel_reference_is_stft_and_bounds_the_fp32_pipeline():
+    """float64 torch.stft (centre, reflect, periodic Hann) agrees with the reference; the CPU oracle's fp32 pipeline (numpy
+    FFT, fp32 power / mel / log) stays inside the per-element bound on speech-like audio and after digital silence."""
+    wavs = _logmel_clips()
+    o, plan = _logmel_call(wavs)
+    assert o.written.all() and o.tol is not None and bool((o.tol > 0).all())
+    hann = LogMelSpectrogram("cpu").window.to(D)                   # the fp32 window the kernel multiplies by: periodic Hann
+    assert float((hann - torch.hann_window(1024, periodic=True, dtype=D)).abs().max()) < 2 ** -23
+    for c, w in enumerate(wavs):
+        rows = slice(int(plan.frame_off[c]), int(plan.frame_off[c + 1]))
+        S = torch.stft(torch.from_numpy(w).to(D), 1024, 160, window=hann, center=True, pad_mode="reflect", return_complex=True)
+        M = S.abs().pow(2).t() @ torch.from_numpy(byola_ref.mel_filterbank()).to(D)
+        want = (torch.log(M + lr.LOG_EPS) - byola_ref.NORM_STATS[0]) / byola_ref.NORM_STATS[1]
+        assert float((o.ref[rows] - want).abs().max()) < 1e-12
+        got = torch.from_numpy(byola_ref.log_mel(w)).t().to(D)
+        worst = float(((got - o.ref[rows]).abs() / o.tol[rows]).max())
+        assert worst <= 1.0, (c, worst)
+
+
+def test_logmel_bound_rejects_framing_and_window_mutants():
+    """A symmetric Hann window, edge-repeat reflect padding, a hop of 161: each misses the bound by >= 100x."""
+    wavs = _logmel_clips()[:1]
+    o, _ = _logmel_call(wavs)
+    w = wavs[0].astype(np.float64)
+    nf = 1 + w.shape[0] // 160
+    hann = LogMelSpectrogram("cpu").window.double().numpy()
+
+    def frames(padded, hop):
+        idx = np.minimum(np.arange(nf)[:, None] * hop + np.arange(1024)[None], padded.shape[0] - 1)
+        return torch.from_numpy(padded[idx] * hann)
+
+    sym = torch.from_numpy((0.5 - 0.5 * np.cos(2.0 * np.pi * np.arange(1024) / 1023)).astype(np.float32))
+    mutants = {"symmetric Hann": _logmel_call(wavs, window=sym)[0].ref,
+               "edge-repeat padding": _lms_of_frames(frames(np.pad(w, 512, mode="symmetric"), 160)),
+               "hop 161": _lms_of_frames(frames(np.pad(w, 512, mode="reflect"), 161))}
+    assert float(((_lms_of_frames(frames(np.pad(w, 512, mode="reflect"), 160)) - o.ref).abs() / o.tol).max()) < 1e-3
+    for name, m in mutants.items():
+        assert m.shape == o.ref.shape
+        assert float(((m - o.ref).abs() / o.tol).max()) >= 100.0, name
+
+
+def test_logmel_twiddle_table_is_fp32_exp_minus_i():
+    j = torch.arange(1024, dtype=D) * (2.0 * math.pi / 1024)
+    assert torch.equal(LogMelSpectrogram("cpu").twiddle, torch.stack([torch.cos(j), -torch.sin(j)], 1).float())
+
+
+def _byola_sd():
+    return {k: torch.as_tensor(v, dtype=D) for k, v in syn.synthetic_byola_state_dict(0).items()}
+
+
+def _folded(sd, conv, bn):
+    """BatchNorm (eval) folded into the preceding convolution, in float64."""
+    scale = sd["features.%d.weight" % bn] / torch.sqrt(sd["features.%d.running_var" % bn] + 1e-5)
+    return (sd["features.%d.weight" % conv] * scale[:, None, None, None],
+            sd["features.%d.bias" % bn] + (sd["features.%d.bias" % conv] - sd["features.%d.running_mean" % bn]) * scale)
+
+
+def _bn_block(x, sd, conv, bn):
+    """conv3x3 -> BatchNorm (eval) -> ReLU -> MaxPool 2x2 of byol_a/models.py:54-67, unfolded."""
+    c, n = "features.%d." % conv, "features.%d." % bn
+    y = F.conv2d(x, sd[c + "weight"], sd[c + "bias"], padding=1)
+    y = F.batch_norm(y, sd[n + "running_mean"], sd[n + "running_var"], sd[n + "weight"], sd[n + "bias"], training=False, eps=1e-5)
+    return F.max_pool2d(F.relu(y), 2)
+
+
+def test_byola_conv1_pool_is_conv_bn_relu_maxpool():
+    """Three clips (8, 23 and 40 frames) packed as BatchPlan lays them out: every live slot of the level-1 grid equals
+    features.0-3 on the clip alone; padding slots and steps of no clip are zero; mask_out is the live pattern. Weights
+    with the mel and time taps swapped do not match."""
+    r = g(40)
+    frames = [8, 23, 40]
+    plan = BatchPlan(None, "cpu", frames=frames)
+    clips = [rn(r, 64, f) - 1.0 for f in frames]
+    lms = torch.cat([c.t() for c in clips]).float()
+    sd = _byola_sd()
+    w, b = _folded(sd, 0, 1)
+    out, mo = torch.empty(plan.steps1 * 34, 64), torch.empty(plan.steps1 * 34, dtype=torch.uint8)
+    got = lr.byola_conv1_pool(lms, plan.d_frame_off, w.reshape(64, 9), b, plan.d_clip1, plan.d_t1, out, mo)
+    ref = got["out"].ref.reshape(plan.steps1, 34, 64)
+    live = torch.zeros(plan.steps1, 34, dtype=torch.bool)
+    for c, f in enumerate(frames):
+        s0 = int(plan.d_start1[c])
+        want = _bn_block(lms[plan.frame_off[c]:plan.frame_off[c + 1]].t().to(D)[None, None], sd, 0, 1)[0]   # (64, 32, f // 2)
+        close(ref[s0:s0 + f // 2, 1:33], want.permute(2, 1, 0))
+        live[s0:s0 + f // 2, 1:33] = True
+    assert bool((ref[~live] == 0).all()) and bool(got["out"].zero.reshape(plan.steps1, 34, 64)[~live].all())
+    assert torch.equal(got["mask_out"].ref.reshape(plan.steps1, 34), live.to(D))
+    assert bool((ref[live] == 0).any() and (ref[live] > 0).any())            # the ReLU is alive
+    swapped = w.transpose(2, 3).reshape(64, 9)
+    bad = lr.byola_conv1_pool(lms, plan.d_frame_off, swapped, b, plan.d_clip1, plan.d_t1, out, mo)["out"].ref
+    assert float((bad - got["out"].ref).abs().max() / got["out"].ref.abs().max()) > 1e-2
+
+
+@pytest.mark.parametrize("pad_out", [1, 0])
+def test_byola_pool_is_maxpool_and_fc_row_flattening(pad_out):
+    """MaxPool2d(2) of every clip of a level-1 (pad_out 1: into the level-2 grid) or level-2 grid (pad_out 0: into the fc
+    rows, flattened mel * 64 + channel like byol_a/models.py:80-81 / byola_ref.forward); everything else is zero."""
+    r = g(50 + pad_out)
+    frames = [8, 29, 44]
+    plan = BatchPlan(None, "cpu", frames=frames)
+    lvl = 1 if pad_out else 2
+    mel = 32 if pad_out else 16
+    steps_in, start_in, t_in = (plan.steps1, plan.d_start1, plan.t[1]) if pad_out else (plan.steps2, plan.d_start2, plan.t[2])
+    clip_out, t_out = (plan.d_clip2, plan.d_t2) if pad_out else (plan.d_clip3, plan.d_t3)
+    x = torch.zeros(steps_in, mel + 2, 64, dtype=torch.float16)
+    imgs = []
+    for c in range(len(frames)):
+        v = torch.relu(rn(r, t_in[c], mel, 64)).to(torch.float16)
+        x[int(start_in[c]):int(start_in[c]) + t_in[c], 1:mel + 1] = v
+        imgs.append(v.to(D).permute(2, 1, 0)[None])                      # (1, ch, mel, time)
+    n_out = clip_out.numel()
+    out = torch.empty(n_out * (mel // 2 + 2 * pad_out), 64) if pad_out else torch.empty(n_out, 8 * 64)
+    o = lr.byola_pool(x.reshape(-1, 64), start_in, clip_out, t_out, out, mel_in=mel, pad_out=pad_out,
+                      mask_out=torch.empty(out.numel() // 64, dtype=torch.uint8) if pad_out else None)
+    assert (("mask_out" in o) == bool(pad_out)) and o["out"].written.all()
+    for c in range(len(frames)):
+        p = F.max_pool2d(imgs[c], 2)                                       # (1, ch, mel // 2, time // 2)
+        assert p.shape[-1] == frames[c] >> (lvl + 1)
+        if pad_out:
+            s0 = int(plan.d_start2[c])
+            got = o["out"].ref.reshape(n_out, mel // 2 + 2, 64)[s0:s0 + p.shape[-1], 1:mel // 2 + 1]
+            assert torch.equal(got, p[0].permute(2, 1, 0))
+        else:
+            r0 = int(plan.row_off3[c])
+            got = o["out"].ref[r0:r0 + p.shape[-1]]
+            assert torch.equal(got, p.permute(0, 3, 2, 1).reshape(p.shape[-1], -1))       # byola_ref.forward's flattening
+    live = o["out"].ref.new_zeros(o["out"].ref.shape, dtype=torch.bool)
+    if pad_out:
+        live = o["mask_out"].ref.reshape(-1, 1).expand(-1, 64).reshape(out.shape) != 0
+        assert int(o["mask_out"].ref.sum()) == sum(f >> 2 for f in frames) * (mel // 2)
+    else:
+        live[:int(plan.row_off3[-1])] = True
+    assert torch.equal(o["out"].zero, ~live) and bool((o["out"].ref[~live] == 0).all())
+
+
+def test_check_bound_exact_and_integer_paths():
+    ref = torch.tensor([[1.0, 2.0], [3.0, 4.0]], dtype=D)
+    w, z = torch.ones(2, 2, dtype=torch.bool), torch.zeros(2, 2, dtype=torch.bool)
+    tol = torch.full((2, 2), 1e-3, dtype=D)
+    assert lr.check((ref + 5e-4).float(), lr.Out(ref, w, z, None, tol), 2, 1.0) == pytest.approx(0.5, rel=1e-3)
+    with pytest.raises(AssertionError, match="error / bound"):
+        lr.check((ref + 2e-3).float(), lr.Out(ref, w, z, None, tol), 2, 1.0)
+    assert lr.check(ref.to(torch.bfloat16), lr.Out(ref, w, z, None), 2, 0.0) == 0.0
+    with pytest.raises(AssertionError):                        # bar 0: one ulp off is an error
+        lr.check((ref + 2 ** -6).to(torch.bfloat16), lr.Out(ref, w, z, None), 2, 0.0)
+    m = torch.tensor([0, 1, 1], dtype=torch.uint8)
+    assert lr.check(m, lr.Out(m.to(D), torch.ones(3, dtype=torch.bool), torch.zeros(3, dtype=torch.bool), None), 1, 0.0) == 0.0
+    with pytest.raises(AssertionError, match="element"):
+        lr.check(m, lr.Out(torch.tensor([0.0, 1.0, 0.0], dtype=D), torch.ones(3, dtype=torch.bool), torch.zeros(3, dtype=torch.bool), None), 1, 0.0)
+
+
 # --------------------------------------------------------------------------------------------------- coverage
 def launched_entry_points():
     names = set()
-    for rel in ("audio_visual_deepfake_detection_b200/libs/modeling/engine.py", "audio_visual_deepfake_detection_b200/libs/modeling/meta_archs.py"):
+    for rel in ("audio_visual_deepfake_detection_b200/libs/modeling/engine.py", "audio_visual_deepfake_detection_b200/libs/modeling/meta_archs.py",
+                "audio_visual_deepfake_detection_b200/libs/features/byola.py"):
         with open(os.path.join(ROOT, rel)) as f:
             names |= set(re.findall(r"\bops\.(\w+)\(", f.read()))
     return names
@@ -347,6 +527,7 @@ def test_every_launched_entry_point_has_a_reference():
     from audio_visual_deepfake_detection_b200 import ops
     names = launched_entry_points()
     assert {"conv_gemm", "attention", "mlp_fused", "ln_dwconv_ln"} <= names
+    assert {"logmel", "byola_conv1_pool", "byola_pool"} <= names
     missing = sorted(n for n in names if n not in lr.REFERENCES and n not in lr.EXCLUDED)
     assert not missing, "ops entry points launched by the forward pass without a float64 reference: %s" % missing
     assert set(lr.EXCLUDED) == {"postprocess"}
