@@ -14,7 +14,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["runtime.cu", "interp.cu", "nms.cu", "gemm_simt.cu", "gemm_tc.cu", "mlp_fused.cu", "blocks.cu", "host_pack.cu", "attention_mma.cu", "byola.cu", "eval.cu", "window.cu", "plan.cu"]
+SOURCES = ["runtime.cu", "interp.cu", "nms.cu", "gemm_simt.cu", "gemm_tc.cu", "mlp_fused.cu", "blocks.cu", "host_pack.cu", "attention_mma.cu", "byola.cu", "eval.cu", "window.cu", "plan.cu", "results.cu"]
 LIB = os.path.join(HERE, "libavdf_sm100.so")
 OBJ_DIR = os.path.join(HERE, "build")
 

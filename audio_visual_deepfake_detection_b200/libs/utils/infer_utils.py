@@ -1,7 +1,6 @@
 """Inference driver with the reference's interface (libs/utils/train_utils.py:510-596
 `inference_one_epoch`, :22-40 `fix_random_seed`, `valid_one_epoch`). Training utilities (optimizer,
 scheduler, EMA, checkpoint saving) are outside the accelerated path."""
-import json
 import os
 import pickle
 import random
@@ -9,6 +8,10 @@ import time
 
 import numpy as np
 import torch
+
+from ...native import AvdfError
+from .result_writer import write_result_records
+from .sharding import record_width
 
 
 class AverageMeter(object):
@@ -41,29 +44,62 @@ def result_item(video_id, out):
             "segments": out["segments"].numpy().tolist() if n else []}
 
 
+def pack_outputs(outputs):
+    """Model output dicts (segments [n, 2], scores [n], video_cls [1], fp32) -> (records fp32 [len, 3 + 3K], K) in the
+    layout of sharding.pack_records with K = the largest n (at least 1) and index 0; one scatter per field."""
+    n = torch.tensor([int(o["scores"].shape[0]) for o in outputs], dtype=torch.long)
+    K = max(1, int(n.max())) if len(outputs) else 1
+    rec = torch.zeros((len(outputs), record_width(K)), dtype=torch.float32)
+    if not outputs:
+        return rec, K
+    rec[:, 1] = n.float()
+    rec[:, 2] = torch.cat([o["video_cls"].reshape(-1)[:1] for o in outputs]).float()
+    valid = torch.arange(K)[None, :] < n[:, None]
+    rec[:, 3:3 + K][valid] = torch.cat([o["scores"].reshape(-1) for o in outputs]).float()
+    rec[:, 3 + K:].view(len(outputs), K, 2)[valid] = torch.cat([o["segments"].reshape(-1, 2) for o in outputs]).float()
+    return rec, K
+
+
+def one_epoch_records(val_loader, model, output_folder, dump_every=5000):
+    """The loop of inference_one_epoch: runs `model(video_list)` over the loader and writes `data_left<iter>.json` every
+    `dump_every` iterations plus a final `data_left.json` through the GPU writer. Returns the files written, in order, as
+    (file name, ids, records on the device, K), and the model outputs of the last dump window."""
+    model.eval()
+    os.makedirs(output_folder, exist_ok=True)
+    device = torch.device("cuda", torch.cuda.current_device()) if torch.cuda.is_available() else None
+    files, ids, outs = [], [], []
+
+    def dump(name):
+        rec, K = pack_outputs(outs)
+        if device is None:
+            raise AvdfError("inference_one_epoch writes its results on sm_100a kernels; no CUDA device is visible")
+        rec = rec.to(device)
+        write_result_records(os.path.join(output_folder, name), ids, rec, K)
+        files.append((name, list(ids), rec, K))
+    for iter_idx, video_list in enumerate(val_loader, 0):
+        if iter_idx > 0 and iter_idx % dump_every == 0:
+            dump(f"data_left{iter_idx}.json")
+            ids, outs = [], []
+        with torch.no_grad():
+            output = model(video_list)
+        for vid_idx in range(len(output)):
+            ids.append(video_list[vid_idx]["video_id"])
+            outs.append(output[vid_idx])
+    if len(outs) > 0:
+        dump("data_left.json")
+    return files, list(zip(ids, outs))
+
+
 def inference_one_epoch(val_loader, model, curr_epoch, ext_score_file=None, evaluator=None, output_folder=None,
                         tb_writer=None, print_freq=20, subset="test", max_avg_nr_proposal=100, dataset_name="",
                         dump_every=5000):
     """Runs `model(video_list)` over the loader and writes `data_left<iter>.json` every `dump_every`
-    iterations plus a final `data_left.json` (train_utils.py:546-595). Returns the records of the last dump
-    window (the reference returns None; callers ignore it)."""
+    iterations plus a final `data_left.json` (train_utils.py:546-595), with the bytes json.dump writes (the text is
+    formatted on the GPU, libs/utils/result_writer.py). Returns the records of the last dump window (the reference
+    returns None; callers ignore it)."""
     assert (evaluator is not None) or (output_folder is not None)
-    model.eval()
-    os.makedirs(output_folder, exist_ok=True)
-    batch_results = []
-    for iter_idx, video_list in enumerate(val_loader, 0):
-        if iter_idx > 0 and iter_idx % dump_every == 0:
-            with open(f"{output_folder}/data_left{iter_idx}.json", "w", encoding="utf-8") as f:
-                json.dump(batch_results, f, ensure_ascii=False, indent=4)
-            batch_results = []
-        with torch.no_grad():
-            output = model(video_list)
-        for vid_idx in range(len(output)):
-            batch_results.append(result_item(video_list[vid_idx]["video_id"], output[vid_idx]))
-    if len(batch_results) > 0:
-        with open(f"{output_folder}/data_left.json", "w", encoding="utf-8") as f:
-            json.dump(batch_results, f, ensure_ascii=False, indent=4)
-    return batch_results
+    _, last = one_epoch_records(val_loader, model, output_folder, dump_every)
+    return [result_item(vid, out) for vid, out in last]
 
 
 def valid_one_epoch(val_loader, model, curr_epoch, ext_score_file=None, evaluator=None, output_file=None, tb_writer=None,
@@ -110,18 +146,11 @@ def valid_one_epoch(val_loader, model, curr_epoch, ext_score_file=None, evaluato
     return mAP
 
 
-def inference_sharded(dataset, model, output_folder, batch_size=32, rank=0, world=1, print_freq=0, window=None, hop=None):
-    """Multi-GPU form of inference_one_epoch: one process per GPU (torchrun), rank r takes videos r, r + world, ... of the
-    dataset (the reference splits its list into 7 files run as 7 processes, libs/datasets/deepfake_video_audio.py:420-431,
-    inference.py:116-124); each rank streams its shard through `model.stream` (pinned staging, H2D, CUDA graph), the
-    postprocess kernel appends one fixed-size record per video to a device ring, and ONE all-gather of those records
-    (NCCL) is the path's only exchange. Rank 0 writes `data_left.json` in dataset order, exactly the records
-    inference_one_epoch writes for the same list. Returns the records on rank 0, None elsewhere.
-
-    window / hop (seconds): recordings longer than `window` run as overlapping windows merged on the GPU
-    (model.forward_streams(..., window, hop)); still one record per recording. Per-window metadata uses the dataset's
-    feat_stride / num_frames."""
-    from .sharding import gather_records, shard_indices, unpack_records
+def sharded_records(dataset, model, output_folder, batch_size=32, rank=0, world=1, print_freq=0, window=None, hop=None):
+    """The work of inference_sharded up to its file: streams this rank's shard, all-gathers the records and writes
+    `data_left.json` on rank 0 from the gathered device records. Returns (ids in dataset order, records, order, K) on
+    rank 0 (order[j] = the record row of video j), None elsewhere."""
+    from .sharding import gather_records, shard_indices
     model.eval()
     n = len(dataset)
     mine = shard_indices(n, rank, world)
@@ -157,10 +186,34 @@ def inference_sharded(dataset, model, output_folder, batch_size=32, rank=0, worl
         runner.enable_records(None)
     if rank != 0:
         return None
-    by_index = unpack_records(rec, K)
-    assert len(by_index) == n, (len(by_index), n)
-    results = [result_item(dataset.data_list[j]["id"], by_index[j]) for j in range(n)]
+    index = rec[:, 0]
+    valid = index >= 0
+    order = torch.full((n,), -1, dtype=torch.int32, device=rec.device)
+    order[index[valid].long()] = torch.nonzero(valid).reshape(-1).int()
+    assert int(valid.sum()) == n and bool((order >= 0).all()), (int(valid.sum()), n)
+    ids = [dataset.data_list[j]["id"] for j in range(n)]
     os.makedirs(output_folder, exist_ok=True)
-    with open(f"{output_folder}/data_left.json", "w", encoding="utf-8") as f:
-        json.dump(results, f, ensure_ascii=False, indent=4)
-    return results
+    write_result_records(f"{output_folder}/data_left.json", ids, rec, K, order)
+    return ids, rec, order, K
+
+
+def inference_sharded(dataset, model, output_folder, batch_size=32, rank=0, world=1, print_freq=0, window=None, hop=None):
+    """Multi-GPU form of inference_one_epoch: one process per GPU (torchrun), rank r takes videos r, r + world, ... of the
+    dataset (the reference splits its list into 7 files run as 7 processes, libs/datasets/deepfake_video_audio.py:420-431,
+    inference.py:116-124); each rank streams its shard through `model.stream` (pinned staging, H2D, CUDA graph), the
+    postprocess kernel appends one fixed-size record per video to a device ring, and ONE all-gather of those records
+    (NCCL) is the path's only exchange. Rank 0 writes `data_left.json` in dataset order from the gathered device records
+    (the text is formatted on the GPU, libs/utils/result_writer.py), exactly the bytes inference_one_epoch writes for the
+    same list. Returns the records on rank 0, None elsewhere.
+
+    window / hop (seconds): recordings longer than `window` run as overlapping windows merged on the GPU
+    (model.forward_streams(..., window, hop)); still one record per recording. Per-window metadata uses the dataset's
+    feat_stride / num_frames."""
+    from .sharding import unpack_records
+    res = sharded_records(dataset, model, output_folder, batch_size, rank, world, print_freq, window, hop)
+    if res is None:
+        return None
+    ids, rec, _, K = res
+    by_index = unpack_records(rec, K)
+    assert len(by_index) == len(ids), (len(by_index), len(ids))
+    return [result_item(ids[j], by_index[j]) for j in range(len(ids))]

@@ -32,6 +32,7 @@ EXPORTS = [
     "avdf_plan_open", "avdf_plan_get_info", "avdf_plan_upload", "avdf_plan_close",
     "avdf_session_create", "avdf_session_get_io", "avdf_session_run", "avdf_session_destroy",
     "avdf_plan_window_layout", "avdf_session_window_bytes", "avdf_session_attach_windows", "avdf_session_run_windows",
+    "avdf_format_results_workspace_bytes", "avdf_format_results",
 ]
 
 
@@ -154,6 +155,17 @@ class WindowRunArgs(Structure):
     ]
 
 
+class FormatArgs(Structure):
+    _fields_ = [
+        ("mode", c_int32), ("K", c_int32), ("records", c_void_p), ("n_records", c_int64), ("order", c_void_p), ("n_pos", c_int64),
+        ("ids", c_void_p), ("id_off", c_void_p), ("id_bytes_max", c_int32), ("pos_begin", c_int64), ("n_rows", c_int32),
+        ("min_score", c_double), ("out", c_void_p), ("out_capacity", c_size_t), ("out_bytes", c_void_p),
+        ("workspace", c_void_p), ("workspace_bytes", c_size_t),
+    ]
+
+
+FORMAT_RECORDS, FORMAT_PREDICTIONS = 0, 1
+
 # status bits of avdf_eval_detection / avdf_eval_proposal (AVDF_EVAL_*)
 EVAL_PRED_LIMIT, EVAL_GT_LIMIT, EVAL_BAD_OFFSETS, EVAL_BAD_KEEP = 1, 2, 4, 8
 
@@ -230,12 +242,15 @@ def lib():
     L.avdf_session_window_bytes.argtypes = [c_void_p, c_int32, c_int32]
     L.avdf_session_attach_windows.argtypes = [c_void_p, c_void_p, c_size_t, c_int32, c_int32]
     L.avdf_session_run_windows.argtypes = [c_void_p, POINTER(WindowRunArgs), c_void_p]
+    L.avdf_format_results_workspace_bytes.restype = c_size_t
+    L.avdf_format_results_workspace_bytes.argtypes = [c_int32]
+    L.avdf_format_results.argtypes = [POINTER(FormatArgs), c_void_p]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("avdf_last_error", "avdf_nms_workspace_bytes", "avdf_postprocess_workspace_bytes",
                         "avdf_conv_gemm_workspace_bytes", "avdf_eval_workspace_bytes", "avdf_eval_proposal_workspace_bytes",
                         "avdf_window_merge_workspace_bytes", "avdf_abi_version", "avdf_plan_close", "avdf_session_destroy",
-                        "avdf_session_window_bytes"):
+                        "avdf_session_window_bytes", "avdf_format_results_workspace_bytes"):
             fn.restype = c_int32
     if L.avdf_abi_version() != 3:
         raise AvdfError("libavdf_sm100.so ABI version mismatch")

@@ -597,3 +597,28 @@ def eval_proposal(prop_off, prop_seg, prop_score, keep, gt_off, gt_seg, threshol
                                   (nv.EVAL_BAD_KEEP, "keep is outside 0 .. proposals of its video")) if st & b]
             raise nv.AvdfError("avdf_eval_proposal: %s (status %d); no results were written" % ("; ".join(why), st))
     return matches, status
+
+
+# ---------------------------------------------------------------------------- result files (JSON text)
+def format_results(mode, records, K, order, ids, id_off, id_bytes_max, pos_begin, n_rows, out, out_bytes, *, min_score=0.2,
+                   workspace=None):
+    """JSON text of output positions [pos_begin, pos_begin + n_rows) into the uint8 buffer `out`, its byte count into
+    int64 out_bytes [1] (include/avdf.h avdf_format_results; -1 when a row was invalid). records fp32 [R, 3 + 3K],
+    order int32 [P], ids uint8 blob, id_off int64 [P + 1] (device); mode nv.FORMAT_RECORDS or nv.FORMAT_PREDICTIONS.
+    Returns the workspace used (pass it back to reuse it)."""
+    L = nv.lib()
+    _chk(records, torch.float32, "records"); _chk(order, torch.int32, "order"); _chk(ids, torch.uint8, "ids")
+    _chk(id_off, torch.int64, "id_off"); _chk(out, torch.uint8, "out"); _chk(out_bytes, torch.int64, "out_bytes")
+    assert records.dim() == 2 and records.shape[1] == 3 + 3 * K and id_off.numel() == order.numel() + 1
+    need = L.avdf_format_results_workspace_bytes(n_rows)
+    if workspace is None or workspace.numel() < need:
+        workspace = torch.empty(need, dtype=torch.uint8, device=records.device)
+    a = nv.FormatArgs()
+    a.mode, a.K, a.records, a.n_records = mode, K, records.data_ptr(), records.shape[0]
+    a.order, a.n_pos, a.ids, a.id_off, a.id_bytes_max = order.data_ptr(), order.numel(), ids.data_ptr(), id_off.data_ptr(), id_bytes_max
+    a.pos_begin, a.n_rows, a.min_score = pos_begin, n_rows, float(min_score)
+    a.out, a.out_capacity, a.out_bytes = out.data_ptr(), out.numel(), out_bytes.data_ptr()
+    a.workspace, a.workspace_bytes = workspace.data_ptr(), workspace.numel()
+    _call("avdf_format_results", L.avdf_format_results, (ctypes.byref(a), _stream(),), launches=3,
+          work={"bytes": n_rows * records.shape[1] * 4})
+    return workspace

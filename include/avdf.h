@@ -44,6 +44,8 @@
  *   avdf_eval_detection             libs/utils/metrics.py ANETdetection (AP and Recall@kx of one class), the evaluator
  *                                   valid_one_epoch calls (libs/utils/train_utils.py)
  *   avdf_eval_proposal              libs/utils/Evaluation/eval_proposal.py ANETproposal (ActivityNet AR vs. AN)
+ *   avdf_format_results             the json.dump of data_left.json (libs/utils/train_utils.py inference_one_epoch) and of
+ *                                   prediction.json (generate_results.ipynb cell 2)
  */
 #ifndef AVDF_H_
 #define AVDF_H_
@@ -444,6 +446,45 @@ typedef struct avdf_eval_proposal_args {
 } avdf_eval_proposal_args;        /* host struct */
 AVDF_API size_t avdf_eval_proposal_workspace_bytes(int32_t n_video);
 AVDF_API int avdf_eval_proposal(const avdf_eval_proposal_args* args, void* stream);
+
+/* ---- result files: the JSON text of result records (csrc/results.cu) ----
+ * records are the fixed-size rows of the inference path (libs/utils/sharding.py): fp32 [n_records, 3 + 3K],
+ * row = [index, n, video_cls, scores[K], segments[K, 2]], the first n scores / segments valid (0 <= n <= K, integral).
+ * Output position p shows row order[p] under the id text ids[id_off[p] .. id_off[p + 1]): that id already quoted and
+ * escaped by Python's json string encoder (ensure_ascii=False) and UTF-8 encoded; the kernel copies its bytes.
+ *   AVDF_FORMAT_RECORDS      one data_left.json item per position, exactly json.dump([{"video_id", "video_cls": [cls],
+ *                            "scores": [...], "segments": [[s, e], ...]}, ...], ensure_ascii=False, indent=4)
+ *   AVDF_FORMAT_PREDICTIONS  one prediction.json entry per position, `"id": [[score, start, end], ...]` keeping the
+ *                            segments with (double)score > min_score, `[[0, 0, 0]]` (ints) when none is kept, exactly
+ *                            json.dump(..., sort_keys=True, ensure_ascii=False, indent=4) when order lists the
+ *                            de-duplicated ids in sorted order
+ * Numbers are float.__repr__ of the fp32 values widened to float64 (NaN / Infinity / -Infinity as json writes them).
+ * A call formats positions [pos_begin, pos_begin + n_rows) into out and stores the byte count in *out_bytes. Every
+ * position's text is preceded by ",\n" except position 0's; the caller writes the opening "[\n" / "{\n" before position
+ * 0 and the closing "\n]" / "\n}" after the last one ("[]" / "{}" when there are no positions). out_capacity must hold
+ * n_rows times the longest text of a position, L(K, id_bytes_max) bytes (csrc/results.cu row_bytes_max, restated by
+ * libs/utils/result_writer.py). A row index outside the records, an invalid n or an id longer than id_bytes_max makes
+ * the call write nothing and store -1 in *out_bytes. No host synchronisation. */
+enum { AVDF_FORMAT_RECORDS = 0, AVDF_FORMAT_PREDICTIONS = 1 };
+typedef struct avdf_format_args {
+  int32_t mode;                  /* AVDF_FORMAT_RECORDS or AVDF_FORMAT_PREDICTIONS */
+  int32_t K;                     /* segments per record, >= 1 */
+  const float* records;          /* [n_records, 3 + 3K] */
+  int64_t n_records;
+  const int32_t* order;          /* [n_pos] row of each output position */
+  int64_t n_pos;
+  const uint8_t* ids;            /* id text blob */
+  const int64_t* id_off;         /* [n_pos + 1] */
+  int32_t id_bytes_max;          /* longest id text in bytes (host value) */
+  int64_t pos_begin;             /* first position of this call */
+  int32_t n_rows;                /* positions of this call, >= 1 */
+  double min_score;              /* AVDF_FORMAT_PREDICTIONS: keep scores above it */
+  uint8_t* out; size_t out_capacity;
+  int64_t* out_bytes;            /* [1] */
+  void* workspace; size_t workspace_bytes;   /* 256-byte aligned, avdf_format_results_workspace_bytes(n_rows) */
+} avdf_format_args;               /* host struct */
+AVDF_API size_t avdf_format_results_workspace_bytes(int32_t n_rows);
+AVDF_API int avdf_format_results(const avdf_format_args* args, void* stream);
 
 /* ---- HOST: gather n byte spans (src[i] -> dst[i], nbytes[i] bytes; all HOST pointers, any alignment; dst is normally
  * a slice of a pinned staging buffer) with up to n_threads threads of a pool that lives inside the library

@@ -7,7 +7,8 @@ loads the yaml with the reference's DEFAULTS merge, builds the inference dataset
 `deepfake_test_sub{sub_index}.txt` list), the meta-arch by name, loads `checkpoint['state_dict_ema']` (DataParallel
 `module.` keys accepted) and writes `<ckpt dir>/<sub_index>/data_left*.json` exactly like inference_one_epoch does.
 New: `-b` videos per model call (default 32; the reference is fixed to 1) and `--merge` to also write the challenge's
-prediction.txt / prediction.json (generate_results.ipynb) for this shard.
+prediction.txt / prediction.json (generate_results.ipynb) for this shard. Every result file is formatted on the GPU from
+the device records (libs/utils/result_writer.py), byte for byte what json.dump writes.
 `--window SEC [--hop SEC]` (hop defaults to window / 2): recordings longer than SEC seconds run as overlapping windows at
 the model's trained time scale, merged into one result per recording on the GPU (libs/modeling/windows.py); such runs
 always go through inference_sharded, single-process and torchrun alike. The window is a user choice: no setting of it
@@ -22,6 +23,7 @@ files for 7 separate processes, inference.py:116-124), streams it through the mo
 result records are all-gathered once over NCCL; rank 0 writes the same data_left.json a single process writes.
 """
 import argparse
+import glob
 import os
 import time
 
@@ -30,7 +32,9 @@ import torch
 from audio_visual_deepfake_detection_b200.libs.core import load_config
 from audio_visual_deepfake_detection_b200.libs.datasets import make_data_loader, make_inference_dataset
 from audio_visual_deepfake_detection_b200.libs.modeling import make_meta_arch
-from audio_visual_deepfake_detection_b200.libs.utils import fix_random_seed, inference_one_epoch, inference_sharded, merge_results
+from audio_visual_deepfake_detection_b200.libs.utils import fix_random_seed, merge_results
+from audio_visual_deepfake_detection_b200.libs.utils.infer_utils import one_epoch_records, sharded_records
+from audio_visual_deepfake_detection_b200.libs.utils.result_writer import write_predictions
 
 
 def main(args):
@@ -62,17 +66,44 @@ def main(args):
     out_dir = os.path.join(os.path.dirname(args.ckpt), str(args.sub_index))
     start = time.time()
     if world > 1 or args.window is not None:
-        inference_sharded(dataset, model, out_dir, batch_size=args.batch, rank=rank, world=world, print_freq=args.print_freq,
-                          window=args.window, hop=args.hop)
+        res = sharded_records(dataset, model, out_dir, batch_size=args.batch, rank=rank, world=world, print_freq=args.print_freq,
+                              window=args.window, hop=args.hop)
+        files = [] if res is None else [("data_left.json",) + res]
     else:
-        inference_one_epoch(loader, model, -1, output_folder=out_dir, print_freq=args.print_freq, dataset_name=cfg["dataset_name"])
+        written, _ = one_epoch_records(loader, model, out_dir)
+        files = [(name, ids, rec, None, K) for name, ids, rec, K in written]
     if rank == 0:
         print("All done! Total time: {:0.2f} sec".format(time.time() - start))
         if args.merge:
-            merge_results([out_dir], out_dir)
+            write_merged(out_dir, files)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def write_merged(out_dir, files):
+    """prediction.txt / prediction.json of this shard. When the folder's result files (those merge_results reads) are
+    exactly the files this run wrote, they are written on the GPU from the records in hand, in merge_results' file order;
+    otherwise (files of an earlier run in the folder) merge_results reads the folder as before."""
+    names = sorted(os.path.basename(p) for p in glob.glob(os.path.join(out_dir, "*.json"))
+                   if not os.path.basename(p).startswith("prediction"))
+    if not files or names != sorted(f[0] for f in files):
+        merge_results([out_dir], out_dir)
+        return
+    files = sorted(files, key=lambda f: f[0])
+    K = max(f[4] for f in files)
+    ids, recs, orders, base = [], [], [], 0
+    for name, f_ids, rec, order, k in files:
+        if k != K:                       # widen to the common K: segments move to their K-strided place
+            wide = torch.zeros((rec.shape[0], 3 + 3 * K), dtype=rec.dtype, device=rec.device)
+            wide[:, :3 + k] = rec[:, :3 + k]
+            wide[:, 3 + K:3 + K + 2 * k] = rec[:, 3 + k:]
+            rec = wide
+        ids += f_ids
+        orders.append((torch.arange(len(f_ids), device=rec.device, dtype=torch.int32) if order is None else order) + base)
+        recs.append(rec)
+        base += rec.shape[0]
+    write_predictions(out_dir, ids, torch.cat(recs), K, order=torch.cat(orders))
 
 
 if __name__ == "__main__":
