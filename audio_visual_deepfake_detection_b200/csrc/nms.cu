@@ -218,14 +218,17 @@ __device__ int soft_nms_block(const Cand& c, int n, float thr, float sigma, floa
     int wbase = 0;
     for (int q = 0; q < w; ++q) wbase += sh.scan[q];
     int run = wbase + inc - cnt;                     // failures strictly before this chunk
+    int run_hi = run;                                // ... and strictly before max(cb, new_n)
     for (int p = cb; p < ce; ++p) {
       bool fail = c.sc[p] < min_score;
       if (fail && p < new_n) c.hole[run] = p;        // ascending rank among failures == rank among holes
       run += fail ? 1 : 0;
+      if (p < new_n) run_hi = run;
     }
     __syncthreads();
-    run = wbase + inc - cnt;
-    for (int p = cb; p < ce; ++p) {
+    // the moves below fill holes (< new_n) while other threads still scan their chunks: read positions >= new_n only
+    run = run_hi;
+    for (int p = max(cb, new_n); p < ce; ++p) {
       bool fail = c.sc[p] < min_score;
       run += fail ? 1 : 0;                           // inclusive failure count through p
       if (!fail && p >= new_n) {
@@ -462,14 +465,17 @@ nms_cluster_kernel(const float* __restrict__ segs, const float* __restrict__ sco
       int wbase = before;
       for (int q = 0; q < w; ++q) wbase += sh.scan[q];
       int run = wbase + inc - cnt;                     // failures strictly before this chunk, over the whole list
+      int run_hi = run;                                // ... and strictly before max(cb, new_n)
       for (int p = cb; p < ce; ++p) {
         const bool fail = sc[p - base] < min_score;
         if (fail && p < new_n) hole[run] = p;
         run += fail ? 1 : 0;
+        if (p < new_n) run_hi = run;
       }
       cl_sync();                                       // the hole list (global memory) is complete
-      run = wbase + inc - cnt;
-      for (int p = cb; p < ce; ++p) {
+      // remote stores fill holes (< new_n) while other threads still scan: read positions >= new_n only
+      run = run_hi;
+      for (int p = max(cb, new_n); p < ce; ++p) {
         const int o = p - base;
         const bool fail = sc[o] < min_score;
         run += fail ? 1 : 0;                           // inclusive failure count through p

@@ -1,5 +1,6 @@
 """float64 references of the `ops` entry points the localization forward pass and the BYOL-A extractor launch, one per
-entry point, with the entry point's own keyword arguments.
+entry point, with the entry point's own keyword arguments (postprocess also reads the candidates its launch decoded:
+READS_OUTPUTS).
 
 TEST INFRASTRUCTURE (see oracle/model_ref.py's header).
 
@@ -14,6 +15,7 @@ device of its operands) and returns a dict {output path: Out}. The path names th
            their value can cancel to far below the size of the fp32 rounding of its terms.
   tol      float64 per-element absolute error bound, or None (the row-wise bar). The log-mel spectrogram has one: its
            smallest mel bins sit ~1e-6 below the row's largest, where the fp32 FFT's rounding is all the value holds.
+           postprocess has one per output: 0 (exact) for its NMS results, a derived bound for its sigmoid and voting.
 Operands are what the kernel saw: 16-bit tensors convert exactly to float64. Intermediate roundings are modelled only
 where the code documents them: the 16-bit hidden activations of mlp_fused (csrc/mlp_fused.cu: "-> 16-bit -> shared
 memory") and the 16-bit LN2 operand of the block tail (mlp_fused proj=: "writes the 16-bit x tile").
@@ -529,12 +531,271 @@ def byola_pool(x, clip_step_in, clip_of_step, t_of_step, out, *, mel_in, pad_out
     return outs
 
 
+# --------------------------------------------------------------------------------------------------- postprocess
+F32 = np.float32
+# the sigmoid of decode: the device expf is within 2 ulp (4u relative), then 1 + e and 1 / (.) round once each
+SIGMOID_REL = 6 * FP32_U
+# counters of the decode membership check and the voting bound, summed over postprocess calls until reset
+POSTPROCESS_STATS = {"videos": 0, "near_cut": 0, "near_cut_moved": 0}
+
+
+def reset_postprocess_stats():
+    POSTPROCESS_STATS.update(videos=0, near_cut=0, near_cut_moved=0)
+
+
+def voting_ref(picks, all_segs, all_scores, thr):
+    """seg_voting (nms.py:67-101) of `picks` [k, 2] against every candidate, as float64 values with a per-element error
+    bound for the kernel's float32 evaluation (csrc/nms.cu postprocess_kernel). Returns (value [k, 2], bound [k, 2]).
+
+    The weights w_j = fl(fl([iou_j >= thr] * s_j) * iou_j), with iou_j, inter and the lengths computed in float32 by
+    the kernel's own elementwise IEEE operations, are reproduced exactly (numpy float32; fmax / fmin like fmaxf /
+    fminf), so every `iou >= thr` decision matches. What remains is the order of the sums. Per pick, the kernel
+        S~ = sum_j w_j                 lane-strided fp32 sums (ceil(n / 32) terms) + a 5-level warp tree
+        q_j = fl(w_j / S~)             one rounding
+        V~ = sum_j fma(q_j, b_j, .)    the same reduction, one rounding per fma and per tree add
+    With m = ceil(n / 32) + 5 roundings on any path, g = m u / (1 - m u), u = 2^-24, W = sum |w_j|, A = sum |w_j b_j|:
+        S~ = S + e,  |e| <= g W                                 (standard summation bound)
+        V~ = sum_j (w_j b_j / S~)(1 + d_j)(1 + t_j),  |d_j| <= u, |t_j| <= g
+        V~ - V = sum_j w_j b_j ((1 + d_j)(1 + t_j) - 1) / S~  +  sum_j w_j b_j (1 / S~ - 1 / S)
+        |V~ - V| <= A (u + g + u g) / |S~|  +  A g W / (|S~| |S|)     with |S~| >= |S| - g W
+    so bound = A (u + g + u g + g W / |S|) / (|S| - g W), plus 2^-126 for underflow. V = sum w_j b_j / sum w_j in
+    float64 (its own error, ~n 2^-53 relative, is far below the bound). A NaN weight (a zero-length pick against a
+    zero-length candidate at the same place: 0 / 0) makes the value NaN, and the kernel's must be NaN too."""
+    picks = np.asarray(picks, F32).reshape(-1, 2)
+    segs = np.asarray(all_segs, F32).reshape(-1, 2)
+    sc = np.asarray(all_scores, F32)
+    n = len(sc)
+    val = np.zeros((len(picks), 2))
+    bound = np.zeros((len(picks), 2))
+    if len(picks) == 0:
+        return val, bound
+    m = -(-n // 32) + 5
+    g = m * FP32_U / (1 - m * FP32_U)
+    b0, b1 = segs[:, 0], segs[:, 1]
+    lb = b1 - b0
+    thr32 = F32(thr)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        for q, (a0, a1) in enumerate(picks):
+            la = a1 - a0
+            inter = np.fmax(np.fmin(a1, b1) - np.fmax(a0, b0), F32(0))
+            iou = inter / ((la + lb) - inter)
+            w = ((iou >= thr32).astype(F32) * sc) * iou
+            w64 = w.astype(np.float64)
+            S, W = w64.sum(), np.abs(w64).sum()
+            for c, b in enumerate((b0, b1)):
+                val[q, c] = (w64 * b).sum() / S
+                A = np.abs(w64 * b).sum()
+                den = abs(S) - g * W
+                bound[q, c] = (A * (FP32_U + g + FP32_U * g + g * W / abs(S)) / den if den > 0 else np.inf) + 2.0 ** -126
+    return val, bound
+
+
+def nms_picks(segs, scores, iou_threshold, min_score, sigma, max_num, soft, method):
+    """The picks of one video's batched_nms (class-agnostic, nms.py:159-180) on float32 candidates, by the C oracle:
+    (candidate index [k], score [k] f32, segment [k, 2] f32) in pick order, at most max_num."""
+    import nms_ref
+    segs = np.asarray(segs, F32).reshape(-1, 2)
+    scores = np.asarray(scores, F32)
+    if len(scores) == 0:
+        return np.zeros(0, np.int64), np.zeros(0, F32), np.zeros((0, 2), F32)
+    if soft:
+        idx, dets = nms_ref.softnms(segs, scores, iou_threshold, sigma, min_score, method, max_num=max_num)
+        return idx, dets[:, 2].copy(), dets[:, :2].copy()
+    keep = np.nonzero(scores > F32(min_score))[0] if min_score > 0 else np.arange(len(scores))
+    idx = keep[nms_ref.nms(segs[keep], scores[keep], iou_threshold)][:max_num]
+    return idx, scores[idx], segs[idx]
+
+
+def to_seconds(v, stride, half_nframes, fps, duration):
+    """av_fd_no_recon.py:860-865 in the kernel's float32 operations: (v * stride + half_nframes) / fps, <= 0 -> v * 0,
+    >= duration -> v * 0 + duration."""
+    st, hn, fp, du = F32(stride), F32(half_nframes), F32(fps), F32(duration)
+    with np.errstate(invalid="ignore", over="ignore"):
+        o = ((np.asarray(v, F32) * st) + hn) / fp
+        o = np.where(o <= 0, o * F32(0), o)
+        return np.where(o >= du, o * F32(0) + du, o).astype(F32)
+
+
+def seconds_bound(val, bound, stride, half_nframes, fps):
+    """A float64 value known within `bound`, taken to seconds by the three float32 roundings of to_seconds: the bound
+    of the result (the clamps are 1-Lipschitz, so they add nothing)."""
+    st, hn, fp = float(F32(stride)), float(F32(half_nframes)), float(F32(fps))
+    return (bound * st + 4 * FP32_U * ((np.abs(val) + bound) * st + abs(hn))) / fp
+
+
+def _sec64(v, stride, half_nframes, fps, duration):
+    st, hn, fp, du = (float(F32(x)) for x in (stride, half_nframes, fps, duration))
+    o = (v * st + hn) / fp
+    return np.where(o >= du, du, np.where(o <= 0, 0.0, o))
+
+
+def decode_check(logits, offsets, mask, level_len, level_stride, pre_nms_thresh, pre_nms_topk, duration_thresh,
+                 segs, scores, count):
+    """Checks one video's decoded candidates (the kernel's segs [n, 2], scores [n], in its order) against a float64
+    decode of logits [P] / offsets [P, 2] / mask [P] (av_fd_no_recon.py:775-823) and returns, per candidate, its point
+    (level-major index), the float64 probability and the float32 segment:
+      * every candidate is a point of the current or a later level with the same float32 segment (tt = t * s,
+        left = tt - o0 * s, right = tt + o1 * s: bit-exact) whose probability is within SIGMOID_REL of the float64
+        sigmoid; levels appear in order, scores do not increase within a level, and equal scores come in ascending
+        point order (the kernel's tie rule);
+      * per level the candidate set equals the float64 one - probability > pre_nms_thresh, the pre_nms_topk highest,
+        right - left > duration_thresh - except for points within the sigmoid's error of pre_nms_thresh, or within
+        twice that of the cut score (two such points may swap across the cut). Those are counted in
+        POSTPROCESS_STATS['near_cut'], and the ones whose membership differs in 'near_cut_moved'."""
+    lg = np.asarray(logits, np.float64)
+    of = np.asarray(offsets, F32).reshape(-1, 2)
+    mk = np.asarray(mask).astype(bool)
+    thr = float(F32(pre_nms_thresh))
+    dthr = F32(duration_thresh)
+    with np.errstate(over="ignore"):
+        p64 = np.where(mk, 1.0 / (1.0 + np.exp(-lg)), 0.0)
+    tol = SIGMOID_REL * p64
+    offs = np.cumsum([0] + [int(v) for v in level_len])
+    left = np.zeros(len(lg), F32)
+    right = np.zeros(len(lg), F32)
+    certain, possible, member64, exempt = [], [], [], []
+    level_of = np.zeros(len(lg), np.int64)
+    for l, n in enumerate(level_len):
+        s = F32(level_stride[l])
+        pts = np.arange(int(n))
+        tt = pts.astype(F32) * s
+        sl = slice(offs[l], offs[l + 1])
+        left[sl] = tt - of[sl, 0] * s
+        right[sl] = tt + of[sl, 1] * s
+        level_of[sl] = l
+        p = p64[sl]
+        valid = np.nonzero(p > thr)[0]
+        order = valid[np.argsort(-p[valid], kind="stable")]
+        k = min(int(pre_nms_topk), len(order))
+        member = np.zeros(int(n), bool)
+        member[order[:k]] = True
+        near = np.abs(p - thr) <= tol[sl]
+        if len(order) > k:
+            cut = p[order[k - 1]] if k > 0 else p[order[0]]
+            near |= np.abs(p - cut) <= 2 * SIGMOID_REL * cut
+        dur = (right[sl] - left[sl]) > dthr
+        certain.append(set((offs[l] + np.nonzero(member & ~near & dur)[0]).tolist()))
+        possible.append(set((offs[l] + np.nonzero((member | near) & dur)[0]).tolist()))
+        member64.append(set((offs[l] + np.nonzero(member & near & dur)[0]).tolist()))
+        exempt.append(set((offs[l] + np.nonzero(near & dur)[0]).tolist()))
+    segs = np.asarray(segs, F32).reshape(-1, 2)[:count]
+    scores = np.asarray(scores)[:count].astype(np.float64)
+    by_seg = {}
+    for l in range(len(level_len)):
+        for pt in sorted(possible[l]):
+            by_seg.setdefault((l, left[pt].tobytes(), right[pt].tobytes()), []).append(pt)
+    point = np.zeros(count, np.int64)
+    used = set()
+    lvl = 0
+    for c in range(count):
+        key = segs[c, 0].tobytes(), segs[c, 1].tobytes()
+        hit = None
+        for l in range(lvl, len(level_len)):
+            for pt in by_seg.get((l,) + key, ()):
+                if pt not in used and abs(scores[c] - p64[pt]) <= tol[pt]:
+                    hit = pt
+                    break
+            if hit is not None:
+                break
+        assert hit is not None, ("decoded candidate %d (%r, %r, score %r) is no point of level >= %d with that float32 "
+                                 "segment and a probability within the sigmoid's error" % (c, segs[c, 0], segs[c, 1], scores[c], lvl))
+        if level_of[hit] == lvl and c > 0 and level_of[point[c - 1]] == lvl:
+            assert scores[c] < scores[c - 1] or (scores[c] == scores[c - 1] and hit > point[c - 1]), \
+                "decoded candidates %d, %d of level %d are out of order (score, then point index)" % (c - 1, c, lvl)
+        lvl = int(level_of[hit])
+        used.add(hit)
+        point[c] = hit
+    for l in range(len(level_len)):
+        got = {pt for pt in used if level_of[pt] == l}
+        missing, extra = certain[l] - got, got - possible[l]
+        assert not missing and not extra, "level %d: decode membership differs from float64 away from the cut: missing " \
+                                          "points %s, extra %s" % (l, sorted(missing)[:8], sorted(extra)[:8])
+        POSTPROCESS_STATS["near_cut"] += len(exempt[l])
+        POSTPROCESS_STATS["near_cut_moved"] += len((got & exempt[l]) ^ member64[l])
+    return point, p64[point], np.stack([left[point], right[point]], 1)
+
+
+def postprocess(batch, *, logits=None, offsets=None, mask=None, level_len=(), level_stride=(), pre_nms_thresh=0.001,
+                pre_nms_topk=2000, duration_thresh=0.001, cand_segs, cand_scores, cand_count, iou_threshold, min_score,
+                sigma, voting_thresh, max_seg_num, use_soft_nms, soft_method=2, vid_meta=None, out_segs, out_scores,
+                out_count, workspace=None, records=None, out_index=None):
+    """Fused decode + batched_nms + seconds conversion. With logits, cand_segs / cand_scores / cand_count are what the
+    kernel decoded (outputs of the launch, passed in by the checker): decode_check validates them against a float64
+    decode; then NMS, the final stable sort by score and the cap are the C oracle on those same candidates, bit-exact;
+    voting is voting_ref's float64 value and bound; the seconds conversion is exact float32 on exact values and
+    seconds_bound on voted ones. nms 'none' (use_soft_nms None): every candidate, in order, to seconds."""
+    if records is not None:
+        raise NotImplementedError("the postprocess reference does not model the result-record ring")
+    B, K = int(batch), int(max_seg_num)
+    n_all = np.asarray(cand_count.cpu()).astype(np.int64)
+    cs = cand_segs.detach().cpu().numpy().astype(F32).reshape(B, -1, 2)
+    cc = cand_scores.detach().cpu().numpy().astype(F32).reshape(B, -1)
+    meta = None if vid_meta is None else [t.detach().cpu().numpy().astype(F32) for t in vid_meta]
+    dev = out_segs.device
+    outs = {}
+    if logits is not None:
+        lg = logits.detach().cpu().numpy()
+        of = offsets.detach().cpu().numpy().reshape(B, -1, 2)
+        mk = mask.detach().cpu().numpy()
+        c_ref, c_tol = np.zeros(cc.shape), np.zeros(cc.shape)
+        c_wr = np.zeros(cc.shape, bool)
+        for b in range(B):
+            n = int(n_all[b])
+            _, p, _ = decode_check(lg[b], of[b], mk[b], level_len, level_stride, pre_nms_thresh, pre_nms_topk,
+                                   duration_thresh, cs[b], cc[b], n)
+            c_ref[b, :n], c_tol[b, :n], c_wr[b, :n] = p, SIGMOID_REL * p, True
+            POSTPROCESS_STATS["videos"] += 1
+        t = lambda a, like: torch.from_numpy(np.ascontiguousarray(a)).to(like.device).reshape(like.shape)
+        s_wr = np.repeat(c_wr[..., None], 2, -1)
+        outs["cand_scores"] = Out(t(c_ref, cand_scores), t(c_wr, cand_scores), _false(cand_scores), None, t(c_tol, cand_scores))
+        outs["cand_segs"] = Out(t(cs.astype(np.float64), cand_segs), t(s_wr, cand_segs), _false(cand_segs), None,
+                                t(np.zeros(s_wr.shape), cand_segs))
+        outs["cand_count"] = Out(t(n_all.astype(np.float64), cand_count), ~_false(cand_count), _false(cand_count), None)
+    width = out_scores.shape[1]
+    o_ref = np.zeros((B, width, 2))
+    o_tol = np.zeros((B, width, 2))
+    s_ref = np.zeros((B, width))
+    wr = np.zeros((B, width), bool)
+    i_ref = np.zeros((B, width))
+    cnt = np.zeros(B)
+    for b in range(B):
+        n = int(n_all[b])
+        segs, sc = cs[b, :n], cc[b, :n]
+        st = (1.0, 0.0, 1.0, 0.0) if meta is None else tuple(float(meta[i][b]) for i in range(4))
+        if use_soft_nms is None:
+            v = segs if meta is None else to_seconds(segs, *st)
+            o_ref[b, :n], s_ref[b, :n], wr[b, :n], cnt[b] = v, sc, True, n
+            continue
+        idx, ps, pseg = nms_picks(segs, sc, iou_threshold, min_score, sigma, K, bool(use_soft_nms), soft_method)
+        order = np.argsort(-ps, kind="stable")
+        idx, ps, pseg = idx[order], ps[order], pseg[order]
+        k = len(idx)
+        if voting_thresh > 0 and k:
+            val, bnd = voting_ref(pseg, segs, sc, voting_thresh)
+            if meta is not None:
+                bnd = seconds_bound(val, bnd, *st[:3])
+                val = _sec64(val, *st)
+            o_ref[b, :k], o_tol[b, :k] = val, bnd
+        else:
+            o_ref[b, :k] = pseg if meta is None else to_seconds(pseg, *st)
+        s_ref[b, :k], i_ref[b, :k], wr[b, :k], cnt[b] = ps, idx, True, k
+    t = lambda a, like: torch.from_numpy(np.ascontiguousarray(a)).to(dev).reshape(like.shape)
+    outs["out_segs"] = Out(t(o_ref, out_segs), t(np.repeat(wr[..., None], 2, -1), out_segs), _false(out_segs), None,
+                           t(o_tol, out_segs))
+    outs["out_scores"] = Out(t(s_ref, out_scores), t(wr, out_scores), _false(out_scores), None, t(np.zeros(wr.shape), out_scores))
+    outs["out_count"] = Out(t(cnt, out_count), ~_false(out_count), _false(out_count), None)
+    if out_index is not None and use_soft_nms is not None:
+        outs["out_index"] = Out(t(i_ref, out_index), t(wr, out_index), _false(out_index), None)
+    return outs
+
+
 REFERENCES = {f.__name__: f for f in (interp_concat, interp_concat_ranges, pack_feats, conv_gemm, mlp_fused, ln_dwconv_ln,
                                       attention, ln_rows, instnorm_lrelu, fpn_fuse, head_final, head_combine, vcls_exp12,
-                                      vcls_exp13, logmel, byola_conv1_pool, byola_pool)}
+                                      vcls_exp13, logmel, byola_conv1_pool, byola_pool, postprocess)}
 # entry points the forward pass launches that have no reference here, and why
-EXCLUDED = {"postprocess": "decode + NMS + seconds conversion: compared bit for bit with the C oracle (oracle/nms_ref.c) "
-                           "in tests/test_gpu_kernels.py and tests/test_gpu_model.py"}
+EXCLUDED = {}
+# outputs of a launch its reference reads: postprocess checks the candidates the kernel decoded, then runs NMS on them
+READS_OUTPUTS = {"postprocess": ("cand_segs", "cand_scores", "cand_count")}
 
 
 def ulp(x, dtype):
@@ -546,7 +807,8 @@ def ulp(x, dtype):
 
 def check(got, o, width, bar, what=""):
     """Asserts a kernel output against its reference Out: integer outputs equal; structural zeros exactly 0; with a
-    per-element bound o.tol, |got - ref| <= bar * tol everywhere; otherwise the row-wise error max|got - ref| /
+    per-element bound o.tol, |got - ref| <= bar * tol everywhere (a bound of 0 asks for the exact value, a NaN
+    reference for a NaN); otherwise the row-wise error max|got - ref| /
     max(|ref|, mag) over rows of `width` values within `bar` (16-bit outputs: beyond one ulp of their type at |ref|;
     bar 0 asks for exact values, without that ulp). Returns the worst row-wise error (err / tol with a bound)."""
     ref, written = o.ref.to(got.device), o.written.to(got.device)
@@ -562,7 +824,9 @@ def check(got, o, width, bar, what=""):
         raise AssertionError("%s: element %s must be exactly 0, got %r" % (what, i, float(got[i])))
     err = (got.to(F64) - ref).abs()
     if o.tol is not None:
-        rel = torch.where(written, torch.nan_to_num(err / o.tol.to(got.device), nan=float("inf")), torch.zeros_like(err))
+        err = torch.where(torch.isnan(got) & torch.isnan(ref), torch.zeros_like(err), err)       # NaN where NaN is due
+        rel = torch.where(err == 0, torch.zeros_like(err), err / o.tol.to(got.device))          # bound 0: exact
+        rel = torch.where(written, torch.nan_to_num(rel, nan=float("inf")), torch.zeros_like(err))
         kind = "error / bound"
     else:
         if got.dtype in (torch.float16, torch.bfloat16) and bar > 0:

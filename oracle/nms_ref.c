@@ -69,10 +69,14 @@ int64_t ref_nms_1d(const float *segs, const float *scores, int64_t n,
 }
 
 /* nms_cpu.cpp:67-160. dets [n,3] is written in place (x1, x2, score per
- * pick); out_inds gets the original indices in pick order; returns count. */
-int64_t ref_softnms_1d(const float *segs, const float *scores, float *dets,
-                       int64_t n, float iou_threshold, float sigma,
-                       float min_score, int method, int64_t *out_inds) {
+ * pick); out_inds gets the original indices in pick order; returns count.
+ * max_num > 0 stops after that many picks: pick i depends on picks 0..i-1
+ * only, so the result is the prefix of the full run (what the kernels'
+ * max_num returns), at a fraction of the O(n * picks) cost. */
+int64_t ref_softnms_1d_capped(const float *segs, const float *scores, float *dets,
+                              int64_t n, float iou_threshold, float sigma,
+                              float min_score, int method, int64_t max_num,
+                              int64_t *out_inds) {
   if (n == 0) return 0;
   float *x1 = (float *)malloc(sizeof(float) * n), *x2 = (float *)malloc(sizeof(float) * n);
   float *sc = (float *)malloc(sizeof(float) * n), *ar = (float *)malloc(sizeof(float) * n);
@@ -83,6 +87,7 @@ int64_t ref_softnms_1d(const float *segs, const float *scores, float *dets,
   }
   int64_t nsegs = n;
   for (int64_t i = 0; i < nsegs; i++) {
+    if (max_num > 0 && i >= max_num) { nsegs = i; break; }
     float max_score = sc[i];
     int64_t max_pos = i;
     for (int64_t pos = i + 1; pos < nsegs; pos++)
@@ -117,6 +122,13 @@ int64_t ref_softnms_1d(const float *segs, const float *scores, float *dets,
   memcpy(out_inds, inds, sizeof(int64_t) * nsegs);
   free(x1); free(x2); free(sc); free(ar); free(inds);
   return nsegs;
+}
+
+int64_t ref_softnms_1d(const float *segs, const float *scores, float *dets,
+                       int64_t n, float iou_threshold, float sigma,
+                       float min_score, int method, int64_t *out_inds) {
+  return ref_softnms_1d_capped(segs, scores, dets, n, iou_threshold, sigma,
+                               min_score, method, 0, out_inds);
 }
 
 /* nms.py:67-101 (score_offset is computed but unused there). nms_segs [k,2]

@@ -33,6 +33,9 @@ def lib():
         L.ref_softnms_1d.restype = ctypes.c_int64
         L.ref_softnms_1d.argtypes = [f32p, f32p, f32p, ctypes.c_int64, ctypes.c_float, ctypes.c_float,
                                      ctypes.c_float, ctypes.c_int, i64p]
+        L.ref_softnms_1d_capped.restype = ctypes.c_int64
+        L.ref_softnms_1d_capped.argtypes = [f32p, f32p, f32p, ctypes.c_int64, ctypes.c_float, ctypes.c_float,
+                                            ctypes.c_float, ctypes.c_int, ctypes.c_int64, i64p]
         L.ref_seg_voting.restype = None
         L.ref_seg_voting.argtypes = [f32p, ctypes.c_int64, f32p, f32p, ctypes.c_int64, ctypes.c_float, f32p]
         _lib = L
@@ -56,15 +59,16 @@ def nms(segs, scores, iou_threshold):
     return out[:k].copy()
 
 
-def softnms(segs, scores, iou_threshold, sigma, min_score, method):
-    """nms_1d_cpu.softnms equivalent; returns (inds, dets[:K])."""
+def softnms(segs, scores, iou_threshold, sigma, min_score, method, max_num=0):
+    """nms_1d_cpu.softnms equivalent; returns (inds, dets[:K]). max_num > 0: the first max_num picks only (the prefix
+    of the full result)."""
     segs = np.ascontiguousarray(segs, np.float32).reshape(-1, 2)
     scores = np.ascontiguousarray(scores, np.float32)
     n = len(scores)
     dets = np.zeros((max(n, 1), 3), np.float32)
     out = np.empty(max(n, 1), np.int64)
-    k = lib().ref_softnms_1d(_f(segs), _f(scores), _f(dets), n, float(iou_threshold), float(sigma),
-                             float(min_score), int(method), _i(out))
+    k = lib().ref_softnms_1d_capped(_f(segs), _f(scores), _f(dets), n, float(iou_threshold), float(sigma),
+                                    float(min_score), int(method), int(max_num), _i(out))
     return out[:k].copy(), dets[:k].copy()
 
 

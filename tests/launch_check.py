@@ -9,6 +9,7 @@ cloned before it runs and its outputs right after; then
               position's channels; 16-bit outputs may in addition differ by one ulp of their type at |ref|), or
               |got - ref| <= bar * tol element-wise where the reference gives a bound; uint8 outputs equal
   (c) zeros   every element the reference defines as zero (masked / padding rows, ReLU-clamped values) is exactly 0.0
+A reference listed in launch_ref.READS_OUTPUTS (postprocess) is given the launch's own values of those outputs.
 A failure names the op, the product call site, the shapes / dtypes and the worst element with both values."""
 import collections
 import inspect
@@ -30,8 +31,9 @@ BAR = 5e-5                 # results accumulated in fp32
 # hidden activations (and the tail's 16-bit LN2 operand) round at ties the kernel's fp32 and the reference's fp64 values
 # fall on different sides of
 BAR_MLP, BAR_TAIL = 2e-4, 2e-3
-# logmel: the reference's per-element bound is the whole allowance; byola_pool: a max of stored values, exact
-BAR_LOGMEL, BAR_POOL = 1.0, 0.0
+# logmel: the reference's per-element bound is the whole allowance; byola_pool: a max of stored values, exact;
+# postprocess: per-element bounds too (0 for its NMS results, which must be bit-exact)
+BAR_LOGMEL, BAR_POOL, BAR_POST = 1.0, 0.0, 1.0
 
 
 def _tensors(v):
@@ -78,6 +80,8 @@ def _bar(name, kw):
         return BAR_LOGMEL
     if name == "byola_pool":
         return BAR_POOL
+    if name == "postprocess":
+        return BAR_POST
     return BAR
 
 
@@ -123,6 +127,9 @@ def _output_paths(name, kw):
         return ["lms"]
     if name in ("byola_conv1_pool", "byola_pool"):
         return ["out"] + (["mask_out"] if kw["mask_out"] is not None else [])
+    if name == "postprocess":
+        return (["cand_segs", "cand_scores", "cand_count"] if kw["logits"] is not None else []) + \
+               ["out_segs", "out_scores", "out_count"] + (["out_index"] if kw["out_index"] is not None else [])
     return ["out"]
 
 
@@ -130,10 +137,16 @@ class LaunchChecker:
     def __init__(self):
         self.count = collections.Counter()
         self.worst = {}
+        self.worst_path = {}              # (op, output path) -> worst error / bar
         self.launches = []                # (op, its scalar arguments) per checked launch, in call order
 
     def check(self, name, site, orig, kw_in, recorded):
-        refs = launch_ref.REFERENCES[name](**kw_in)
+        # a reference that reads some of the launch's outputs (launch_ref.READS_OUTPUTS) gets what the launch wrote
+        kw_ref = dict(kw_in)
+        for k in launch_ref.READS_OUTPUTS.get(name, ()):
+            if kw_in[k] is not None and id(kw_in[k]) in recorded:
+                kw_ref[k] = recorded[id(kw_in[k])]
+        refs = launch_ref.REFERENCES[name](**kw_ref)
         groups = {}                       # one entry per distinct output tensor: (tensor, [Out ...])
         for path, o in refs.items():
             t = launch_ref.get_path(kw_in, path)
@@ -173,6 +186,7 @@ class LaunchChecker:
             worst = launch_ref.check(got, launch_ref.Out(ref, written, zero, mag, tol), _row_width(name, path, kw_in, ref), bar,
                                      "%s: %s" % (ctx, path))
             self.worst[name] = max(self.worst.get(name, 0.0), worst / bar if bar > 0 else worst)
+            self.worst_path[(name, path)] = max(self.worst_path.get((name, path), 0.0), worst / bar if bar > 0 else worst)
         self.count[name] += 1
         self.launches.append((name, {k: v for k, v in kw_in.items() if isinstance(v, (int, float))}))
 

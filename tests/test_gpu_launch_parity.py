@@ -4,7 +4,8 @@ the overlap, replay, error and zeros checks at once). A failure names the op, th
 dtypes and the worst element with both values.
 Passes: every MODEL_CASES entry in fp32 and mixed at batch 3 and in mixed at batch 32 (the benchmark's batch: the only
 passes that take the launch configurations that depend on the SM count), and exp12 mixed at batch 32 with each of the
-engine's A/B switches AVDF_FUSE_TAIL, AVDF_FUSE_LN2, AVDF_FUSED_MLP turned off."""
+engine's A/B switches AVDF_FUSE_TAIL, AVDF_FUSE_LN2, AVDF_FUSED_MLP turned off. Each pass ends in the fused postprocess
+(decode, NMS - soft in the mixed batch-3 passes, hard otherwise - voting, seconds), checked the same way."""
 import collections
 import time
 
@@ -54,16 +55,23 @@ def test_every_launch_of_a_forward_pass(case, precision, batch, switch_off, reco
     model = make_meta_arch(cfg["model_name"], **cfg["model"], precision=precision, max_batch=batch)
     model.load_state_dict(syn.synthetic_state_dict(cfg["model"], model_name, seed=wseed))
     model = model.to("cuda").eval()
+    if precision == "mixed" and batch == 3:
+        model.test_nms_method = "soft"               # the configs ship hard NMS; these passes check the soft path
     t0 = time.time()
-    model.dense_outputs(_items(use_video, batch))
+    launch_ref.reset_postprocess_stats()
+    model(_items(use_video, batch))                  # forward pass + decode / NMS / voting / seconds (postprocess)
     torch.cuda.synchronize()
     n = sum(recorder.count.values())
-    assert n > 0 and recorder.count["pack_feats"] == batch
+    assert n > 0 and recorder.count["pack_feats"] == batch and recorder.count["postprocess"] == 1
     for op in ("conv_gemm", "attention", "ln_dwconv_ln"):
         assert recorder.count[op] > 0, op
-    print("\nlaunch parity %s: %d launches checked in %.1f s; %s; worst error / bar: %s" % (
-        "-".join(str(v) for v in (case, precision, batch, switch_off) if v is not None), n, time.time() - t0,
-        dict(recorder.count), {k: round(v, 3) for k, v in sorted(recorder.worst.items())}))
+    ps = launch_ref.POSTPROCESS_STATS
+    assert ps["videos"] == batch
+    print("\nlaunch parity %s: %d launches checked in %.1f s; %s; worst error / bar: %s; postprocess (%s NMS): %d decode "
+          "points near the cut exempt, %d of them kept or dropped unlike float64; voting error / bound %.3g" % (
+              "-".join(str(v) for v in (case, precision, batch, switch_off) if v is not None), n, time.time() - t0,
+              dict(recorder.count), {k: round(v, 3) for k, v in sorted(recorder.worst.items())}, model.test_nms_method,
+              ps["near_cut"], ps["near_cut_moved"], recorder.worst_path.get(("postprocess", "out_segs"), 0.0)))
     for k, v in recorder.count.items():
         STATS[k][0] += v
         STATS[k][1] = max(STATS[k][1], recorder.worst.get(k, 0.0))

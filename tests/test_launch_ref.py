@@ -1,7 +1,7 @@
 """CPU checks of the float64 per-launch references (oracle/launch_ref.py) against independent torch formulations
 (nn.Conv1d / ConvTranspose1d / Conv2d, nn.LayerNorm, nn.InstanceNorm1d, F.interpolate, a dense band-masked softmax,
-torch.stft, BatchNorm + MaxPool2d), their mask semantics and error bounds, and a static check that every `ops` entry
-point the forward pass and the BYOL-A extractor call has a reference."""
+torch.stft, BatchNorm + MaxPool2d, the oracle's batched_nms and decode), their mask semantics and error bounds, and a
+static check that every `ops` entry point the forward pass and the BYOL-A extractor call has a reference."""
 import math
 import os
 import re
@@ -13,6 +13,9 @@ import torch.nn.functional as F
 
 import byola_ref
 import launch_ref as lr
+import model_ref
+import nms_ref
+import postprocess_cases as pc
 from audio_visual_deepfake_detection_b200.libs.features.byola import BatchPlan, LogMelSpectrogram
 from audio_visual_deepfake_detection_b200.libs.modeling.engine import up_weight
 from audio_visual_deepfake_detection_b200.libs.utils import synthetic as syn
@@ -513,6 +516,181 @@ def test_check_bound_exact_and_integer_paths():
         lr.check(m, lr.Out(torch.tensor([0.0, 1.0, 0.0], dtype=D), torch.ones(3, dtype=torch.bool), torch.zeros(3, dtype=torch.bool), None), 1, 0.0)
 
 
+# --------------------------------------------------------------------------------------------------- postprocess
+def warp_voting(picks, segs, scores, thr):
+    """csrc/nms.cu's voting in numpy float32, in the kernel's order: lane l sums candidates l, l + 32, ... (fma for the
+    coordinate sums), then a 5-level xor butterfly; the result of lane 0."""
+    picks, segs, sc = np.asarray(picks, np.float32), np.asarray(segs, np.float32), np.asarray(scores, np.float32)
+    n = len(sc)
+    out = np.zeros(picks.shape, np.float32)
+    b0, b1 = segs[:, 0], segs[:, 1]
+
+    def warp_sum(lanes):
+        for o in (16, 8, 4, 2, 1):
+            lanes = (lanes + lanes[np.arange(32) ^ o]).astype(np.float32)
+        return lanes[0]
+
+    with np.errstate(invalid="ignore", divide="ignore"):
+        for q, (a0, a1) in enumerate(picks):
+            inter = np.fmax(np.fmin(a1, b1) - np.fmax(a0, b0), np.float32(0))
+            iou = inter / (((a1 - a0) + (b1 - b0)) - inter)
+            w = ((iou >= np.float32(thr)).astype(np.float32) * sc) * iou
+            lanes = np.zeros(32, np.float32)
+            for j in range(n):
+                lanes[j % 32] = lanes[j % 32] + w[j]
+            sw = warp_sum(lanes)
+            for c, b in enumerate((b0, b1)):
+                lanes = np.zeros(32, np.float32)
+                for j in range(n):              # fma: one rounding of the exact w' * b + acc
+                    lanes[j % 32] = np.float32(float(w[j] / sw) * float(b[j]) + float(lanes[j % 32]))
+                out[q, c] = warp_sum(lanes)
+    return out
+
+
+def test_voting_ref_bounds_the_kernels_summation_order():
+    """The warp-ordered float32 voting lies within voting_ref's derived bound on every element, NaN exactly where the
+    float64 value is NaN (zero-length picks voting with themselves); a weight that drops its score misses the bound."""
+    worst = 0.0
+    for seed, fam in ((1, pc.grid_ties), (2, pc.zero_length), (3, pc.identical_segments)):
+        segs, sc = fam(700, seed)
+        idx = nms_ref.nms(segs, sc, 0.1)[:40]
+        val, bnd = lr.voting_ref(segs[idx], segs, sc, 0.75)
+        got = warp_voting(segs[idx], segs, sc, 0.75).astype(np.float64)
+        nan = np.isnan(val)
+        assert np.array_equal(nan, np.isnan(got))
+        if fam is pc.zero_length:
+            assert nan.any()
+        assert bool((bnd[~nan] > 0).all())
+        worst = max(worst, float((np.abs(got - val)[~nan] / bnd[~nan]).max()))
+        assert worst <= 1.0, (fam.__name__, worst)
+        unweighted = lr.voting_ref(segs[idx], segs, np.ones_like(sc), 0.75)[0]
+        ok = ~nan & ~np.isnan(unweighted)
+        assert float((np.abs(unweighted - val)[ok] / bnd[ok]).max()) > 100.0
+    print("voting: worst error / bound %.3g" % worst)
+
+
+def test_voting_ref_matches_the_c_oracle():
+    segs, sc = pc.grid_ties(500, 4)
+    idx = nms_ref.nms(segs, sc, 0.1)
+    val, bnd = lr.voting_ref(segs[idx], segs, sc, 0.9)
+    c = nms_ref.seg_voting(segs[idx], segs, sc, 0.9).astype(np.float64)
+    assert float((np.abs(c - val) / np.maximum(bnd, 1e-30)).max()) < 500        # sequential fp32 sum: same values, looser order
+
+
+def _emulated_decode(logits, offsets, mask, lens, topk, thr=0.001, dthr=0.001):
+    """The kernel's decode in numpy float32: sigmoid, the topk per level (descending, ties by point), duration cut."""
+    segs, scores = [], []
+    off = np.cumsum([0] + list(lens))
+    for l, n in enumerate(lens):
+        s = np.float32(2.0 ** l)
+        lg = logits[off[l]:off[l + 1]].astype(np.float32)
+        p = (np.float32(1) / (np.float32(1) + np.exp(-lg))) * mask[off[l]:off[l + 1]].astype(np.float32)
+        pts = np.nonzero(p > np.float32(thr))[0]
+        pts = pts[np.lexsort((pts, -p[pts]))][:topk]
+        tt = pts.astype(np.float32) * s
+        of = offsets[off[l]:off[l + 1]][pts]
+        left, right = tt - of[:, 0] * s, tt + of[:, 1] * s
+        ok = (right - left) > np.float32(dthr)
+        segs.append(np.stack([left, right], 1)[ok]); scores.append(p[pts][ok])
+    return np.concatenate(segs).astype(np.float32), np.concatenate(scores).astype(np.float32)
+
+
+def test_decode_check_accepts_the_kernel_rule_and_rejects_mutants():
+    """decode_check passes a float32 decode with the kernel's tie rule on the adversarial decode inputs (exact ties at
+    1.0f, duplicated logits, the topk cut inside a tied group, segments exactly duration_thresh long) and agrees with
+    the oracle's stable-sort decode; it rejects a tie broken the other way, a candidate one ulp off, a score 10 ulp
+    off, a dropped candidate."""
+    lens = [64, 33, 7, 1]
+    topk = 20
+    logits, offsets, mask = pc.decode_case(5, lens, topk)
+    strides = pc.decode_level_strides(lens)
+
+    class Stub(model_ref.OracleModel):
+        def __init__(self):
+            self.test_cfg = {"pre_nms_thresh": 0.001, "pre_nms_topk": topk, "duration_thresh": 0.001}
+            self.fpn_strides = [int(s) for s in strides]; self.num_classes = 1
+    off = np.cumsum([0] + lens)
+    for b in range(len(logits)):
+        segs, sc = _emulated_decode(logits[b], offsets[b], mask[b], lens, topk)
+        lr.reset_postprocess_stats()
+        pts, p64, s32 = lr.decode_check(logits[b], offsets[b], mask[b], lens, strides, 0.001, topk, 0.001, segs, sc, len(sc))
+        assert np.array_equal(s32, segs)
+        o_segs, o_sc, _ = Stub().decode([torch.from_numpy(logits[b, off[l]:off[l + 1]]).unsqueeze(-1) for l in range(len(lens))],
+                                        [torch.from_numpy(offsets[b, off[l]:off[l + 1]]) for l in range(len(lens))],
+                                        [torch.from_numpy(mask[b, off[l]:off[l + 1]].astype(bool)) for l in range(len(lens))])
+        assert np.array_equal(o_segs.numpy(), segs)            # torch's sigmoid may differ from numpy's by an ulp
+        assert bool((np.abs(o_sc.numpy().astype(np.float64) - sc) <= 2 * lr.SIGMOID_REL * sc).all())
+        if b == 2:
+            assert len(sc) == 0
+            continue
+        ties = np.nonzero((sc[1:] == sc[:-1]) & (np.diff(pts) > 0) & (np.diff(pts) < lens[0]))[0]
+        if len(ties):
+            i = ties[0]
+            bad = segs.copy(); bad[[i, i + 1]] = bad[[i + 1, i]]
+            if not np.array_equal(bad, segs):
+                with pytest.raises(AssertionError, match="out of order|no point"):
+                    lr.decode_check(logits[b], offsets[b], mask[b], lens, strides, 0.001, topk, 0.001, bad, sc, len(sc))
+        bad = segs.copy(); bad[0, 1] = np.nextafter(bad[0, 1], np.float32(np.inf))
+        with pytest.raises(AssertionError, match="no point"):
+            lr.decode_check(logits[b], offsets[b], mask[b], lens, strides, 0.001, topk, 0.001, bad, sc, len(sc))
+        bad = sc.copy(); bad[-1] = bad[-1] * np.float32(1 - 10 * 2.0 ** -24)
+        with pytest.raises(AssertionError, match="no point"):
+            lr.decode_check(logits[b], offsets[b], mask[b], lens, strides, 0.001, topk, 0.001, segs, bad, len(sc))
+        with pytest.raises(AssertionError, match="membership"):
+            # the last candidate is of a level shorter than topk: no cut there, its membership is certain
+            lr.decode_check(logits[b], offsets[b], mask[b], lens, strides, 0.001, topk, 0.001, segs[:-1], sc[:-1], len(sc) - 1)
+    # video 0: the topk cut of level 0 falls inside the saturated group, whose probabilities are all within the
+    # sigmoid's error of each other: those points are exempt, and counted
+    segs, sc = _emulated_decode(logits[0], offsets[0], mask[0], lens, topk)
+    lr.reset_postprocess_stats()
+    lr.decode_check(logits[0], offsets[0], mask[0], lens, strides, 0.001, topk, 0.001, segs, sc, len(sc))
+    assert lr.POSTPROCESS_STATS["near_cut"] > topk
+
+
+def test_postprocess_reference_is_the_oracles_batched_nms():
+    """Candidate mode, no voting: out_* of the reference are nms_ref.batched_nms's results (hard and soft), the
+    seconds conversion is model_ref's float32 formula bit for bit, out_index points at the picked candidates."""
+    cases = [pc.grid_ties(300, 6), pc.min_score_ties(150, 7), (np.zeros((0, 2), np.float32), np.zeros(0, np.float32))]
+    B, cap, K = len(cases), 300, 50
+    cs, cc = torch.zeros(B, cap, 2), torch.zeros(B, cap)
+    cn = torch.tensor([len(c[1]) for c in cases], dtype=torch.int32)
+    for b, (sg, sc) in enumerate(cases):
+        cs[b, :len(sc)] = torch.from_numpy(sg); cc[b, :len(sc)] = torch.from_numpy(sc)
+    meta = [torch.tensor([1.3, 0.7, 0.9], dtype=torch.float32), torch.tensor([0.65, 0.0, 2.0], dtype=torch.float32),
+            torch.tensor([25.0, 30.0, 25.0], dtype=torch.float32), torch.tensor([20.0, 9.5, 7.0], dtype=torch.float32)]
+    item = lambda b: {"feat_stride": float(meta[0][b]), "feat_num_frames": 2 * float(meta[1][b]), "fps": float(meta[2][b]),
+                      "duration": float(meta[3][b])}
+    for soft in (False, True):
+        o = lr.postprocess(B, cand_segs=cs, cand_scores=cc, cand_count=cn, iou_threshold=0.1, min_score=0.2, sigma=0.75,
+                           voting_thresh=0.0, max_seg_num=K, use_soft_nms=soft, vid_meta=meta, out_segs=torch.empty(B, K, 2),
+                           out_scores=torch.empty(B, K), out_count=torch.empty(B, dtype=torch.int32),
+                           out_index=torch.empty(B, K, dtype=torch.int32))
+        for b, (sg, sc) in enumerate(cases):
+            ws, wp, _ = nms_ref.batched_nms(torch.from_numpy(sg), torch.from_numpy(sc), torch.zeros(len(sc), dtype=torch.long),
+                                            0.1, 0.2, K, use_soft_nms=soft, multiclass=False, sigma=0.75,
+                                            voting_thresh=0.0)
+            k = len(wp)
+            assert int(o["out_count"].ref[b]) == k
+            assert torch.equal(o["out_scores"].ref[b, :k], wp.to(D)) and bool(o["out_scores"].written[b, :k].all())
+            assert not bool(o["out_scores"].written[b, k:].any())
+            fs, _, _ = model_ref.OracleModel.postprocess(type("S", (), {"test_cfg": {"nms_method": "none"}})(), ws, wp, None, item(b), None)
+            assert torch.equal(o["out_segs"].ref[b, :k], fs.reshape(-1, 2).to(D)) and bool((o["out_segs"].tol[b] == 0).all())
+            idx = o["out_index"].ref[b, :k].long()
+            if k:
+                assert torch.equal(cc[b, idx], wp) or soft               # soft: the scores are decayed
+
+
+def test_check_bound_zero_is_exact_and_nan_matches_nan():
+    ref = torch.tensor([1.0, float("nan"), 3.0], dtype=D)
+    w, z = torch.ones(3, dtype=torch.bool), torch.zeros(3, dtype=torch.bool)
+    tol = torch.tensor([0.0, 0.0, 1e-3], dtype=D)
+    assert lr.check(torch.tensor([1.0, float("nan"), 3.0005]), lr.Out(ref, w, z, None, tol), 3, 1.0) == pytest.approx(0.5, rel=1e-3)
+    with pytest.raises(AssertionError, match="error / bound"):
+        lr.check(torch.tensor([np.nextafter(np.float32(1), np.float32(2)), float("nan"), 3.0]), lr.Out(ref, w, z, None, tol), 3, 1.0)
+    with pytest.raises(AssertionError, match="error / bound"):
+        lr.check(torch.tensor([1.0, 2.0, 3.0]), lr.Out(ref, w, z, None, tol), 3, 1.0)
+
+
 # --------------------------------------------------------------------------------------------------- coverage
 def launched_entry_points():
     names = set()
@@ -523,14 +701,14 @@ def launched_entry_points():
     return names
 
 
-def test_every_launched_entry_point_has_a_reference():
+def test_every_launched_entry_point_has_a_reference_postprocess_included():
     from audio_visual_deepfake_detection_b200 import ops
     names = launched_entry_points()
     assert {"conv_gemm", "attention", "mlp_fused", "ln_dwconv_ln"} <= names
     assert {"logmel", "byola_conv1_pool", "byola_pool"} <= names
     missing = sorted(n for n in names if n not in lr.REFERENCES and n not in lr.EXCLUDED)
     assert not missing, "ops entry points launched by the forward pass without a float64 reference: %s" % missing
-    assert set(lr.EXCLUDED) == {"postprocess"}
+    assert "postprocess" in names and not lr.EXCLUDED
     import inspect
     for name, ref in lr.REFERENCES.items():           # the references take the entry points' own arguments
         assert list(inspect.signature(ref).parameters) == list(inspect.signature(getattr(ops, name)).parameters), name
