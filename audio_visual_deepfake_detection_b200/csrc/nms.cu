@@ -16,6 +16,8 @@
 //   * the gaussian weight uses a restatement of glibc's expf (double polynomial + table),
 //     which is what std::exp(float) resolves to in the reference build.
 #include <stdlib.h>
+#include <algorithm>
+#include <cmath>
 #include "common.cuh"
 
 namespace avdf {
@@ -509,6 +511,7 @@ constexpr int DEC_MAX_T = 2048;        // largest level length handled by the in
 
 struct DecodeParams {
   const float* logits; const float* offsets; const unsigned char* mask;
+  const int* valid_len;            // [B], used when mask == nullptr: point t of level l is kept iff t * stride_l < valid
   int B, P, n_levels;
   int lvl_off[AVDF_MAX_LEVELS]; int lvl_len[AVDF_MAX_LEVELS]; float lvl_stride[AVDF_MAX_LEVELS];
   float pre_nms_thresh; int pre_nms_topk; float duration_thresh;
@@ -528,7 +531,8 @@ __device__ int decode_block(const DecodeParams& d, int b, float* key, int* val, 
       float p = -1.f;        // sentinel below any probability
       if (t < T) {
         float lg = d.logits[(size_t)b * d.P + off + t];
-        float m = d.mask[(size_t)b * d.P + off + t] ? 1.f : 0.f;
+        const bool keep = d.mask ? d.mask[(size_t)b * d.P + off + t] != 0 : __fmul_rn((float)t, stride) < (float)d.valid_len[b];
+        float m = keep ? 1.f : 0.f;
         float pr = __fmul_rn(__fdiv_rn(1.f, __fadd_rn(1.f, expf(-lg))), m);
         p = (pr > d.pre_nms_thresh) ? pr : -1.f;
       }
@@ -590,6 +594,120 @@ __device__ int decode_block(const DecodeParams& d, int b, float* key, int* val, 
     __syncthreads();
   }
   return s_base;
+}
+
+// ---------------------------------------------------------------------------------------------
+// batched_nms of one video (nms.py:103-190, class-agnostic) from its decoded candidates: hard NMS (with NMSop's score
+// filter) or soft NMS, then seg_voting against ALL candidates. Shared by postprocess_kernel and postprocess_sweep_kernel.
+// ---------------------------------------------------------------------------------------------
+struct PickShared {    // the picks of one video: boundaries (voted when voting is on), scores, candidate index
+  float p_x1[AVDF_MAX_SEGS], p_x2[AVDF_MAX_SEGS], p_sc[AVDF_MAX_SEGS];
+  float dets[3 * AVDF_MAX_SEGS];
+  int idx[AVDF_MAX_SEGS];
+};
+
+// c: working arrays (shared memory or global workspace) of capacity >= n; all_segs / all_scores [n]: the candidates.
+// Returns the number of picks k <= K in ps (in pick order).
+__device__ int nms_vote_block(const Cand& c, const float* all_segs, const float* all_scores, int n, bool soft, int method,
+                              float iou_thr, float min_score, float sigma, float voting_thresh, int K, PickShared& ps,
+                              NmsShared& sh) {
+  float* p_x1 = ps.p_x1; float* p_x2 = ps.p_x2; float* p_sc = ps.p_sc;
+  float* dets_sh = ps.dets; int* idx_sh = ps.idx;
+  int k = 0;
+  if (n > 0) {
+    if (!soft) {
+      // NMSop: score filter first (nms.py:15-21), order preserved
+      for (int p = threadIdx.x; p < n; p += NMS_THREADS) {
+        float a = all_segs[2 * p], e = all_segs[2 * p + 1], s = all_scores[p];
+        c.x1[p] = a; c.x2[p] = e; c.sc[p] = s; c.ar[p] = __fadd_rn(__fsub_rn(e, a), 1e-6f);
+        bool keep = (min_score > 0.f) ? (s > min_score) : true;
+        c.id[p] = keep ? p : ~p;
+      }
+      __syncthreads();
+      k = hard_nms_block(c, n, iou_thr, K, idx_sh, sh);
+      __syncthreads();
+      for (int q = threadIdx.x; q < k; q += NMS_THREADS) {
+        int p = idx_sh[q];
+        p_x1[q] = c.x1[p]; p_x2[q] = c.x2[p]; p_sc[q] = c.sc[p];
+      }
+    } else {
+      for (int p = threadIdx.x; p < n; p += NMS_THREADS) {
+        float a = all_segs[2 * p], e = all_segs[2 * p + 1];
+        c.x1[p] = a; c.x2[p] = e; c.sc[p] = all_scores[p]; c.ar[p] = __fadd_rn(__fsub_rn(e, a), 1e-6f);
+        c.id[p] = p;
+      }
+      __syncthreads();
+      k = soft_nms_block(c, n, iou_thr, sigma, min_score, method, K, dets_sh, idx_sh, sh);
+      __syncthreads();
+      for (int q = threadIdx.x; q < k; q += NMS_THREADS) {
+        p_x1[q] = dets_sh[3 * q]; p_x2[q] = dets_sh[3 * q + 1]; p_sc[q] = dets_sh[3 * q + 2];
+      }
+    }
+    __syncthreads();
+    // seg_voting (nms.py:67-101) against ALL candidates, one warp per pick
+    if (voting_thresh > 0.f && k > 0) {
+      const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+      for (int q = w; q < k; q += NMS_WARPS) {
+        const float a0 = p_x1[q], a1 = p_x2[q], la = __fsub_rn(a1, a0);
+        float sw = 0.f;
+        for (int j = lane; j < n; j += 32) {
+          float b0 = all_segs[2 * j], b1 = all_segs[2 * j + 1];
+          float inter = fmaxf(__fsub_rn(fminf(a1, b1), fmaxf(a0, b0)), 0.f);
+          float iou = __fdiv_rn(inter, __fsub_rn(__fadd_rn(la, __fsub_rn(b1, b0)), inter));
+          float wgt = __fmul_rn(__fmul_rn((iou >= voting_thresh) ? 1.f : 0.f, all_scores[j]), iou);
+          sw += wgt;
+        }
+        sw = warp_sum(sw);
+        float s0 = 0.f, s1 = 0.f;
+        for (int j = lane; j < n; j += 32) {
+          float b0 = all_segs[2 * j], b1 = all_segs[2 * j + 1];
+          float inter = fmaxf(__fsub_rn(fminf(a1, b1), fmaxf(a0, b0)), 0.f);
+          float iou = __fdiv_rn(inter, __fsub_rn(__fadd_rn(la, __fsub_rn(b1, b0)), inter));
+          float wgt = __fmul_rn(__fmul_rn((iou >= voting_thresh) ? 1.f : 0.f, all_scores[j]), iou);
+          wgt = __fdiv_rn(wgt, sw);
+          s0 = fmaf(wgt, b0, s0); s1 = fmaf(wgt, b1, s1);
+        }
+        s0 = warp_sum(s0); s1 = warp_sum(s1);
+        __syncwarp();
+        if (lane == 0) { dets_sh[3 * q] = s0; dets_sh[3 * q + 1] = s1; }
+      }
+      __syncthreads();
+      for (int q = threadIdx.x; q < k; q += NMS_THREADS) { p_x1[q] = dets_sh[3 * q]; p_x2[q] = dets_sh[3 * q + 1]; }
+      __syncthreads();
+    }
+  }
+  return k;
+}
+
+struct VideoMeta { bool to_sec; float st, hn, fps, dur; };
+__device__ __forceinline__ VideoMeta video_meta(const float* stride, const float* half_nframes, const float* fps,
+                                                const float* duration, int b) {
+  VideoMeta m; m.to_sec = fps != nullptr; m.st = 1.f; m.hn = 0.f; m.fps = 1.f; m.dur = 0.f;
+  if (m.to_sec) { m.st = stride[b]; m.hn = half_nframes[b]; m.fps = fps[b]; m.dur = duration[b]; }
+  return m;
+}
+
+// final stable sort by score desc + cap (nms.py:184-189): rank by counting (k <= AVDF_MAX_SEGS), then feature grid ->
+// seconds with the reference's clamping (av_fd_no_recon.py:860-865). o_segs [k, 2] / o_scores [k] in output order.
+__device__ void rank_seconds_block(const PickShared& ps, int k, const VideoMeta& m, float* o_segs, float* o_scores,
+                                   int* out_index) {
+  const float* p_sc = ps.p_sc;
+  for (int q = threadIdx.x; q < k; q += NMS_THREADS) {
+    float s = p_sc[q];
+    int rank = 0;
+    for (int r = 0; r < k; ++r) rank += (p_sc[r] > s || (p_sc[r] == s && r < q)) ? 1 : 0;
+    float v0 = ps.p_x1[q], v1 = ps.p_x2[q];
+    if (m.to_sec) {
+      v0 = __fdiv_rn(__fadd_rn(__fmul_rn(v0, m.st), m.hn), m.fps);
+      v1 = __fdiv_rn(__fadd_rn(__fmul_rn(v1, m.st), m.hn), m.fps);
+      if (v0 <= 0.f) v0 = __fmul_rn(v0, 0.f);
+      if (v1 <= 0.f) v1 = __fmul_rn(v1, 0.f);
+      if (v0 >= m.dur) v0 = __fadd_rn(__fmul_rn(v0, 0.f), m.dur);
+      if (v1 >= m.dur) v1 = __fadd_rn(__fmul_rn(v1, 0.f), m.dur);
+    }
+    o_segs[2 * rank] = v0; o_segs[2 * rank + 1] = v1; o_scores[rank] = s;
+    if (out_index) out_index[rank] = ps.idx[q];
+  }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -658,92 +776,11 @@ __global__ void __launch_bounds__(NMS_THREADS, 1) postprocess_kernel(const PostP
   // pick buffers live after the candidate arrays' hole[] region is no longer needed -> use out_* directly
   float* o_segs = prm.out_segs + (size_t)b * K * 2;
   float* o_scores = prm.out_scores + (size_t)b * K;
-  __shared__ float p_x1[AVDF_MAX_SEGS], p_x2[AVDF_MAX_SEGS], p_sc[AVDF_MAX_SEGS];
-  __shared__ float dets_sh[3 * AVDF_MAX_SEGS];
-  __shared__ int idx_sh[AVDF_MAX_SEGS];
-  int k = 0;
-  if (n > 0) {
-    if (!prm.soft) {
-      // NMSop: score filter first (nms.py:15-21), order preserved
-      for (int p = threadIdx.x; p < n; p += NMS_THREADS) {
-        float a = all_segs[2 * p], e = all_segs[2 * p + 1], s = all_scores[p];
-        c.x1[p] = a; c.x2[p] = e; c.sc[p] = s; c.ar[p] = __fadd_rn(__fsub_rn(e, a), 1e-6f);
-        bool keep = (prm.min_score > 0.f) ? (s > prm.min_score) : true;
-        c.id[p] = keep ? p : ~p;
-      }
-      __syncthreads();
-      k = hard_nms_block(c, n, prm.iou_thr, K, idx_sh, sh);
-      __syncthreads();
-      for (int q = threadIdx.x; q < k; q += NMS_THREADS) {
-        int p = idx_sh[q];
-        p_x1[q] = c.x1[p]; p_x2[q] = c.x2[p]; p_sc[q] = c.sc[p];
-      }
-    } else {
-      for (int p = threadIdx.x; p < n; p += NMS_THREADS) {
-        float a = all_segs[2 * p], e = all_segs[2 * p + 1];
-        c.x1[p] = a; c.x2[p] = e; c.sc[p] = all_scores[p]; c.ar[p] = __fadd_rn(__fsub_rn(e, a), 1e-6f);
-        c.id[p] = p;
-      }
-      __syncthreads();
-      k = soft_nms_block(c, n, prm.iou_thr, prm.sigma, prm.min_score, prm.method, K, dets_sh, idx_sh, sh);
-      __syncthreads();
-      for (int q = threadIdx.x; q < k; q += NMS_THREADS) {
-        p_x1[q] = dets_sh[3 * q]; p_x2[q] = dets_sh[3 * q + 1]; p_sc[q] = dets_sh[3 * q + 2];
-      }
-    }
-    __syncthreads();
-    // seg_voting (nms.py:67-101) against ALL candidates, one warp per pick
-    if (prm.voting_thresh > 0.f && k > 0) {
-      const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-      for (int q = w; q < k; q += NMS_WARPS) {
-        const float a0 = p_x1[q], a1 = p_x2[q], la = __fsub_rn(a1, a0);
-        float sw = 0.f;
-        for (int j = lane; j < n; j += 32) {
-          float b0 = all_segs[2 * j], b1 = all_segs[2 * j + 1];
-          float inter = fmaxf(__fsub_rn(fminf(a1, b1), fmaxf(a0, b0)), 0.f);
-          float iou = __fdiv_rn(inter, __fsub_rn(__fadd_rn(la, __fsub_rn(b1, b0)), inter));
-          float wgt = __fmul_rn(__fmul_rn((iou >= prm.voting_thresh) ? 1.f : 0.f, all_scores[j]), iou);
-          sw += wgt;
-        }
-        sw = warp_sum(sw);
-        float s0 = 0.f, s1 = 0.f;
-        for (int j = lane; j < n; j += 32) {
-          float b0 = all_segs[2 * j], b1 = all_segs[2 * j + 1];
-          float inter = fmaxf(__fsub_rn(fminf(a1, b1), fmaxf(a0, b0)), 0.f);
-          float iou = __fdiv_rn(inter, __fsub_rn(__fadd_rn(la, __fsub_rn(b1, b0)), inter));
-          float wgt = __fmul_rn(__fmul_rn((iou >= prm.voting_thresh) ? 1.f : 0.f, all_scores[j]), iou);
-          wgt = __fdiv_rn(wgt, sw);
-          s0 = fmaf(wgt, b0, s0); s1 = fmaf(wgt, b1, s1);
-        }
-        s0 = warp_sum(s0); s1 = warp_sum(s1);
-        __syncwarp();
-        if (lane == 0) { dets_sh[3 * q] = s0; dets_sh[3 * q + 1] = s1; }
-      }
-      __syncthreads();
-      for (int q = threadIdx.x; q < k; q += NMS_THREADS) { p_x1[q] = dets_sh[3 * q]; p_x2[q] = dets_sh[3 * q + 1]; }
-      __syncthreads();
-    }
-  }
-  // final stable sort by score desc + cap (nms.py:184-189): rank by counting (k <= AVDF_MAX_SEGS)
-  float st = 1.f, hn = 0.f, fps = 1.f, dur = 0.f;
-  const bool to_sec = prm.vid_fps != nullptr;
-  if (to_sec) { st = prm.vid_stride[b]; hn = prm.vid_half_nframes[b]; fps = prm.vid_fps[b]; dur = prm.vid_duration[b]; }
-  for (int q = threadIdx.x; q < k; q += NMS_THREADS) {
-    float s = p_sc[q];
-    int rank = 0;
-    for (int r = 0; r < k; ++r) rank += (p_sc[r] > s || (p_sc[r] == s && r < q)) ? 1 : 0;
-    float v0 = p_x1[q], v1 = p_x2[q];
-    if (to_sec) {      // av_fd_no_recon.py:860-865
-      v0 = __fdiv_rn(__fadd_rn(__fmul_rn(v0, st), hn), fps);
-      v1 = __fdiv_rn(__fadd_rn(__fmul_rn(v1, st), hn), fps);
-      if (v0 <= 0.f) v0 = __fmul_rn(v0, 0.f);
-      if (v1 <= 0.f) v1 = __fmul_rn(v1, 0.f);
-      if (v0 >= dur) v0 = __fadd_rn(__fmul_rn(v0, 0.f), dur);
-      if (v1 >= dur) v1 = __fadd_rn(__fmul_rn(v1, 0.f), dur);
-    }
-    o_segs[2 * rank] = v0; o_segs[2 * rank + 1] = v1; o_scores[rank] = s;
-    if (prm.out_index) prm.out_index[(size_t)b * K + rank] = idx_sh[q];
-  }
+  __shared__ PickShared ps;
+  const int k = nms_vote_block(c, all_segs, all_scores, n, prm.soft != 0, prm.method, prm.iou_thr, prm.min_score, prm.sigma,
+                               prm.voting_thresh, K, ps, sh);
+  VideoMeta vm = video_meta(prm.vid_stride, prm.vid_half_nframes, prm.vid_fps, prm.vid_duration, b);
+  rank_seconds_block(ps, k, vm, o_segs, o_scores, prm.out_index ? prm.out_index + (size_t)b * K : nullptr);
   if (threadIdx.x == 0) prm.out_count[b] = k;
   if (prm.rec_ring != nullptr) {
     // one fixed-size record per video into the ring: [index, count, video_cls, scores[K], segs[K][2]]
@@ -767,6 +804,75 @@ __global__ void __launch_bounds__(NMS_THREADS, 1) postprocess_kernel(const PostP
 }
 
 static size_t nms_smem_bytes() { return (size_t)NMS_SMEM_CAP * 6 * sizeof(float); }
+
+// ---------------------------------------------------------------------------------------------
+// postprocess sweep: many test_cfg settings over the same dense outputs. One CTA per video (persistent over the batch);
+// the settings arrive sorted by decode group (equal pre_nms_thresh / pre_nms_topk / duration_thresh): the CTA decodes
+// once per group into its workspace slice and runs every NMS setting of the group from that list, with the same device
+// functions as postprocess_kernel. The candidate arrays are sized to the pyramid (not NMS_SMEM_CAP), so two CTAs fit on
+// an SM where postprocess_kernel fits one. A decoded list never exceeds the shared-memory capacity: decode takes levels
+// of <= DEC_MAX_T points, and a pyramid of halving levels holds < 2 * DEC_MAX_T points.
+// ---------------------------------------------------------------------------------------------
+constexpr int SWEEP_MAX = 64;            // settings per launch
+constexpr int SWEEP_MAX_CTAS = 1024;     // persistent grid: the workspace holds one candidate list per CTA
+constexpr int SWEEP_MIN_BLOCKS = 2;
+struct SweepDecode { float pre_nms_thresh; int pre_nms_topk; float duration_thresh; };
+struct SweepSetting { float iou_thr, min_score, sigma, voting_thresh; int max_num, soft, group, row; };
+struct SweepParams {
+  DecodeParams dec;                      // logits / offsets / valid_len / levels (thresholds come from grp[])
+  SweepDecode grp[SWEEP_MAX]; int n_groups;
+  SweepSetting set[SWEEP_MAX]; int n_set;        // sorted by group; set[i].row = the setting's index in the caller's table
+  const float* vid_stride; const float* vid_half_nframes; const float* vid_fps; const float* vid_duration;
+  const float* vid_cls; const int* vid_index;
+  float* out_rows; long long rows_per_setting; int row_k;
+  void* ws; size_t ws_per_cta; int cap_sh;       // cap_sh: capacity of the shared-memory candidate arrays (>= P)
+};
+static_assert(2 * DEC_MAX_T <= NMS_SMEM_CAP, "a decoded pyramid must fit the shared-memory candidate arrays");
+
+static size_t sweep_ws_per_cta(int P) { return ((size_t)P * 3 * sizeof(float) + 255) / 256 * 256; }   // segments [P, 2] + scores [P]
+
+__global__ void __launch_bounds__(NMS_THREADS, SWEEP_MIN_BLOCKS) postprocess_sweep_kernel(const SweepParams prm) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ NmsShared sh;
+  __shared__ PickShared ps;
+  __shared__ int s_n;
+  const int P = prm.dec.P, K = prm.row_k, rec_len = 3 + 3 * prm.row_k;
+  unsigned char* ws = reinterpret_cast<unsigned char*>(prm.ws) + (size_t)blockIdx.x * prm.ws_per_cta;
+  float* all_segs = reinterpret_cast<float*>(ws);
+  float* all_scores = all_segs + 2 * (size_t)P;
+  float* key = reinterpret_cast<float*>(smem_raw);
+  int* val = reinterpret_cast<int*>(key + DEC_MAX_T);
+  for (int b = blockIdx.x; b < prm.dec.B; b += gridDim.x) {
+    const long long row = prm.vid_index ? prm.vid_index[b] : b;
+    const bool row_ok = row >= 0 && row < prm.rows_per_setting;
+    const VideoMeta vm = video_meta(prm.vid_stride, prm.vid_half_nframes, prm.vid_fps, prm.vid_duration, b);
+    const float vcls = prm.vid_cls ? prm.vid_cls[b] : 0.f;
+    int si = 0;
+    for (int g = 0; g < prm.n_groups; ++g) {
+      DecodeParams d = prm.dec;
+      d.pre_nms_thresh = prm.grp[g].pre_nms_thresh; d.pre_nms_topk = prm.grp[g].pre_nms_topk;
+      d.duration_thresh = prm.grp[g].duration_thresh;
+      __syncthreads();                                 // the previous setting is done with smem_raw / the candidates
+      const int cnt = decode_block(d, b, key, val, all_segs, all_scores);
+      if (threadIdx.x == 0) s_n = cnt;
+      __syncthreads();
+      const int n = s_n;
+      __threadfence_block();
+      const Cand c = carve(smem_raw, prm.cap_sh);
+      for (; si < prm.n_set && prm.set[si].group == g; ++si) {
+        const SweepSetting& st = prm.set[si];
+        __syncthreads();                               // the previous setting's tail is done with ps
+        const int k = nms_vote_block(c, all_segs, all_scores, n, st.soft != 0, 2, st.iou_thr, st.min_score, st.sigma,
+                                     st.voting_thresh, st.max_num, ps, sh);
+        if (!row_ok) continue;
+        float* rec = prm.out_rows + ((size_t)st.row * prm.rows_per_setting + row) * rec_len;
+        rank_seconds_block(ps, k, vm, rec + 3 + K, rec + 3, nullptr);
+        if (threadIdx.x == 0) { rec[0] = (float)row; rec[1] = (float)k; rec[2] = vcls; }
+        for (int q = k + threadIdx.x; q < K; q += NMS_THREADS) { rec[3 + q] = 0.f; rec[3 + K + 2 * q] = 0.f; rec[3 + K + 2 * q + 1] = 0.f; }
+      }
+    }
+  }
+}
 
 }  // namespace avdf
 
@@ -906,4 +1012,90 @@ extern "C" int avdf_postprocess(const avdf_postprocess_args* a, void* stream) {
   AVDF_SMEM_ATTR_ONCE(postprocess_kernel, nms_smem_bytes());
   postprocess_kernel<<<a->batch, NMS_THREADS, nms_smem_bytes(), reinterpret_cast<cudaStream_t>(stream)>>>(p);
   return check_launch("postprocess_kernel");
+}
+
+static int sweep_points(int32_t n_levels, const int32_t* level_len) {
+  if (n_levels <= 0 || n_levels > AVDF_MAX_LEVELS) return -1;
+  int P = 0;
+  for (int l = 0; l < n_levels; ++l) {
+    if (level_len[l] <= 0 || level_len[l] > DEC_MAX_T) return -1;
+    P += level_len[l];
+  }
+  return P;
+}
+
+extern "C" size_t avdf_postprocess_sweep_workspace_bytes(int32_t batch, int32_t n_points) {
+  if (batch <= 0 || n_points <= 0) return 0;
+  return (size_t)std::min(batch, SWEEP_MAX_CTAS) * sweep_ws_per_cta(n_points);
+}
+
+extern "C" int avdf_postprocess_sweep(const avdf_postprocess_sweep_args* a, void* stream) {
+  AVDF_CHECK_ARG(a != nullptr, "args is null");
+  AVDF_CHECK_ARG(a->batch >= 0, "batch < 0");
+  AVDF_CHECK_ARG(a->n_settings >= 1 && a->n_settings <= SWEEP_MAX, "n_settings must be 1..64");
+  AVDF_CHECK_ARG(a->settings != nullptr, "settings is null");
+  AVDF_CHECK_ARG(a->row_k >= 1 && a->row_k <= AVDF_MAX_SEGS, "row_k out of range");
+  const int P = sweep_points(a->n_levels, a->level_len);
+  AVDF_CHECK_ARG(P > 0 && P <= NMS_SMEM_CAP, "n_levels or a level length out of range");
+  for (int l = 0; l < a->n_levels; ++l)
+    AVDF_CHECK_ARG(std::isfinite(a->level_stride[l]) && a->level_stride[l] > 0.f, "level_stride must be finite and > 0");
+  SweepParams p{};
+  for (int i = 0; i < a->n_settings; ++i) {
+    const avdf_sweep_setting& s = a->settings[i];
+    AVDF_CHECK_ARG(std::isfinite(s.pre_nms_thresh) && std::isfinite(s.duration_thresh) && std::isfinite(s.iou_threshold) &&
+                   std::isfinite(s.min_score) && std::isfinite(s.sigma) && std::isfinite(s.voting_thresh),
+                   "a setting holds a non-finite value");
+    AVDF_CHECK_ARG(s.use_soft_nms == 0 || s.use_soft_nms == 1, "use_soft_nms must be 0 (hard) or 1 (soft)");
+    AVDF_CHECK_ARG(s.max_seg_num >= 1 && s.max_seg_num <= a->row_k, "max_seg_num must be 1..row_k");
+    AVDF_CHECK_ARG(s.pre_nms_topk >= 0, "pre_nms_topk < 0");
+    AVDF_CHECK_ARG(!s.use_soft_nms || s.sigma > 0.f, "soft NMS needs sigma > 0");
+  }
+  AVDF_CHECK_ARG(a->rows_per_setting >= 1 && (a->vid_index != nullptr || a->rows_per_setting >= a->batch),
+                 "rows_per_setting smaller than the batch");
+  AVDF_CHECK_ARG(a->out_rows != nullptr, "out_rows is null");
+  if (a->vid_fps) AVDF_CHECK_ARG(a->vid_feat_stride && a->vid_half_nframes && a->vid_duration, "incomplete video meta arrays");
+  if (a->batch == 0) return AVDF_OK;
+  AVDF_CHECK_ARG(a->logits && a->offsets && a->valid_len, "logits, offsets and valid_len are required");
+  const size_t need = avdf_postprocess_sweep_workspace_bytes(a->batch, P);
+  AVDF_CHECK_ARG(a->workspace != nullptr && a->workspace_bytes >= need, "workspace too small");
+  // decode groups in order of first appearance; the settings of a group run one after the other from its candidate list
+  int n_groups = 0;
+  int grp_of[SWEEP_MAX];
+  for (int i = 0; i < a->n_settings; ++i) {
+    const avdf_sweep_setting& s = a->settings[i];
+    int g = 0;
+    for (; g < n_groups; ++g)
+      if (p.grp[g].pre_nms_thresh == s.pre_nms_thresh && p.grp[g].pre_nms_topk == s.pre_nms_topk &&
+          p.grp[g].duration_thresh == s.duration_thresh) break;
+    if (g == n_groups) { p.grp[g] = SweepDecode{s.pre_nms_thresh, s.pre_nms_topk, s.duration_thresh}; ++n_groups; }
+    grp_of[i] = g;
+  }
+  p.n_groups = n_groups;
+  for (int g = 0; g < n_groups; ++g)
+    for (int i = 0; i < a->n_settings; ++i) {
+      if (grp_of[i] != g) continue;
+      const avdf_sweep_setting& s = a->settings[i];
+      p.set[p.n_set++] = SweepSetting{s.iou_threshold, s.min_score, s.sigma, s.voting_thresh, s.max_seg_num, s.use_soft_nms, g, i};
+    }
+  DecodeParams& d = p.dec;
+  d.logits = a->logits; d.offsets = a->offsets; d.mask = nullptr; d.valid_len = a->valid_len;
+  d.B = a->batch; d.n_levels = a->n_levels; d.P = P;
+  int off = 0;
+  for (int l = 0; l < a->n_levels; ++l) {
+    d.lvl_off[l] = off; d.lvl_len[l] = a->level_len[l]; d.lvl_stride[l] = a->level_stride[l];
+    off += a->level_len[l];
+  }
+  p.vid_stride = a->vid_feat_stride; p.vid_half_nframes = a->vid_half_nframes; p.vid_fps = a->vid_fps;
+  p.vid_duration = a->vid_duration; p.vid_cls = a->vid_cls; p.vid_index = a->vid_index;
+  p.out_rows = a->out_rows; p.rows_per_setting = a->rows_per_setting; p.row_k = a->row_k;
+  p.ws = a->workspace; p.ws_per_cta = sweep_ws_per_cta(P);
+  p.cap_sh = P;
+  int max_t = 1;
+  for (int l = 0; l < a->n_levels; ++l) { int np2 = 1; while (np2 < a->level_len[l]) np2 <<= 1; max_t = std::max(max_t, np2); }
+  // the decode's sort keys (key / val) and the candidate arrays share the dynamic shared memory
+  const size_t smem = std::max((size_t)p.cap_sh * 6 * sizeof(float), (size_t)(DEC_MAX_T + max_t) * sizeof(float));
+  AVDF_SMEM_ATTR_ONCE(postprocess_sweep_kernel, nms_smem_bytes());
+  const int grid = std::min(a->batch, SWEEP_MAX_CTAS);
+  postprocess_sweep_kernel<<<grid, NMS_THREADS, smem, reinterpret_cast<cudaStream_t>(stream)>>>(p);
+  return check_launch("postprocess_sweep_kernel");
 }

@@ -133,6 +133,59 @@ class PackedWeights:
 PRECISIONS = ("mixed", "fp32")
 
 
+class DenseStore:
+    """Caller-owned device copy of what the in-graph post-processing reads, batch after batch: pyramid logits [P],
+    offsets [P, 2], video_cls, the four seconds-conversion scalars (feat_stride, half frames, fps, duration) and the valid
+    length of every video (the pyramid mask is rebuilt from it). Pass it as `dense=` to `forward_streams`, `stream` or
+    `model(video_list)` (feats items); libs/utils/sweep.py then post-processes the kept outputs under many test_cfg
+    settings without another forward pass. About 18 KB per video at max_seq_len 768.
+
+    Videos are kept in the order they were added, in chunks of `chunk` videos that share one pyramid layout (feats items
+    longer than max_seq_len are padded to other lengths)."""
+
+    def __init__(self, chunk=4096):
+        self.chunk = int(chunk)
+        self.ids = []
+        self.chunks = []              # dicts: L, level_len, level_stride, n, logits, offsets, vcls, meta, valid, pos (host)
+        self._open = {}               # L -> chunk being filled
+
+    def __len__(self):
+        return len(self.ids)
+
+    def nbytes(self):
+        return sum(sum(c[k].numel() * c[k].element_size() for k in ("logits", "offsets", "vcls", "meta")) for c in self.chunks)
+
+    def add(self, ids, L, level_len, level_stride, logits, offsets, vcls, meta, valid):
+        """Device-to-device copies (on the current stream) of a batch: logits [B, P], offsets [B, P, 2], vcls [B],
+        meta [4, B] fp32 (device); valid: host ints [B]."""
+        B, P = logits.shape
+        pos0 = len(self.ids)
+        self.ids.extend(ids)
+        done = 0
+        while done < B:
+            c = self._open.get(L)
+            if c is None or c["n"] == self.chunk:
+                dev = logits.device
+                c = {"L": L, "level_len": list(level_len), "level_stride": list(level_stride), "n": 0,
+                     "logits": torch.empty((self.chunk, P), dtype=torch.float32, device=dev),
+                     "offsets": torch.empty((self.chunk, P, 2), dtype=torch.float32, device=dev),
+                     "vcls": torch.empty((self.chunk,), dtype=torch.float32, device=dev),
+                     "meta": torch.empty((4, self.chunk), dtype=torch.float32, device=dev),
+                     "valid": np.zeros(self.chunk, np.int32), "pos": np.zeros(self.chunk, np.int32)}
+                self.chunks.append(c)
+                self._open[L] = c
+            m = min(B - done, self.chunk - c["n"])
+            dst, src = slice(c["n"], c["n"] + m), slice(done, done + m)
+            c["logits"][dst].copy_(logits[src], non_blocking=True)
+            c["offsets"][dst].copy_(offsets[src], non_blocking=True)
+            c["vcls"][dst].copy_(vcls[src], non_blocking=True)
+            c["meta"][:, dst].copy_(meta[:, src], non_blocking=True)
+            c["valid"][dst] = np.asarray(valid[done:done + m], np.int32)
+            c["pos"][dst] = np.arange(pos0 + done, pos0 + done + m, dtype=np.int32)
+            c["n"] += m
+            done += m
+
+
 class LocalizationEngine:
     def __init__(self, model_cfg, model_name, state_dict, device, precision="mixed", max_batch=32):
         if not torch.cuda.is_available():
@@ -611,6 +664,10 @@ class LocalizationEngine:
                        w.vec("cls_head.cls_head.conv.bias"), w.dense("reg_head.offset_head.conv.weight", torch.float32),
                        w.vec("reg_head.offset_head.conv.bias"), self._scales, logits, offsets, batch=B, level_len=lens)
         return logits, offsets, vcls, masks, lens
+
+    def keep_dense(self, store, ids, L, logits, offsets, vcls, meta, valid):
+        """Copy a batch's dense outputs at padded length L (what `postprocess` reads) into a DenseStore."""
+        store.add(ids, L, self.level_lens(L), [float(s) for s in self.strides], logits, offsets, vcls, meta, valid)
 
     def postprocess(self, logits, offsets, masks, lens, meta, nms_method=None, records=None, vcls=None):
         """meta: device fp32 [4, B] rows = feat_stride, 0.5*feat_num_frames, fps, duration (or None).

@@ -155,20 +155,22 @@ class _LocalizationBase(nn.Module):
         return self._engine
 
     # ------------------------------------------------------------------ forward
-    def forward(self, video_list):
+    def forward(self, video_list, dense=None):
+        """dense: optional DenseStore (libs/modeling/engine.py) that keeps every batch's dense outputs for
+        libs/utils/sweep.py; the results are the same with or without it."""
         if self.training:
             raise NotImplementedError("training (losses / label assignment) is outside the accelerated inference path")
         if len(video_list) and "feats" not in video_list[0] and "streams" in video_list[0]:
             # items of the inference datasets of this package: raw streams, resampled on the GPU
-            return self.forward_streams(video_list)
+            return self.forward_streams(video_list, dense=dense)
         out = []
         for i in range(0, len(video_list), self.max_batch):
-            out.extend(self._forward_items(video_list[i:i + self.max_batch]))
+            out.extend(self._forward_items(video_list[i:i + self.max_batch], dense))
         return out
 
     @torch.no_grad()
     @_on_model_device
-    def _forward_items(self, items):
+    def _forward_items(self, items, dense=None):
         eng = self.engine()
         B = len(items)
         lens = [int(it["feats"].shape[-1]) for it in items]
@@ -180,7 +182,7 @@ class _LocalizationBase(nn.Module):
                 raise AvdfError("feats has %d channels, model expects %d" % (f.shape[0], eng.c_in))
             f = f.to(device=eng.device, dtype=torch.float32, non_blocking=True).contiguous()
             ops.pack_feats(f, x[b])
-        return self._run(eng, x, lens, items)
+        return self._run(eng, x, lens, items, dense)
 
     @torch.no_grad()
     @_on_model_device
@@ -198,7 +200,7 @@ class _LocalizationBase(nn.Module):
         return logits.cpu(), offsets.cpu(), vcls.cpu()
 
     @torch.no_grad()
-    def forward_streams(self, batch, window=None, hop=None):
+    def forward_streams(self, batch, window=None, hop=None, dense=None):
         """batch: list of dicts {video_id, duration, streams: {'video'?: [T_v,256], 'byola': [T_b,2048],
         'emo': [T_e,768]} fp32 numpy/torch, time-major like the `.npy` files}. Runs the dataset's resampling to
         max_seq_len + concat (deepfake_video_audio.py:513-547) on the GPU, then the model; returns the same list
@@ -207,23 +209,31 @@ class _LocalizationBase(nn.Module):
         window / hop (seconds, hop defaults to window / 2): recordings longer than `window` are cut into overlapping
         windows that each run at the model's trained time scale, and their results are merged on the GPU into one
         result per recording (libs/modeling/windows.py). Recordings no longer than `window` give exactly the
-        result they give without it."""
+        result they give without it.
+
+        dense: optional DenseStore (libs/modeling/engine.py): every batch's dense outputs are copied into it on the
+        device after the pass, for libs/utils/sweep.py. Not with windows."""
         runner = self.runner()
         if window is not None:
+            if dense is not None:
+                raise AvdfError("dense outputs are kept per video pass, not for sliding windows")
             return runner.run_windows(batch, window, hop)
         out = []
         for i in range(0, len(batch), self.max_batch):
-            out.extend(runner.run(batch[i:i + self.max_batch]))
+            out.extend(runner.run(batch[i:i + self.max_batch], dense=dense))
         return out
 
     @torch.no_grad()
-    def stream(self, batches, window=None, hop=None):
+    def stream(self, batches, window=None, hop=None, dense=None):
         """Pipelined variant for serving loops: `for results in model.stream(iterable_of_batches)` overlaps the
         host-side packing of batch i+1 with the copies and GPU work of batch i (two pinned staging slots).
-        window / hop: as forward_streams; each batch's recordings are windowed and merged, one result per recording."""
+        window / hop: as forward_streams; each batch's recordings are windowed and merged, one result per recording.
+        dense: as forward_streams."""
         if window is None:
-            yield from self.runner().stream(batches)
+            yield from self.runner().stream(batches, dense=dense)
             return
+        if dense is not None:
+            raise AvdfError("dense outputs are kept per video pass, not for sliding windows")
         runner = self.runner()
         for chunk in batches:
             yield runner.run_windows(chunk, window, hop)
@@ -303,7 +313,7 @@ class _LocalizationBase(nn.Module):
         osg, osc, ocn = eng.postprocess(logits, offsets, masks, lens, staged["meta"], nms_method=self.test_nms_method,
                                         records=rec, vcls=vcls)
         eng.lane = 0
-        return {"ids": staged["ids"], "segs": osg, "scores": osc, "counts": ocn, "vcls": vcls}
+        return {"ids": staged["ids"], "segs": osg, "scores": osc, "counts": ocn, "vcls": vcls, "dense": (logits, offsets)}
 
     @_on_model_device
     def capture(self, staged, lane=0):
@@ -358,7 +368,7 @@ class _LocalizationBase(nn.Module):
     def d2h_bytes(res):
         return sum(res[k].numel() * res[k].element_size() for k in ("segs", "scores", "counts", "vcls"))
 
-    def _run(self, eng, x, valid, items):
+    def _run(self, eng, x, valid, items, dense=None):
         B = x.shape[0]
         self._sync_test_cfg(eng)
         logits, offsets, vcls, masks, lens = eng.forward_dense(x, valid)
@@ -368,6 +378,8 @@ class _LocalizationBase(nn.Module):
                           np.float32(it["duration"]))
         meta_d = torch.from_numpy(meta).to(eng.device, non_blocking=True)
         osg, osc, ocn = eng.postprocess(logits, offsets, masks, lens, meta_d, nms_method=self.test_nms_method)
+        if dense is not None:
+            eng.keep_dense(dense, [it["video_id"] for it in items], x.shape[1], logits, offsets, vcls, meta_d, valid)
         return self.fetch({"ids": [it["video_id"] for it in items], "segs": osg, "scores": osc, "counts": ocn, "vcls": vcls})
 
 

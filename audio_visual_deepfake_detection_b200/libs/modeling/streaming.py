@@ -218,13 +218,13 @@ class StreamRunner:
             vidx[b] = int(c.get("index", b))
         slot.rows, slot.chans, slot.B, slot.ids, slot.item = rows, chans, B, [c["video_id"] for c in chunk], item
 
-    def _launch(self, slot):
+    def _launch(self, slot, dense=None):
         with torch.cuda.device(self.eng.device):      # the caller's thread may have another device selected
             slot.stream.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(slot.stream):
-                self._launch_on_stream(slot)
+                self._launch_on_stream(slot, dense)
 
-    def _launch_on_stream(self, slot):
+    def _launch_on_stream(self, slot, dense=None):
         eng, B = self.eng, slot.B
         nbytes = 0
         if slot.direct is not None:
@@ -256,6 +256,9 @@ class StreamRunner:
             res = g.replay()
         else:
             res = self.model.run_staged(staged, lane=slot.index)
+        if dense is not None:         # copies of what the pass's post-processing read, after the pass, on this stream
+            logits, offsets = res["dense"]
+            eng.keep_dense(dense, slot.ids, eng.max_seq_len, logits, offsets, res["vcls"], staged["meta"], [eng.max_seq_len] * B)
         if res["segs"].shape[1] != slot.h_segs.shape[1]:      # nms_method 'none': every decoded candidate comes back
             n_out = res["segs"].shape[1]
             slot.h_segs = torch.zeros((eng.max_batch, n_out, 2), dtype=torch.float32, pin_memory=True)
@@ -453,17 +456,17 @@ class StreamRunner:
                  "labels": empty_labels[:int(cnt[r])], "video_cls": vcls[r:r + 1]} for r, c in enumerate(items)]
 
     # ---------------------------------------------------------------- public
-    def run(self, chunk):
-        """One batch, synchronously."""
+    def run(self, chunk, dense=None):
+        """One batch, synchronously. dense: optional DenseStore that keeps the batch's dense outputs."""
         slot = self.slots[0]
         with torch.cuda.device(self.eng.device):
             if slot.busy:
                 self._collect(slot)
             self._pack(slot, chunk)
-            self._launch(slot)
+            self._launch(slot, dense)
             return self._collect(slot)
 
-    def stream(self, batches):
+    def stream(self, batches, dense=None):
         """Generator over an iterable of batches (each <= max_batch videos): yields every batch's results in order.
         A packer thread fills free staging slots (pinned memcpy on the worker pool, GIL released) while this thread
         launches slot i (H2D + graph + D2H on the slot's stream) and collects slot i - (n_slots - 1)."""
@@ -538,7 +541,7 @@ class StreamRunner:
                 slot = ready.get()
                 if slot is None:
                     break
-                self._launch(slot)
+                self._launch(slot, dense)
                 inflight.append(slot)
                 if len(inflight) >= len(self.slots) - 1:
                     done = inflight.pop(0)

@@ -28,7 +28,7 @@ import numpy as np
 import torch
 
 from .... import ops
-from ..metrics import _device, _np, load_gt, prediction_columns, video_codes, video_csr
+from ..metrics import _device, _np, load_gt, prediction_columns, rows_csr, video_codes, video_csr
 
 GROUND_TRUTH_FIELDS = ["database", "taxonomy", "version"]
 PROPOSAL_FIELDS = ["results", "version", "external_data"]
@@ -96,6 +96,49 @@ def average_recall_vs_avg_nr_proposals(ground_truth, proposals, max_avg_nr_propo
                                    torch.from_numpy(score[p_rows]).to(dev), torch.from_numpy(keep.astype(np.int32)).to(dev),
                                    torch.from_numpy(gt_off).to(dev), torch.from_numpy(np.ascontiguousarray(g_se)).to(dev),
                                    thr, pcn)
+    recall = matches.cpu().numpy().astype(np.float64) / float(g_code.size)
+    avg_recall = recall.mean(axis=0)
+    proposals_per_video = pcn * (float(total) / n_video)
+    return recall, avg_recall, proposals_per_video
+
+
+def average_recall_from_rows(ground_truth, rows, K, layout, max_avg_nr_proposals=None, tiou_thresholds=DEFAULT_TIOU):
+    """average_recall_vs_avg_nr_proposals of result rows on the device ([N, 3 + 3K] fp32, record layout) of the videos
+    `layout` (metrics.RowsLayout over ground_truth) lists, in that order: the same numbers as for the records of those
+    videos. The proposal CSR and the per-video budgets are computed on the device; only the totals are read back."""
+    thr = np.asarray(tiou_thresholds, dtype=np.float64).reshape(-1)
+    dev = rows.device
+    g_code = layout.g_code
+    has_gt = np.zeros(layout.n_codes, dtype=bool)
+    has_gt[g_code] = True
+    sel = np.nonzero(has_gt[:layout.n])[0]
+    n_tail = int(has_gt[layout.n:].sum())
+    n_video = sel.size + n_tail
+    if n_video == 0:
+        raise ValueError("the ground truth has no rows: average recall is undefined")
+    n_prop = int(rows[:, 1].to(torch.int64).sum())
+    if n_prop == 0:
+        raise ValueError("there are no proposals: the average number of proposals is undefined")
+    if not max_avg_nr_proposals:
+        max_avg_nr_proposals = float(n_prop) / n_video
+    if max_avg_nr_proposals < 0:
+        raise ValueError("max_avg_nr_proposals must not be negative")
+    ratio = max_avg_nr_proposals * float(n_video) / n_prop
+    off, seg, score = rows_csr(rows, K, torch.from_numpy(sel).to(dev), n_tail)
+    n_p = off[1:] - off[:-1]
+    keep = torch.minimum((n_p.to(torch.float64) * ratio).to(torch.int64), n_p)
+    total = int(keep.sum())
+    if total == 0:
+        raise ValueError("max_avg_nr_proposals keeps no proposal of any video with ground truth")
+    pcn = np.arange(1, 101) / 100.0 * (max_avg_nr_proposals * float(n_video) / total)
+    local = np.cumsum(has_gt) - 1
+    g_loc = local[g_code]
+    g_rows = np.argsort(g_loc, kind="stable")
+    gt_off = np.zeros(n_video + 1, dtype=np.int32)
+    gt_off[1:] = np.cumsum(np.bincount(g_loc, minlength=n_video))
+    g_se = np.stack([ground_truth["t-start"].values, ground_truth["t-end"].values], 1).astype(np.float64)[g_rows]
+    matches, _ = ops.eval_proposal(off, seg, score, keep.to(torch.int32), torch.from_numpy(gt_off).to(dev),
+                                   torch.from_numpy(np.ascontiguousarray(g_se)).to(dev), thr, pcn)
     recall = matches.cpu().numpy().astype(np.float64) / float(g_code.size)
     avg_recall = recall.mean(axis=0)
     proposals_per_video = pcn * (float(total) / n_video)

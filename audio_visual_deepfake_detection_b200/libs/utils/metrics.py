@@ -156,6 +156,37 @@ def video_csr(p_code, g_code, n_codes, gt_videos_only=False):
     return p_rows, order, pred_off, g_rows, gt_off
 
 
+def rows_csr(rows, K, sel=None, n_tail=0):
+    """Prediction CSR of result rows on the device ([V, 3 + 3K] fp32 in the record layout [index, count, video_cls,
+    scores[K], segs[K][2]], scores sorted within a row): rows `sel` (int64 device tensor; None = all) in that order, then
+    n_tail videos without predictions. -> (pred_off int64 [V' + 1], pred_seg fp64 [N, 2], pred_score fp64 [N]); the
+    prediction order is row order, then output order within a row."""
+    r = rows if sel is None else rows.index_select(0, sel)
+    cnt = r[:, 1].to(torch.int64)
+    live = torch.arange(K, device=rows.device)[None, :] < cnt[:, None]
+    score = r[:, 3:3 + K][live].to(torch.float64)
+    seg = r[:, 3 + K:].reshape(-1, K, 2)[live].to(torch.float64)
+    off = torch.zeros(r.shape[0] + n_tail + 1, dtype=torch.int64, device=rows.device)
+    torch.cumsum(cnt, 0, out=off[1:r.shape[0] + 1])
+    off[r.shape[0] + 1:] = off[r.shape[0]]
+    return off, seg.contiguous(), score.contiguous()
+
+
+class RowsLayout:
+    """Where the GT rows of a ground-truth table fall relative to an ordered list of (unique) video ids: what evaluating
+    result rows of those videos needs besides the rows. codes 0..N-1 are the ids in order, N.. the videos only GT has."""
+
+    def __init__(self, gt, video_ids):
+        import pandas as pd
+        ids = np.asarray(list(video_ids), dtype=object)
+        codes, _ = pd.factorize(np.concatenate([ids, gt["video-id"].values.astype(object)]))
+        if ids.size and (codes[:ids.size] != np.arange(ids.size)).any():
+            raise ValueError("video ids of the result rows are not unique")
+        self.n = ids.size
+        self.n_codes = int(codes.max()) + 1 if codes.size else 0
+        self.g_code = codes[ids.size:]
+
+
 class ANETdetection(object):
     """The reference's evaluator. ant_file: ActivityNet-format JSON or AV-Deepfake1M metadata JSON (or a ground-truth
     DataFrame from one of the loaders). num_workers is accepted for compatibility and unused."""
@@ -200,6 +231,44 @@ class ANETdetection(object):
             for idx, k in enumerate(self.top_k):
                 block += "Recall@{:d}x = {:>4.2f} (%) ".format(k, tiou_mRecall[idx] * 100)
         return block + "\nAverage-mAP: {:>4.2f} (%)".format(average_mAP * 100)
+
+    def evaluate_rows(self, rows, K, layout, verbose=False):
+        """evaluate() of result rows on the device ([N, 3 + 3K] fp32, record layout, label 0) of the videos `layout`
+        (RowsLayout over this ground truth) lists, in that order: the same numbers evaluate() gives for the records of
+        those videos in that order. The prediction CSR is built on the device from the rows."""
+        dev = rows.device
+        gt = self.ground_truth
+        g_lab = gt["label"].values.astype(np.int64)
+        g_se = np.stack([gt["t-start"].values, gt["t-end"].values], 1).astype(np.float64)
+        n_thr, n_k, n_cls = len(self.tiou_thresholds), len(self.top_k), len(self.activity_index)
+        p_cls = self.activity_index.get(0, 0)
+        ap = np.zeros((n_thr, n_cls))
+        recall = np.zeros((n_thr, n_k, n_cls))
+        empty = None
+        for c in range(n_cls):
+            gsel = np.nonzero(g_lab == c)[0]
+            g_rows = gsel[np.argsort(layout.g_code[gsel], kind="stable")]
+            gt_off = np.zeros(layout.n_codes + 1, dtype=np.int32)
+            gt_off[1:] = np.cumsum(np.bincount(layout.g_code[gsel], minlength=layout.n_codes))
+            if c == p_cls:
+                off, seg, score = rows_csr(rows, K, n_tail=layout.n_codes - layout.n)
+            else:
+                if empty is None:
+                    empty = (torch.zeros(layout.n_codes + 1, dtype=torch.int64, device=dev),
+                             torch.zeros((0, 2), dtype=torch.float64, device=dev), torch.zeros(0, dtype=torch.float64, device=dev))
+                off, seg, score = empty
+            a, h, _ = ops.eval_detection(off, seg, score, torch.from_numpy(gt_off).to(dev),
+                                         torch.from_numpy(np.ascontiguousarray(g_se[g_rows])).to(dev),
+                                         self.tiou_thresholds, self.top_k)
+            ap[:, c] = a.cpu().numpy()
+            recall[:, :, c] = h.cpu().numpy() / float(gsel.size)
+        self.ap, self.recall = ap, recall
+        mAP = ap.mean(axis=1)
+        mRecall = recall.mean(axis=2)
+        average_mAP = mAP.mean()
+        if verbose:
+            print(self.table(mAP, average_mAP, mRecall))
+        return mAP, average_mAP, mRecall
 
     def evaluate_classes(self, preds, want_tp=False):
         """-> (ap [n_thr, n_cls], recall [n_thr, n_topk, n_cls], tp_mask): tp_mask (want_tp) is a uint16 array over the

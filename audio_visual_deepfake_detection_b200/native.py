@@ -33,6 +33,7 @@ EXPORTS = [
     "avdf_session_create", "avdf_session_get_io", "avdf_session_run", "avdf_session_destroy",
     "avdf_plan_window_layout", "avdf_session_window_bytes", "avdf_session_attach_windows", "avdf_session_run_windows",
     "avdf_format_results_workspace_bytes", "avdf_format_results",
+    "avdf_postprocess_sweep_workspace_bytes", "avdf_postprocess_sweep",
 ]
 
 
@@ -55,6 +56,28 @@ class PostprocessArgs(Structure):
         ("workspace", c_void_p), ("workspace_bytes", c_size_t),
         ("rec_ring", c_void_p), ("rec_counter", c_void_p), ("rec_cap", c_int32), ("vid_index", c_void_p), ("vid_cls", c_void_p),
         ("out_index", c_void_p),
+    ]
+
+
+class SweepSetting(Structure):
+    _fields_ = [
+        ("pre_nms_thresh", c_float), ("pre_nms_topk", c_int32), ("duration_thresh", c_float),
+        ("iou_threshold", c_float), ("min_score", c_float), ("sigma", c_float), ("voting_thresh", c_float),
+        ("max_seg_num", c_int32), ("use_soft_nms", c_int32),
+    ]
+
+
+class PostprocessSweepArgs(Structure):
+    _fields_ = [
+        ("batch", c_int32),
+        ("logits", c_void_p), ("offsets", c_void_p), ("valid_len", c_void_p),
+        ("n_levels", c_int32),
+        ("level_len", c_int32 * MAX_LEVELS), ("level_stride", c_float * MAX_LEVELS),
+        ("vid_feat_stride", c_void_p), ("vid_half_nframes", c_void_p), ("vid_fps", c_void_p), ("vid_duration", c_void_p),
+        ("vid_cls", c_void_p), ("vid_index", c_void_p),
+        ("n_settings", c_int32), ("settings", POINTER(SweepSetting)),
+        ("out_rows", c_void_p), ("rows_per_setting", c_int64), ("row_k", c_int32),
+        ("workspace", c_void_p), ("workspace_bytes", c_size_t),
     ]
 
 
@@ -200,6 +223,9 @@ def lib():
     L.avdf_postprocess_workspace_bytes.restype = c_size_t
     L.avdf_postprocess_workspace_bytes.argtypes = [c_int32, c_int32]
     L.avdf_postprocess.argtypes = [POINTER(PostprocessArgs), c_void_p]
+    L.avdf_postprocess_sweep_workspace_bytes.restype = c_size_t
+    L.avdf_postprocess_sweep_workspace_bytes.argtypes = [c_int32, c_int32]
+    L.avdf_postprocess_sweep.argtypes = [POINTER(PostprocessSweepArgs), c_void_p]
     L.avdf_conv_gemm_workspace_bytes.restype = c_size_t
     L.avdf_conv_gemm_workspace_bytes.argtypes = [POINTER(ConvGemmArgs)]
     L.avdf_conv_gemm.argtypes = [POINTER(ConvGemmArgs), c_void_p]
@@ -250,7 +276,8 @@ def lib():
         if name not in ("avdf_last_error", "avdf_nms_workspace_bytes", "avdf_postprocess_workspace_bytes",
                         "avdf_conv_gemm_workspace_bytes", "avdf_eval_workspace_bytes", "avdf_eval_proposal_workspace_bytes",
                         "avdf_window_merge_workspace_bytes", "avdf_abi_version", "avdf_plan_close", "avdf_session_destroy",
-                        "avdf_session_window_bytes", "avdf_format_results_workspace_bytes"):
+                        "avdf_session_window_bytes", "avdf_format_results_workspace_bytes",
+                        "avdf_postprocess_sweep_workspace_bytes"):
             fn.restype = c_int32
     if L.avdf_abi_version() != 3:
         raise AvdfError("libavdf_sm100.so ABI version mismatch")

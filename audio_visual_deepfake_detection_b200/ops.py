@@ -255,6 +255,41 @@ def postprocess_workspace_bytes(batch, cand_cap):
     return nv.lib().avdf_postprocess_workspace_bytes(batch, cand_cap)
 
 
+def postprocess_sweep(logits, offsets, valid_len, *, level_len, level_stride, settings, out_rows, vid_meta=None, vid_cls=None,
+                      vid_index=None, workspace=None):
+    """Post-processing of the same dense outputs under up to 64 settings in one launch (include/avdf.h
+    avdf_postprocess_sweep). logits [B, P] / offsets [B, P, 2] fp32, valid_len int32 [B]; settings: sequence of
+    nv.SweepSetting; out_rows fp32 [S, R, 3 + 3K] (video b of setting s -> out_rows[s, vid_index[b] or b]).
+    vid_meta: optional 4 fp32 [B] tensors (feat_stride, half frames, fps, duration). Returns the workspace used."""
+    L = nv.lib()
+    _chk(logits, torch.float32, "logits"); _chk(offsets, torch.float32, "offsets"); _chk(valid_len, torch.int32, "valid_len")
+    _chk(out_rows, torch.float32, "out_rows"); _chk(vid_cls, torch.float32, "vid_cls"); _chk(vid_index, torch.int32, "vid_index")
+    B, P = logits.shape
+    S = len(settings)
+    assert offsets.shape == (B, P, 2) and valid_len.numel() == B and out_rows.dim() == 3 and out_rows.shape[0] == S
+    a = nv.PostprocessSweepArgs()
+    a.batch, a.logits, a.offsets, a.valid_len = B, logits.data_ptr(), offsets.data_ptr(), valid_len.data_ptr()
+    a.n_levels = len(level_len)
+    for i, (n, s) in enumerate(zip(level_len, level_stride)):
+        a.level_len[i] = int(n); a.level_stride[i] = float(s)
+    if vid_meta is not None:
+        for t in vid_meta:
+            _chk(t, torch.float32, "vid_meta")
+        a.vid_feat_stride, a.vid_half_nframes, a.vid_fps, a.vid_duration = [t.data_ptr() for t in vid_meta]
+    a.vid_cls = vid_cls.data_ptr() if vid_cls is not None else None
+    a.vid_index = vid_index.data_ptr() if vid_index is not None else None
+    table = (nv.SweepSetting * max(1, S))(*settings)
+    a.n_settings, a.settings = S, table
+    a.out_rows, a.rows_per_setting, a.row_k = out_rows.data_ptr(), out_rows.shape[1], (out_rows.shape[2] - 3) // 3
+    need = L.avdf_postprocess_sweep_workspace_bytes(B, P)
+    if need and (workspace is None or workspace.numel() * workspace.element_size() < need):
+        workspace = torch.empty(need, dtype=torch.uint8, device=logits.device)
+    if need:
+        a.workspace, a.workspace_bytes = workspace.data_ptr(), need
+    _call("avdf_postprocess_sweep", L.avdf_postprocess_sweep, (ctypes.byref(a), _stream(),), launches=1, work=None)
+    return workspace
+
+
 # ---------------------------------------------------------------------------- conv GEMM
 def conv_gemm(a, w, *, taps, stride=1, batch, c_in, n_out, segs, a_rows, o_rows, bias=None, row_mask=None, ln=None,
               act=ACT_NONE, pe=None, residual=None, gamma=None, out_f32=None, out_h=None, workspace=None,

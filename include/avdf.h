@@ -167,6 +167,45 @@ typedef struct avdf_postprocess_args {
 AVDF_API size_t avdf_postprocess_workspace_bytes(int32_t batch, int32_t cand_cap);
 AVDF_API int avdf_postprocess(const avdf_postprocess_args* args, void* stream);
 
+/* ---- post-processing sweep: up to 64 test_cfg settings over the same dense outputs, one launch ----
+ * Every setting gives, per video, exactly what avdf_postprocess gives with that setting on these inputs (decode with
+ * the setting's pre_nms_thresh / pre_nms_topk / duration_thresh, hard NMS or soft NMS method 2, voting, stable sort and
+ * cap, seconds). Settings with equal decode triples share one decoded candidate list per video. The pyramid mask is
+ * rebuilt from valid_len: point t of level l is kept iff t * level_stride[l] < valid_len[b] (the model's nearest
+ * down-sampled mask). Video b of setting s writes row s * rows_per_setting + r, r = vid_index[b] (b when NULL), in the
+ * avdf_postprocess record layout [r, count, video_cls, scores[row_k], segs[row_k][2]], zero beyond count; a video whose r
+ * is outside [0, rows_per_setting) writes nothing. The settings table is read on the host and validated before any
+ * launch (-1 and no launch on a bad argument); no memory is allocated. */
+typedef struct avdf_sweep_setting {
+  float pre_nms_thresh; int32_t pre_nms_topk; float duration_thresh;
+  float iou_threshold, min_score, sigma, voting_thresh;   /* voting_thresh 0: no voting (also multiclass_nms) */
+  int32_t max_seg_num;           /* 1 .. row_k */
+  int32_t use_soft_nms;          /* 0 hard, 1 soft (method 2; sigma > 0) */
+} avdf_sweep_setting;
+typedef struct avdf_postprocess_sweep_args {
+  int32_t batch;
+  const float* logits;           /* [batch, P]      P = sum(level_len) */
+  const float* offsets;          /* [batch, P, 2]   */
+  const int32_t* valid_len;      /* [batch]         */
+  int32_t n_levels;
+  int32_t level_len[AVDF_MAX_LEVELS];
+  float level_stride[AVDF_MAX_LEVELS];
+  const float* vid_feat_stride;  /* [batch] seconds conversion, as avdf_postprocess (all NULL: feature grid) */
+  const float* vid_half_nframes;
+  const float* vid_fps;
+  const float* vid_duration;
+  const float* vid_cls;          /* [batch] or NULL */
+  const int32_t* vid_index;      /* [batch] or NULL */
+  int32_t n_settings;            /* 1 .. 64 */
+  const avdf_sweep_setting* settings;   /* host array [n_settings] */
+  float* out_rows;               /* [n_settings, rows_per_setting, 3 + 3 * row_k] */
+  int64_t rows_per_setting;
+  int32_t row_k;                 /* >= every max_seg_num, <= AVDF_MAX_SEGS */
+  void* workspace; size_t workspace_bytes;   /* avdf_postprocess_sweep_workspace_bytes(batch, P) */
+} avdf_postprocess_sweep_args;   /* host struct */
+AVDF_API size_t avdf_postprocess_sweep_workspace_bytes(int32_t batch, int32_t n_points);
+AVDF_API int avdf_postprocess_sweep(const avdf_postprocess_sweep_args* args, void* stream);
+
 /* ---- cross-window merge of the sliding-window path (csrc/window.cu) ----
  * Recording r owns window rows [rec_win[r], rec_win[r+1]) of the window outputs (the per-window postprocess results:
  * seconds within the window, sorted, win_count[w] <= max_seg_num of them). For a recording with more than one window:
